@@ -11,7 +11,10 @@ contiguous ranges of 4096 / N per GPU (pressurefieldcontact.jl_b200/parallel.py:
 no collective on the path.  Secondary blocks of the same line: `weak` (4096 environments on every GPU) and `large_scenes` (C4 / C5:
 one very large scene; at N > 1 its candidate-pair lists are split over the N GPUs and the per-instruction partial sums cross NCCL).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--envs E] [--impl reference] [--dump-outputs DIR]
+
+--dump-outputs DIR also writes what the timed path returned in its last step as DIR/<name>.npy (float64; see dump_outputs): the
+inputs are seeded, so two builds run with the same arguments can be compared array by array.
 
 Prints ONE JSON line (rank 0).  `value` = device-resident throughput (CUDA events on the
 library's stream, L2 flushed between steps); `e2e` = the same metric through pfc_eval_f64 with
@@ -60,6 +63,29 @@ def build_inputs(n_env, start=0):
     X, tw, s = S.boundary_arrays(m, x_all)
     m.x_all = np.ascontiguousarray(x_all)
     return m, np.ascontiguousarray(X), np.ascontiguousarray(tw)
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, local, n_total, rank=0, world=1):
+    """Writes `local` (name -> this rank's rows, one per environment) as out_dir/<name>.npy in float64, the environments of all
+    ranks in global order.  When the rows of all n_total environments exceed DUMP_BYTES, a fixed seeded sample of environments is
+    written instead; env_index.npy always lists the environments written."""
+    if world > 1:
+        import torch.distributed as dist
+        parts = [None] * world
+        dist.all_gather_object(parts, local)
+        local = {k: np.concatenate([p[k] for p in parts]) for k in local}
+    if rank != 0:
+        return
+    per_env = 8 * (1 + sum(a[0].size for a in local.values()))
+    n_keep = min(n_total, DUMP_BYTES // per_env)
+    rows = np.arange(n_total) if n_keep == n_total else np.sort(np.random.default_rng(0).choice(n_total, n_keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "env_index.npy"), rows.astype(np.float64))
+    for name, a in local.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[rows], dtype=np.float64))
 
 
 class ClockSampler:
@@ -234,8 +260,10 @@ def run_reference(args):
         ctx.eval_f64(X, tw)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        ctx.eval_f64(X, tw)
+        out = ctx.eval_f64(X, tw)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {k: out[k] for k in ("wrench", "n_pairs", "flags")}, n_env)
     v = n_env * args.steps / dt
     print(json.dumps({
         "impl": "reference", "metric": METRIC, "value": v, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -257,7 +285,10 @@ def main():
     ap.add_argument("--impl", default="pfc", choices=["pfc", "reference"])
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--no-large", action="store_true", help="skip the secondary single-large-scene measurements (C4 / C5)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (bench_outputs/ is git-ignored)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -347,6 +378,8 @@ def main():
         barrier()
         launches = ctx.launch_count() - launches0
         dev_ms = sum(a.elapsed_time(b) for a, b in zip(ev0, ev1))
+        # the last timed step's results, before the per-kernel split below runs the path again
+        last = {"wrench": w_d.cpu().numpy(), "n_pairs": np_d.cpu().numpy(), "flags": fl_d.cpu().numpy()} if args.dump_outputs else None
         # ---- timed region 2: end to end through pfc_eval_f64 with pinned host buffers (wall clock; the call is synchronous) ----
         barrier()
         t0 = time.perf_counter()
@@ -409,6 +442,8 @@ def main():
     assert np.array_equal(w_host, w_p.numpy()), "device-resident and host-pointer entry points disagree"
     f_chk = S.generalized_forces(m, m.x_all[0], w_host[0])
     assert np.abs(f_p.numpy()[0] - f_chk).max() <= 1e-9 * max(np.abs(f_chk).max(), 1e-300), "state-level entry point disagrees with J' w on the host"
+    if args.dump_outputs:   # f_p still holds the last step of timed region 2's state-level leg
+        dump_outputs(args.dump_outputs, dict(last, f_generalized=f_p.numpy()), n_total, rank, world)
 
     # secondary: one very large scene (C4 / C5); at N > 1 split over the GPUs with an NCCL exchange of the partial sums (all ranks take part)
     large = None if args.no_large else measure_large_scenes(local_rank, rank, world)
