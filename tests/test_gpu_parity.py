@@ -6,7 +6,7 @@ import numpy as np
 import pytest
 
 import pfc_b200  # noqa: F401
-from helpers import boxes_env_states, rot_z, scene_boxes, wrench_rel_err
+from helpers import _sphere_scene, _sphere_states, _tet_tet_scene, boxes_env_states, rot_z, scene_boxes, wrench_rel_err
 from oracle import orc
 from pfc_b200 import geometry as G
 from pfc_b200 import scenario as S
@@ -121,20 +121,6 @@ def test_bristle_sliding_batch():
     assert (c["flags"][1:, 0] & 1).all()
 
 
-def _tet_tet_scene(backend, n_env):
-    r = 0.05
-    c_prop = S.ContactProperties(1.0e6)
-    m = S.MechanismScenario()
-    id_plane = S.add_contact(m, "plane", G.as_tet_eMesh(G.eMesh_half_plane()), c_prop=c_prop)
-    b1 = S.add_body_contact(m, "box_1", G.as_tet_eMesh(G.eMesh_box(r)), i_prop=S.InertiaProperties(400.0), c_prop=c_prop)
-    b2 = S.add_body_contact(m, "box_2", G.as_tet_eMesh(G.eMesh_box(r)), i_prop=S.InertiaProperties(400.0), c_prop=S.ContactProperties(3.0e6))
-    S.add_friction_regularize(m, id_plane, b1[2], mu_d=0.0, chi=0.0, n_quad_rule=2)
-    S.add_friction_regularize(m, b1[2], b2[2], mu_s=0.4, mu_d=0.3, chi=0.7, v_tol=1e-3, n_quad_rule=2)
-    S.add_friction_bristle(m, b2[2], b1[2], mu_d=0.3, chi=0.3, k_bar=1.0e5, tau=0.02, n_quad_rule=1)
-    S.finalize(m, backend, n_env)
-    return m
-
-
 def test_tet_tet_batch_parity():
     """test/test_vol_vol.jl-style volumetric contact (tet-tet), regularized and bristle."""
     n_env = 128
@@ -247,44 +233,6 @@ def force_large_path(monkeypatch):
     """Trees of a few hundred leaves normally take the on-chip path with a bounded pair-list slot (build_tables in csrc/pfc_api.cu);
     these tests are about the multi-kernel large path, so that class is switched off while their scenes are built."""
     monkeypatch.setenv("PFC_MID_LEAVES", "0")
-
-
-def _sphere_scene(n_div_a=4, n_div_b=3, with_small=True):
-    def build(backend, n_env):
-        m = S.MechanismScenario()
-        sa, sb = G.eMesh_sphere(0.05, n_div_a), G.eMesh_sphere(0.06, n_div_b)
-        ground = S.add_contact(m, "ground", G.as_tet_eMesh(sb), c_prop=S.ContactProperties(2.0e6))
-        b1 = S.add_body_contact(m, "s_tri", G.as_tri_eMesh(sa), i_prop=S.InertiaProperties(400.0, d=0.01))
-        b2 = S.add_body_contact(m, "s_tet", G.as_tet_eMesh(sa), i_prop=S.InertiaProperties(400.0), c_prop=S.ContactProperties(1.0e6))
-        S.add_friction_regularize(m, b1[2], ground, mu_s=0.4, mu_d=0.3, chi=0.5, n_quad_rule=2)   # tri-tet, large
-        S.add_friction_regularize(m, b2[2], ground, mu_d=0.3, chi=0.5, n_quad_rule=1)            # tet-tet, large
-        S.add_friction_bristle(m, b1[2], b2[2], mu_d=0.4, k_bar=2.0e4, tau=0.05, n_quad_rule=2)  # tri-tet, large, bristle
-        if with_small:
-            box = S.add_body_contact(m, "box", G.as_tri_eMesh(G.eMesh_box(0.03)), i_prop=S.InertiaProperties(400.0, d=0.01))
-            plane = S.add_contact(m, "plane", G.as_tet_eMesh(G.eMesh_half_plane()), c_prop=S.ContactProperties(1.0e6))
-            S.add_friction_regularize(m, box[2], plane, mu_d=0.3, chi=0.5, n_quad_rule=2)        # small path in the same scene
-        S.finalize(m, backend, n_env)
-        return m
-    return build
-
-
-def _sphere_states(m, n_env, seed, with_small=True):
-    rng = np.random.default_rng(seed)
-    x = np.zeros((n_env, S.num_x(m)))
-    nq = m.nq
-    for e in range(n_env):
-        d1 = rng.standard_normal(3); d1 /= np.linalg.norm(d1)
-        d2 = rng.standard_normal(3); d2 /= np.linalg.norm(d2)
-        x[e, 0:3] = rng.uniform(-0.3, 0.3, 3)
-        x[e, 3:6] = d1 * rng.uniform(0.095, 0.108)
-        x[e, 6:9] = rng.uniform(-0.3, 0.3, 3)
-        x[e, 9:12] = x[e, 3:6] + d2 * rng.uniform(0.085, 0.098) if e % 2 else d2 * rng.uniform(0.095, 0.108)
-        if with_small:
-            x[e, 12:15] = rng.uniform(-0.02, 0.02, 3)
-            x[e, 15:18] = [rng.uniform(-0.1, 0.1), rng.uniform(-0.1, 0.1), 0.03 - rng.uniform(0, 0.003)]
-        x[e, nq:nq + m.nv] = rng.uniform(-1, 1, m.nv) * 0.3
-        x[e, nq + m.nv:] = rng.uniform(-1, 1, 6) * 1e-4
-    return x
 
 
 def test_large_path_spheres(force_large_path):
