@@ -40,7 +40,8 @@ enum {
     PFC_E_CUDA = -2,      /* CUDA runtime error (message has the CUDA string) */
     PFC_E_CAPACITY = -3,  /* a fixed capacity was exceeded and could not be grown */
     PFC_E_NONFINITE = -4, /* the reference's error("Non-finite vertex likely"), src/clip/static_clip.jl:52 */
-    PFC_E_MESH = -5       /* invalid mesh (inverted tetrahedron, src/obb/obb_construction.jl:30; bad tree) */
+    PFC_E_MESH = -5,      /* invalid mesh (inverted tetrahedron, src/obb/obb_construction.jl:30; bad tree) */
+    PFC_E_STEP = -6       /* error("time step is too small, something is wrong") / unacceptable h (src/radau/radau_solve.jl, adaptive.jl:52-57) */
 };
 
 /* per-(environment, instruction) flag bits */
@@ -150,6 +151,29 @@ int pfc_refit_mesh(pfc_ctx* ctx, int mesh_id, int64_t n_point, const double* xyz
  * Gauss-Jordan with partial pivoting in shared memory.  *info (optional) gets bit 0 if a pivot vanished.  Device pointers; asynchronous. */
 int pfc_radau_inv_c_device(pfc_ctx* ctx, int64_t n_mat, int n, const double* neg_J, const double* shift, const int32_t* index, double* inv_c,
                            int32_t* info);
+/* Adaptive Radau IIA (src/radau) for n_env environments of a pfc_set_dynamics scene, every array on the device.
+ * pfc_radau_init resets the per-environment controller to the reference's initial state (RadauStep / RadauRule, radau_struct.jl:64-95:
+ * h = h0, rule 1, cooldown 10, Psi 9999) and sizes the buffers.  max_rule in 1..3 (NR; stages 2 rule - 1); n_x <= 96; tol_newton >= 0.
+ * tol_a = tol_r = 1e-4, h_min = 1e-8, k_iter_max = 15 are the reference's constants.  The context owns the work space; the largest part is
+ * the inverses (h^-1 lambda_i I - J)^-1: n_env (2 max_rule - 1) n_x^2 complex doubles -- 453 MB for 4096 environments of n_x = 48 at
+ * max_rule = 2 -- besides the Jacobians (n_env n_x^2 doubles) and the stage states. */
+int pfc_radau_init(pfc_ctx* ctx, int64_t n_env, int max_rule, double h0, double h_max, double tol_newton);
+/* solveRadau (radau_solve.jl:1-34) for every environment: ONE accepted step each.  x[env][n_x] in/out (principal_value! applied to the
+ * MRPs of SPQuatFloating bodies after the step), t[env] in/out, h_taken[env] out, tau_ext[env][nv] (held constant over the step) or NULL,
+ * stats[env][4] (or NULL) = {stages of the accepted attempt, its Newton iterations, rejected attempts, stage evaluations over all attempts}.
+ * An environment whose attempt fails retries with its own smaller h and rule while the others wait; the Jacobian is not recomputed for a
+ * retry (radau_solve.jl:23-28).  Every environment takes the decisions the single-scene integrator would take for it alone, and its
+ * result does not depend on the batch it is in.  Device pointers; the call synchronises the stream once per Newton iteration to read how
+ * many (environment, stage) states are still active, and once per round of attempts; outputs are ready in stream order when it returns.
+ * Returns PFC_E_STEP when an environment's step size falls below h_min (or becomes unacceptable), PFC_E_NONFINITE / PFC_E_CAPACITY as
+ * pfc_calcxd_f64 does for the evaluations of the step; the outputs are then undefined. */
+int pfc_radau_step_device(pfc_ctx* ctx, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats);
+/* Same on host pointers (copies in and out are part of the call). */
+int pfc_radau_step(pfc_ctx* ctx, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats);
+/* Of the last pfc_radau_step[_device] call: counts[0] = rounds of attempts, counts[1] = host synchronisations; ms[0..3] = device time of
+ * the Jacobian, the stage evaluations, the inverses, and the Newton + controller kernels (CUDA events; zeros unless pfc_set_timing is on).
+ * Either pointer may be NULL. */
+int pfc_radau_step_info(pfc_ctx* ctx, double* ms, int64_t* counts);
 /* Debug / parity: the boundary arrays (X_r2_r1, twist_r2) the prologue computed and the per-instruction wrenches of the last
  * host-pointer evaluation; any pointer may be NULL. */
 int pfc_get_boundary(pfc_ctx* ctx, int64_t n_env, double* X_r2_r1, double* twist_r2, double* wrench_r2);

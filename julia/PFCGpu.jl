@@ -219,6 +219,26 @@ function calcJacobian_batch_gpu!(jac::Array{Float64,3}, xx::Matrix{Float64}, m::
     return nothing
 end
 
+"Resets the batched Radau integrator of the context (pfc_radau_init): n_env environments, h = h0, rule 1 (RadauStep / RadauRule),
+at most `max_rule` (NR) rules, the reference's tolerances."
+function radau_init!(m::MechanismScenario, n_env::Integer; max_rule::Integer = 2, h0::Float64 = 1.0e-4, h_max::Float64 = 0.01,
+                     tol_newton::Float64 = 1.0e-16)
+    check(ccall((:pfc_radau_init, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Float64, Float64, Float64), CTX[m], n_env, max_rule, h0, h_max, tol_newton))
+    return nothing
+end
+
+"One accepted Radau step (solveRadau + principal_value!) of every environment `x[:, env]` (pfc_radau_step, host arrays; pfc_radau_step_device
+for `CuArray`s): `x` and `t` in place, `h_taken[env]` out; `tau_ext[:, env]` is held over the step.  Returns `stats[:, env]` = stages of the
+accepted attempt, its Newton iterations, rejected attempts, stage evaluations."
+function radau_step_batch_gpu!(m::MechanismScenario, x::Matrix{Float64}, t::Vector{Float64}, h_taken::Vector{Float64};
+                               tau_ext::Union{Nothing,Matrix{Float64}} = nothing)
+    stats = zeros(Int32, 4, size(x, 2))
+    tau = tau_ext === nothing ? C_NULL : tau_ext
+    GC.@preserve x t h_taken tau_ext stats check(ccall((:pfc_radau_step, LIB), Cint,
+        (Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}), CTX[m], size(x, 2), x, tau, t, h_taken, stats))
+    return stats
+end
+
 "Moved vertices of mesh `id` (same connectivity): the device rebuilds the mesh's primitive records and refits its tree (pfc_refit_mesh)."
 function refit_mesh_gpu!(m::MechanismScenario, id::MeshID, point::Vector{SVector{3,Float64}})
     xyz = collect(Iterators.flatten(point))

@@ -22,7 +22,7 @@ _vp = C.c_void_p
 SYMBOLS = [
     "pfc_create", "pfc_destroy", "pfc_add_mesh", "pfc_add_instruction", "pfc_finalize", "pfc_eval_f64", "pfc_eval_f64_device",
     "pfc_eval_dual6", "pfc_set_debug", "pfc_get_pairs", "pfc_get_traction", "pfc_set_shard", "pfc_eval_sharded_begin", "pfc_eval_sharded_partials", "pfc_eval_sharded_step", "pfc_sync", "pfc_stream",
-    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
+    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
     "pfc_comm_unique_id", "pfc_comm_init_rank", "pfc_eval_sharded_f64_device", "pfc_group_create", "pfc_group_destroy", "pfc_group_size", "pfc_group_ctx",
     "pfc_group_add_mesh", "pfc_group_add_instruction", "pfc_group_finalize", "pfc_group_eval_f64",
 ]
@@ -70,6 +70,10 @@ def lib():
         L.pfc_calcxd_jacobian_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp]
         L.pfc_refit_mesh.argtypes = [_vp, C.c_int, C.c_int64, _d]
         L.pfc_radau_inv_c_device.argtypes = [_vp, C.c_int64, C.c_int, _vp, _vp, _vp, _vp, _vp]
+        L.pfc_radau_init.argtypes = [_vp, C.c_int64, C.c_int, C.c_double, C.c_double, C.c_double]
+        L.pfc_radau_step.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
+        L.pfc_radau_step_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
+        L.pfc_radau_step_info.argtypes = [_vp, _vp, _vp]
         L.pfc_comm_unique_id.argtypes = [_vp]
         L.pfc_comm_init_rank.argtypes = [_vp, _vp, C.c_int, C.c_int]
         L.pfc_eval_sharded_f64_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
@@ -266,6 +270,34 @@ class Context:
     def radau_inv_c_device(self, n_mat, n, neg_J, shift, index, inv_c, info=None):
         """Batched updateInvC!: device pointers given as integers; asynchronous on self.stream."""
         _check(lib().pfc_radau_inv_c_device(self._h, n_mat, n, neg_J, shift, index, inv_c, info))
+
+    def radau_init(self, n_env, max_rule=2, h0=1.0e-4, h_max=0.01, tol_newton=1.0e-16):
+        """Resets the batched Radau controller of n_env environments (h = h0, rule 1) and sizes its buffers."""
+        _check(lib().pfc_radau_init(self._h, int(n_env), int(max_rule), float(h0), float(h_max), float(tol_newton)))
+
+    def radau_step(self, x, t, tau_ext=None):
+        """One accepted Radau step of every environment: host arrays in -> (x [env][n_x], t [env], h_taken [env], stats [env][4])."""
+        nx = self.nq + self.nv + 6 * self.n_bristle
+        x = _a(x).reshape(-1, nx).copy()
+        n_env = x.shape[0]
+        t = _a(t).reshape(n_env).copy()
+        tau = None if tau_ext is None else _a(tau_ext).reshape(n_env, self.nv)
+        h = np.zeros(n_env)
+        stats = np.zeros((n_env, 4), np.int32)
+        _check(lib().pfc_radau_step(self._h, n_env, _p(x), _p(tau), _p(t), _p(h), _p(stats)))
+        return x, t, h, stats
+
+    def radau_step_device(self, n_env, x, tau_ext, t, h_taken, stats):
+        """Device pointers given as integers (tau_ext / stats may be None); on self.stream."""
+        _check(lib().pfc_radau_step_device(self._h, n_env, x, tau_ext, t, h_taken, stats))
+
+    def radau_step_info(self):
+        """(ms [Jacobian, stage evaluations, inverses, Newton + controller] -- needs set_timing(True) --, rounds, host synchronisations)
+        of the last Radau step."""
+        ms = np.zeros(4)
+        counts = np.zeros(2, np.int64)
+        _check(lib().pfc_radau_step_info(self._h, _p(ms), _p(counts)))
+        return ms, int(counts[0]), int(counts[1])
 
     def calcxd_f64_device(self, n_env, x, tau_ext, xdot, n_pairs, flags):
         """Device pointers given as integers; asynchronous on self.stream."""

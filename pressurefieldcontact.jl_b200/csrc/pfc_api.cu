@@ -17,6 +17,7 @@
 #include "pfc_exact.h"
 #include "pfc_large.h"
 #include "pfc_launch.h"
+#include "pfc_radau_step.cuh"
 
 using namespace pfc;
 
@@ -222,6 +223,20 @@ struct pfc_ctx {
     bool large_index_dirty = true;
     int* h_status = nullptr;    // pinned
     DynDev dyn{};
+    // batched Radau step (pfc_radau_init / pfc_radau_step): controller state and work space for radau_n_env environments
+    struct RadauState {
+        int64_t n_env = -1;
+        int max_rule = 0, s_max = 0;
+        double h_max = 0.0, tol_newton = 0.0;
+        DevBuf<RadauEnv> env;
+        DevBuf<double> X, Xp, Fp, taup, xx0, jac, invc, shift, x, tau, t, h;
+        DevBuf<int> index, state_list, env_list, state_pos, inv_base, counts, stats, flags, flags_stage, info;
+        DevBuf<long long> np, np_stage;
+        int* h_counts = nullptr;   // pinned: counts[0..3] + the status word
+        int64_t rounds = 0, syncs = 0;   // of the last step
+        double ms[4] = {0, 0, 0, 0};     // of the last step with pfc_set_timing on: Jacobian, stage evaluations, inverses, Newton + controller
+        std::vector<cudaEvent_t> ev_pool;
+    } radau;
     bool timing = false;
     cudaEvent_t ev[8] = {};
     bool ev_valid = false;
@@ -311,6 +326,8 @@ int pfc_destroy(pfc_ctx* c) {
     c->d_H.release(); c->d_Hinv.release(); c->d_xdot.release(); c->d_tau.release(); c->d_status.release(); c->d_refit_xyz.release(); c->d_refit_aabb.release();
     for (auto& r : c->refit) { r.idx.release(); r.eps.release(); r.level_nodes.release(); }
     if (c->h_status) { cudaFreeHost(c->h_status); c->h_status = nullptr; }
+    if (c->radau.h_counts) { cudaFreeHost(c->radau.h_counts); c->radau.h_counts = nullptr; }
+    for (cudaEvent_t ev : c->radau.ev_pool) cudaEventDestroy(ev);
     if (c->h_ins_overflow) { cudaFreeHost(c->h_ins_overflow); c->h_ins_overflow = nullptr; }
     if (c->h_arena) { cudaFreeHost(c->h_arena); c->h_arena = nullptr; }
     for (int k = 0; k < 8; ++k) if (c->ev[k]) cudaEventDestroy(c->ev[k]);
@@ -1750,6 +1767,161 @@ int pfc_radau_inv_c_device(pfc_ctx* c, int64_t n_mat, int n, const double* neg_J
     CU(cudaSetDevice(c->device));
     CU(launch_radau_inv_c(n_mat, n, neg_J, shift, index, inv_c, info, c->stream));
     c->launches += 1;
+    return PFC_OK;
+}
+
+// ---- batched adaptive Radau IIA step (solveRadau, radau_solve.jl:1-34) ------------------------------------------------------------
+int pfc_radau_init(pfc_ctx* c, int64_t n_env, int max_rule, double h0, double h_max, double tol_newton) {
+    if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_radau_init: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
+    if (n_env < 0) return fail(PFC_E_ARG, "pfc_radau_init: negative n_env");
+    if (max_rule < 1 || max_rule > kRadauMaxRule) return fail(PFC_E_ARG, "pfc_radau_init: max_rule must be 1, 2 or 3");
+    if (c->state.n_x < 1 || c->state.n_x > 96) return fail(PFC_E_ARG, "pfc_radau_init: the state must have 1 to 96 entries");
+    if (!(std::isfinite(h0) && h0 > 0.0) || !(std::isfinite(h_max) && h_max > 0.0)) return fail(PFC_E_ARG, "pfc_radau_init: h0 and h_max must be finite and positive");
+    if (!(tol_newton >= 0.0) || !std::isfinite(tol_newton)) return fail(PFC_E_ARG, "pfc_radau_init: tol_newton must be finite and >= 0");
+    CU(cudaSetDevice(c->device));
+    pfc_ctx::RadauState& r = c->radau;
+    r.n_env = -1;   // not usable until everything below succeeded
+    const size_t ne = size_t(n_env), nx = size_t(c->state.n_x), nv = size_t(c->state.nv), ni = size_t(c->scene.n_ins);
+    const size_t s_max = size_t(2 * max_rule - 1), ns = std::max<size_t>(ne * s_max, 1), ne1 = std::max<size_t>(ne, 1);
+    CU(r.env.ensure(ne1)); CU(r.X.ensure(ns * nx)); CU(r.Xp.ensure(ns * nx)); CU(r.Fp.ensure(ns * nx)); CU(r.taup.ensure(ns * std::max<size_t>(nv, 1)));
+    CU(r.xx0.ensure(ne1 * nx)); CU(r.jac.ensure(ne1 * nx * nx)); CU(r.invc.ensure(ns * nx * nx * 2)); CU(r.shift.ensure(2 * ns));
+    CU(r.index.ensure(ns)); CU(r.state_list.ensure(ns)); CU(r.env_list.ensure(ne1)); CU(r.state_pos.ensure(ne1)); CU(r.inv_base.ensure(ne1));
+    CU(r.counts.ensure(4)); CU(r.info.ensure(1)); CU(r.flags.ensure(ne1 * ni)); CU(r.np.ensure(ne1 * ni)); CU(r.flags_stage.ensure(ns * ni));
+    CU(r.np_stage.ensure(ns * ni));
+    if (!r.h_counts) CU(cudaHostAlloc(reinterpret_cast<void**>(&r.h_counts), 8 * sizeof(int), cudaHostAllocDefault));
+    std::vector<RadauEnv> h_env(ne1);
+    for (auto& e : h_env) radau_env_reset(e, h0);
+    CU(cudaMemcpy(r.env.p, h_env.data(), sizeof(RadauEnv) * ne1, cudaMemcpyHostToDevice));
+    r.n_env = n_env; r.max_rule = max_rule; r.s_max = int(s_max); r.h_max = h_max; r.tol_newton = tol_newton;
+    return PFC_OK;
+}
+
+static int radau_check(pfc_ctx* c, const char* who, int64_t n_env) {
+    if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, std::string(who) + ": pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
+    if (c->radau.n_env < 0) return fail(PFC_E_ARG, std::string(who) + ": pfc_radau_init first");
+    if (n_env != c->radau.n_env) return fail(PFC_E_ARG, std::string(who) + ": n_env differs from the one given to pfc_radau_init");
+    return PFC_OK;
+}
+
+// One accepted step for every environment.  Host round trips: one per attempt round (how many environments are pending) and one per Newton
+// iteration (how many stage states are still active); the error bits of every evaluation that counts ride along with them.
+static int radau_step_device(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
+    pfc_ctx::RadauState& r = c->radau;
+    const int nx = c->state.n_x, nv = c->state.nv, ni = c->scene.n_ins;
+    r.rounds = 0; r.syncs = 0;
+    for (double& v : r.ms) v = 0.0;
+    RadauBufs b{};
+    b.n_env = n_env; b.nx = nx; b.nv = nv; b.n_ins = ni; b.s_max = r.s_max; b.max_rule = r.max_rule; b.h_max = r.h_max; b.tol_newton = r.tol_newton;
+    b.env = r.env.p; b.x = x; b.tau = tau_ext; b.t = t; b.h_taken = h_taken; b.stats = stats;
+    b.X = r.X.p; b.Xp = r.Xp.p; b.Fp = r.Fp.p; b.taup = r.taup.p; b.xx0 = r.xx0.p; b.jac = r.jac.p; b.invc = r.invc.p; b.shift = r.shift.p;
+    b.index = r.index.p; b.state_list = r.state_list.p; b.env_list = r.env_list.p; b.state_pos = r.state_pos.p; b.inv_base = r.inv_base.p;
+    b.counts = r.counts.p; b.bodies = c->d_bodies.p; b.n_body = c->state.n_body;
+    // phase timing (pfc_set_timing): events around every phase, read after the step's last synchronisation
+    std::vector<std::pair<int, int>> marks;   // (phase, index of its start event; the end event follows)
+    std::vector<cudaEvent_t>& pool = r.ev_pool;
+    auto mark = [&](int phase, bool start) -> cudaError_t {
+        if (!c->timing) return cudaSuccess;
+        if (start) marks.push_back({phase, int(marks.size() * 2)});
+        const size_t k = marks.back().second + (start ? 0 : 1);
+        while (pool.size() <= k) { cudaEvent_t ev; cudaError_t e = cudaEventCreate(&ev); if (e != cudaSuccess) return e; pool.push_back(ev); }
+        return cudaEventRecord(pool[k], c->stream);
+    };
+    auto read_back = [&]() -> int {   // counts + status word to the host, one synchronisation; errors of the evaluations so far
+        CU(cudaMemcpyAsync(r.h_counts, r.counts.p, 4 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaMemcpyAsync(r.h_counts + 4, c->d_status.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        r.syncs += 1;
+        if (r.h_counts[4] & PFC_FLAG_NONFINITE) return fail(PFC_E_NONFINITE, "Non-finite vertex likely");
+        if (r.h_counts[4] & PFC_FLAG_OVERFLOW) return fail(PFC_E_CAPACITY, "candidate-pair capacity exceeded");
+        if (r.h_counts[2] & 2) return fail(PFC_E_STEP, "time step is too small, something is wrong");
+        if (r.h_counts[2] & 1) return fail(PFC_E_STEP, "unacceptable h");
+        return PFC_OK;
+    };
+    CU(status_begin(c));
+    CU(cudaMemsetAsync(r.counts.p, 0, 4 * sizeof(int), c->stream));
+    // calcJacobian! once per step: xx_0 and -J (a retry reuses them, radau_solve.jl:23-28)
+    CU(mark(0, true));
+    { const int rc = jacobian_device(c, n_env, x, tau_ext, r.jac.p, r.xx0.p, r.np.p, r.flags.p, nullptr); if (rc != PFC_OK) return rc; }
+    CU(launch_radau_prepare(b, r.flags.p, c->d_status.p, c->stream));
+    CU(mark(0, false));
+    c->launches += 1;
+    int mode = 2;
+    for (;;) {
+        CU(mark(3, true));
+        CU(launch_radau_plan(b, mode, c->stream));
+        CU(mark(3, false));
+        c->launches += 1;
+        { const int rc = read_back(); if (rc != PFC_OK) return rc; }
+        long long n_states = r.h_counts[0], n_active = r.h_counts[1];
+        if (n_states == 0) break;
+        r.rounds += 1;
+        mode = 1;
+        // updateInvC!: one matrix per (pending environment, stage of its rule)
+        CU(mark(2, true));
+        CU(launch_radau_inv_c(n_states, nx, r.jac.p, r.shift.p, r.index.p, r.invc.p, r.info.p, c->stream));
+        CU(mark(2, false));
+        c->launches += 1;
+        while (n_states > 0) {
+            CU(mark(1, true));
+            CU(launch_radau_gather(b, n_states, c->stream));
+            CU(cudaMemsetAsync(r.Fp.p, 0, sizeof(double) * size_t(n_states) * nx, c->stream));
+            { const int rc = calcxd_device(c, n_states, r.Xp.p, tau_ext ? r.taup.p : nullptr, r.Fp.p, r.np_stage.p, r.flags_stage.p, c->d_status.p); if (rc != PFC_OK) return rc; }
+            CU(mark(1, false));
+            CU(mark(3, true));
+            CU(launch_radau_newton(b, n_active, c->stream));
+            CU(launch_radau_plan(b, 0, c->stream));
+            CU(mark(3, false));
+            c->launches += 3;
+            { const int rc = read_back(); if (rc != PFC_OK) return rc; }
+            n_states = r.h_counts[0]; n_active = r.h_counts[1];
+        }
+        CU(mark(3, true));
+        CU(launch_radau_controller(b, c->stream));
+        CU(mark(3, false));
+        c->launches += 1;
+    }
+    for (const auto& m : marks) {
+        float ms = 0.0f;
+        CU(cudaEventElapsedTime(&ms, pool[m.second], pool[m.second + 1]));
+        r.ms[m.first] += ms;
+    }
+    return PFC_OK;
+}
+
+int pfc_radau_step_device(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
+    { const int rc = radau_check(c, "pfc_radau_step_device", n_env); if (rc != PFC_OK) return rc; }
+    if (n_env == 0) return PFC_OK;
+    if (!x || !t || !h_taken) return fail(PFC_E_ARG, "pfc_radau_step_device: NULL buffer");
+    CU(cudaSetDevice(c->device));
+    return radau_step_device(c, n_env, x, tau_ext, t, h_taken, stats);
+}
+
+int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
+    { const int rc = radau_check(c, "pfc_radau_step", n_env); if (rc != PFC_OK) return rc; }
+    if (n_env == 0) return PFC_OK;
+    if (!x || !t || !h_taken) return fail(PFC_E_ARG, "pfc_radau_step: NULL buffer");
+    CU(cudaSetDevice(c->device));
+    pfc_ctx::RadauState& r = c->radau;
+    const size_t ne = size_t(n_env), nx = size_t(c->state.n_x), nv = size_t(c->state.nv);
+    CU(r.x.ensure(ne * nx)); CU(r.t.ensure(ne)); CU(r.h.ensure(ne)); CU(r.stats.ensure(4 * ne));
+    if (tau_ext) CU(r.tau.ensure(std::max<size_t>(ne * nv, 1)));
+    CU(cudaMemcpyAsync(r.x.p, x, sizeof(double) * ne * nx, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(r.t.p, t, sizeof(double) * ne, cudaMemcpyHostToDevice, c->stream));
+    if (tau_ext) CU(cudaMemcpyAsync(r.tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
+    const int rc = radau_step_device(c, n_env, r.x.p, tau_ext ? r.tau.p : nullptr, r.t.p, r.h.p, r.stats.p);
+    if (rc != PFC_OK) { cudaStreamSynchronize(c->stream); return rc; }
+    CU(cudaMemcpyAsync(x, r.x.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(t, r.t.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(h_taken, r.h.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
+    if (stats) CU(cudaMemcpyAsync(stats, r.stats.p, sizeof(int32_t) * 4 * ne, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return PFC_OK;
+}
+
+int pfc_radau_step_info(pfc_ctx* c, double* ms, int64_t* counts) {
+    if (!c || c->radau.n_env < 0) return fail(PFC_E_ARG, "pfc_radau_step_info: pfc_radau_init first");
+    if (ms) for (int k = 0; k < 4; ++k) ms[k] = c->radau.ms[k];
+    if (counts) { counts[0] = c->radau.rounds; counts[1] = c->radau.syncs; }
     return PFC_OK;
 }
 

@@ -109,4 +109,41 @@ cudaError_t launch_refit(int kind, long long n_prim, long long n_node, const int
 // Batched updateInvC! of the Radau step (pfc_radau.cu): inv_c[m] = inverse((shift[m]) I + neg_J[index ? index[m] : m]), n x n complex, interleaved
 cudaError_t launch_radau_inv_c(long long n_mat, int n, const double* neg_J, const double* shift, const int* index, double* inv_c, int* info, cudaStream_t stream);
 
+// The adaptive Radau IIA step of a batch (pfc_radau.cu; per-environment arithmetic in pfc_radau_step.cuh).  A "state" is one (environment,
+// stage) pair of the current attempt; the packed arrays hold the states of the still-active environments in environment order.
+struct RadauEnv;
+struct RadauBufs {
+    long long n_env;
+    int nx, nv, n_ins, s_max, max_rule;
+    double h_max, tol_newton;
+    RadauEnv* env;              // [env] controller state
+    double* x;                  // [env][nx] the step's start state, overwritten by the accepted state
+    const double* tau;          // [env][nv] or nullptr
+    double* t;                  // [env]
+    double* h_taken;            // [env]
+    int* stats;                 // [env][4] or nullptr
+    double* X;                  // [env][s_max][nx] stage states
+    double* Xp; double* Fp;     // [state][nx] packed stage states / their derivatives
+    double* taup;               // [state][nv] (with tau)
+    const double* xx0;          // [env][nx] calcXd!(x)
+    double* jac;                // [env][nx][nx] d xdot / d x, negated in place into -J
+    double* invc;               // [matrix][nx][nx] complex: (h^-1 lambda_i I - J)^-1, matrices in the order of the round's plan
+    double* shift;              // [matrix][2]
+    int* index;                 // [matrix] environment
+    int* state_list;            // [state] env * 8 + stage
+    int* env_list;              // [active env]
+    int* state_pos;             // [env] first packed state of the environment in this iteration
+    int* inv_base;              // [env] first matrix of the environment in this round
+    int* counts;                // [4]: states, environments of the last plan / compaction; step-size error bits; spare
+    const BodyDev* bodies; int n_body;   // principal_value! of the floating bodies' MRPs
+};
+// mode 2: first round of a step (every environment pending), 1: a new attempt round of the pending environments (matrix list, attempt
+// reset), 0: compaction of the active environments between Newton iterations.  One CTA; writes counts[0..1].
+cudaError_t launch_radau_plan(const RadauBufs& b, int mode, cudaStream_t stream);
+// -J from the Jacobian in place, and the error bits of the Jacobian's flags [env][ins] into *status
+cudaError_t launch_radau_prepare(const RadauBufs& b, const int* flags, int* status, cudaStream_t stream);
+cudaError_t launch_radau_gather(const RadauBufs& b, long long n_states, cudaStream_t stream);
+cudaError_t launch_radau_newton(const RadauBufs& b, long long n_active, cudaStream_t stream);
+cudaError_t launch_radau_controller(const RadauBufs& b, cudaStream_t stream);
+
 }  // namespace pfc

@@ -8,9 +8,21 @@
 // partial (row) pivoting, the pivot search by one warp, the rank-1 update by all threads; the column permutation is undone at
 // the end.  Input is the REAL matrix -J shared by the stages of an environment plus the complex shift; output is interleaved
 // (re, im) row-major, which is the memory layout of a torch.complex128 / Julia ComplexF64 array.
+//
+// The rest of the file is the adaptive step around those inverses (solveRadau, radau_solve.jl:1-34, for a batch): per round of attempts
+// the plan kernel lists the pending environments' matrices and stage states; per Newton iteration the stage states of the still-active
+// environments are packed (gather), evaluated by calcXd! on the host side of the launch sequence, and radau_newton_kernel (one CTA per
+// active environment) does calcEw!, the mat-vecs with invC, updateStageX! and the convergence / divergence tests; radau_controller_kernel
+// (one thread per environment) applies calc_and_update_h! / update_rule! at the end of each round.
 #include <cuda_runtime.h>
 
+#include <algorithm>
+
+#include <cub/block/block_scan.cuh>
+
+#define PFC_RADAU_TABLE_STORAGE __constant__
 #include "pfc_launch.h"
+#include "pfc_radau_step.cuh"
 
 namespace pfc {
 
@@ -91,7 +103,230 @@ __global__ void __launch_bounds__(256) radau_inv_c_kernel(int n, const double* _
     if (threadIdx.x == 0 && singular && info) atomicOr(info, 1);
 }
 
+constexpr int kPlanThreads = 1024;
+
+__global__ void __launch_bounds__(kPlanThreads) radau_plan_kernel(RadauBufs b, int mode) {
+    using Scan = cub::BlockScan<int, kPlanThreads>;
+    __shared__ typename Scan::TempStorage tmp;
+    int base_s = 0, base_e = 0;
+    for (long long c0 = 0; c0 < b.n_env; c0 += kPlanThreads) {
+        const long long e = c0 + threadIdx.x;
+        int flag = 0, s = 0;
+        if (e < b.n_env) {
+            RadauEnv& en = b.env[e];
+            if (mode == 2) { en.pending = 1; en.n_rejected = 0; en.n_evals = 0; }
+            flag = mode == 0 ? en.active : en.pending;
+            s = flag ? 2 * en.rule - 1 : 0;
+        }
+        int ps, pe, agg_s, agg_e;
+        Scan(tmp).ExclusiveSum(s, ps, agg_s);
+        __syncthreads();
+        Scan(tmp).ExclusiveSum(flag, pe, agg_e);
+        __syncthreads();
+        if (flag) {
+            RadauEnv& en = b.env[e];
+            const int pos = base_s + ps;
+            b.env_list[base_e + pe] = (int)e;
+            b.state_pos[e] = pos;
+            for (int st = 0; st < s; ++st) b.state_list[pos + st] = (int)e * 8 + st;
+            if (mode != 0) {   // a new attempt: its matrices (h^-1 lambda_i I - J)^-1 and simple_newton!'s initial state
+                const RadauTableData& T = kRadauTables[en.rule - 1];
+                const double h_inv = 1.0 / en.h;
+                b.inv_base[e] = pos;
+                for (int st = 0; st < s; ++st) {
+                    b.index[pos + st] = (int)e;
+                    b.shift[2 * (pos + st)] = h_inv * T.lam_re[st];
+                    b.shift[2 * (pos + st) + 1] = h_inv * T.lam_im[st];
+                }
+                radau_attempt_begin(en);
+            }
+        }
+        base_s += agg_s;
+        base_e += agg_e;
+    }
+    if (threadIdx.x == 0) { b.counts[0] = base_s; b.counts[1] = base_e; }
+}
+
+__global__ void radau_prepare_kernel(RadauBufs b, const int* __restrict__ flags, int* __restrict__ status) {
+    const long long n = b.n_env * (long long)b.nx * b.nx, nf = b.n_env * (long long)b.n_ins;
+    int bad = 0;
+    for (long long id = blockIdx.x * (long long)blockDim.x + threadIdx.x; id < n; id += (long long)gridDim.x * blockDim.x) {
+        b.jac[id] = -b.jac[id];
+        if (id < nf) bad |= flags[id] & (2 | 8);   // PFC_FLAG_NONFINITE | PFC_FLAG_OVERFLOW
+    }
+    if (bad) atomicOr(status, bad);
+}
+
+// one CTA per packed state: its stage vector (x0 at the first iteration of an attempt, which also initialises the stage) and tau_ext
+__global__ void __launch_bounds__(64) radau_gather_kernel(RadauBufs b) {
+    const long long p = blockIdx.x;
+    const int code = b.state_list[p], e = code >> 3, st = code & 7;
+    const bool first = b.env[e].k_iter == 0;
+    double* Xs = b.X + ((long long)e * b.s_max + st) * b.nx;
+    const double* x0 = b.x + (long long)e * b.nx;
+    for (int n = threadIdx.x; n < b.nx; n += blockDim.x) {
+        const double v = first ? x0[n] : Xs[n];
+        if (first) Xs[n] = v;
+        b.Xp[p * b.nx + n] = v;
+    }
+    if (b.tau)
+        for (int n = threadIdx.x; n < b.nv; n += blockDim.x) b.taup[p * b.nv + n] = b.tau[(long long)e * b.nv + n];
+}
+
+// one Newton iteration of one environment (radau.py _simple_newton loop body); every element summed by one thread in a fixed order
+constexpr int kNewtonThreads = 128;
+__global__ void __launch_bounds__(kNewtonThreads) radau_newton_kernel(RadauBufs b) {
+    extern __shared__ __align__(16) double sm[];
+    __shared__ RadauEnv ctl;
+    __shared__ double red[kRadauMaxStage];
+    __shared__ unsigned div_mask;
+    __shared__ int decision;
+    const int e = b.env_list[blockIdx.x];
+    const int nx = b.nx;
+    if (threadIdx.x == 0) { ctl = b.env[e]; div_mask = 0u; }
+    __syncthreads();
+    const RadauTableData& T = kRadauTables[ctl.rule - 1];
+    const int s = T.s, sn = s * nx;
+    const double h = ctl.h, h_inv = 1.0 / h;
+    double* x0 = sm;
+    double* X = x0 + nx;
+    double* F = X + sn;
+    double* st = F + sn;
+    double* ar = st + sn;
+    double* ai = ar + sn;
+    double* br = ai + sn;
+    double* bi = br + sn;
+    const double* x0g = b.x + (long long)e * nx;
+    double* Xg = b.X + (long long)e * b.s_max * nx;
+    const double* Fg = b.Fp + (long long)b.state_pos[e] * nx;
+    const double* inv = b.invc + (long long)b.inv_base[e] * 2 * nx * nx;
+    for (int id = threadIdx.x; id < sn; id += blockDim.x) { X[id] = Xg[id]; F[id] = Fg[id]; }
+    for (int n = threadIdx.x; n < nx; n += blockDim.x) x0[n] = x0g[n];
+    __syncthreads();
+    for (int id = threadIdx.x; id < sn; id += blockDim.x) st[id] = radau_store(T, h, id / nx, id % nx, nx, x0, X, F);
+    __syncthreads();
+    if (threadIdx.x < s) {   // store_i . store_i
+        double a = 0.0;
+        for (int n = 0; n < nx; ++n) a = a + st[threadIdx.x * nx + n] * st[threadIdx.x * nx + n];
+        red[threadIdx.x] = a;
+    }
+    for (int id = threadIdx.x; id < sn; id += blockDim.x) radau_ew(T, h_inv, id / nx, id % nx, nx, st, &ar[id], &ai[id]);
+    __syncthreads();
+    for (int id = threadIdx.x; id < sn; id += blockDim.x) {
+        const int i = id / nx;
+        radau_matvec_row(inv + (long long)i * 2 * nx * nx, nx, id % nx, ar + i * nx, ai + i * nx, &br[id], &bi[id]);
+    }
+    __syncthreads();
+    unsigned mask = 0u;
+    for (int id = threadIdx.x; id < sn; id += blockDim.x) {
+        const double u = radau_update(T, id / nx, id % nx, nx, br, bi);
+        st[id] = u;
+        if (fabs(u) > 1.0e1) mask |= 1u << (id / nx);
+    }
+    if (mask) atomicOr(&div_mask, mask);
+    __syncthreads();
+    // updateStageX!: stages in order up to the first whose update exceeds 10
+    const int first_div = div_mask ? __ffs(div_mask) - 1 : s;
+    for (int id = threadIdx.x; id < first_div * nx; id += blockDim.x) { X[id] = X[id] - st[id]; Xg[id] = X[id]; }
+    if (threadIdx.x == 0) {
+        double residual = 0.0;
+        for (int i = 0; i < s; ++i) residual += red[i];
+        ctl.n_evals += s;
+        decision = radau_newton_decide(ctl, ctl.k_iter + 1, residual, div_mask != 0u, b.tol_newton);
+    }
+    __syncthreads();
+    if (decision == kRadauConverged) {   // update_x_err_norm! with this iteration's F, the updated last stage and invC of stage 0
+        const double* xx0 = b.xx0 + (long long)e * nx;
+        for (int n = threadIdx.x; n < nx; n += blockDim.x) ar[n] = radau_err_d(T, h, n, nx, xx0, F);
+        __syncthreads();
+        for (int r = threadIdx.x; r < nx; r += blockDim.x) ai[r] = radau_err_term(inv, nx, r, ar, X[(s - 1) * nx + r], x0[r]);
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            double a = 0.0;
+            for (int r = 0; r < nx; ++r) a = a + ai[r];
+            ctl.err_norm = sqrt(a / nx);
+        }
+    }
+    if (threadIdx.x == 0) {
+        if (decision != kRadauIterate) ctl.active = 0;
+        b.env[e] = ctl;
+    }
+}
+
+// calc_and_update_h! / update_rule! of every environment whose attempt just ended; principal_value! on acceptance
+__global__ void __launch_bounds__(128) radau_controller_kernel(RadauBufs b) {
+    const long long e = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (e >= b.n_env) return;
+    RadauEnv ctl = b.env[e];
+    if (!ctl.pending) return;
+    const int s = 2 * ctl.rule - 1, k = ctl.k_iter;
+    double h_taken = 0.0;
+    const int rc = radau_control(ctl, b.max_rule, b.h_max, &h_taken);
+    if (rc == kRadauAccepted) {
+        double* x = b.x + e * b.nx;
+        const double* Xl = b.X + (e * b.s_max + (s - 1)) * b.nx;
+        for (int n = 0; n < b.nx; ++n) x[n] = Xl[n];
+        for (int k2 = 0; k2 < b.n_body; ++k2) {
+            if (b.bodies[k2].joint != 1) continue;
+            double* p = x + b.bodies[k2].q0;
+            const double n2 = p[0] * p[0] + p[1] * p[1] + p[2] * p[2];
+            if (n2 > 1.0) { p[0] = -p[0] / n2; p[1] = -p[1] / n2; p[2] = -p[2] / n2; }
+        }
+        b.t[e] = b.t[e] + h_taken;
+        b.h_taken[e] = h_taken;
+        if (b.stats) { int* o = b.stats + 4 * e; o[0] = s; o[1] = k; o[2] = ctl.n_rejected; o[3] = ctl.n_evals; }
+        ctl.pending = 0;
+    } else if (rc == kRadauRetry) {
+        ctl.n_rejected += 1;
+    } else {
+        atomicOr(b.counts + 2, rc == kRadauBadH ? 1 : 2);
+        ctl.pending = 0;
+    }
+    b.env[e] = ctl;
+}
+
 }  // namespace
+
+cudaError_t launch_radau_plan(const RadauBufs& b, int mode, cudaStream_t stream) {
+    radau_plan_kernel<<<1, kPlanThreads, 0, stream>>>(b, mode);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_radau_prepare(const RadauBufs& b, const int* flags, int* status, cudaStream_t stream) {
+    const long long n = b.n_env * (long long)b.nx * b.nx;
+    const long long blocks = std::min<long long>((n + 255) / 256, 148 * 16);
+    radau_prepare_kernel<<<(unsigned)std::max<long long>(blocks, 1), 256, 0, stream>>>(b, flags, status);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_radau_gather(const RadauBufs& b, long long n_states, cudaStream_t stream) {
+    if (n_states == 0) return cudaSuccess;
+    radau_gather_kernel<<<(unsigned)n_states, 64, 0, stream>>>(b);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_radau_newton(const RadauBufs& b, long long n_active, cudaStream_t stream) {
+    if (n_active == 0) return cudaSuccess;
+    const size_t smem = sizeof(double) * ((size_t)b.nx + 7 * (size_t)b.s_max * b.nx);
+    {
+        struct Tag {};
+        std::lock_guard<std::mutex> g(launch_mutex());
+        LaunchSlot& sl = launch_slot<Tag>();
+        if (smem > sl.smem) {
+            cudaError_t e = cudaFuncSetAttribute(radau_newton_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+            if (e != cudaSuccess) return e;
+            sl.smem = smem;
+        }
+    }
+    radau_newton_kernel<<<(unsigned)n_active, kNewtonThreads, smem, stream>>>(b);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_radau_controller(const RadauBufs& b, cudaStream_t stream) {
+    if (b.n_env == 0) return cudaSuccess;
+    radau_controller_kernel<<<(unsigned)((b.n_env + 127) / 128), 128, 0, stream>>>(b);
+    return cudaGetLastError();
+}
 
 cudaError_t launch_radau_inv_c(long long n_mat, int n, const double* neg_J, const double* shift, const int* index, double* inv_c, int* info, cudaStream_t stream) {
     if (n_mat == 0) return cudaSuccess;

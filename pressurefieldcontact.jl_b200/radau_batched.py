@@ -12,7 +12,11 @@ What runs where
     library's stream (radau_solve.jl:36-99, adaptive.jl) -- every environment follows exactly the decision sequence the
     single-scene integrator would take for it; environments that fail a step retry with their own smaller h while the others wait.
 
-The integrator is caller-side code (the reference's is Julia); it exists to drive the device path end to end the way
+DeviceBatchedRadau is the same integrator behind the library's C ABI (pfc_radau_init / pfc_radau_step_device): the Newton iteration,
+error estimate and step-size / order control run in CUDA kernels, and the host only reads how many stage states are still active once per
+Newton iteration.  It has BatchedRadau's interface (step, integrate, t) so that the tests and scripts/run_batched_radau.py drive both.
+
+BatchedRadau is caller-side code (the reference's is Julia); it exists to drive the device path end to end the way
 integrate_scenario_radau does and to measure batched roll-out throughput.
 """
 from __future__ import annotations
@@ -23,7 +27,7 @@ import torch
 from . import radau as R
 from . import scenario as S
 
-__all__ = ["BatchedRadau"]
+__all__ = ["BatchedRadau", "DeviceBatchedRadau"]
 
 
 class BatchedRadau:
@@ -211,6 +215,46 @@ class BatchedRadau:
             ts, xs = [self.t.cpu().numpy().copy()], [x.cpu().numpy().copy()]
             for _ in range(n_steps):
                 x, _ = self.step(x)
+                ts.append(self.t.cpu().numpy().copy())
+                xs.append(x.cpu().numpy().copy())
+        return np.array(ts), np.array(xs)
+
+
+class DeviceBatchedRadau:
+    """The batched adaptive Radau step of pfc_radau_step_device: same step(x0) -> (x_final, h_taken) / integrate(x0, n_steps) / t as
+    BatchedRadau, over torch tensors on the library's stream.  tau_ext [E, nv] (or None) is held constant over each step."""
+
+    def __init__(self, m, n_env: int, device_index: int = 0, NR: int = 2, tol_newton: float = 1.0e-16, h0: float = 1.0e-4, h_max: float = 0.01):
+        if not getattr(m, "device_dynamics", False):
+            raise RuntimeError("DeviceBatchedRadau needs a CUDA backend with pfc_set_dynamics (floating bodies with InertiaProperties)")
+        self.m, self.ctx, self.E, self.NX, self.NR = m, m.backend, n_env, S.num_x(m), NR
+        self.dev = torch.device("cuda", device_index)
+        self.stream = torch.cuda.ExternalStream(self.ctx.stream, device=self.dev)
+        self.ctx.radau_init(n_env, NR, h0, h_max, tol_newton)
+        with torch.cuda.stream(self.stream):
+            self.t = torch.zeros(n_env, dtype=torch.float64, device=self.dev)
+            self.stats = torch.zeros((n_env, 4), dtype=torch.int32, device=self.dev)
+
+    def step(self, x0: torch.Tensor, tau_ext: torch.Tensor = None):
+        """solveRadau for the batch: returns (x_final [E, NX], h_taken [E]); self.t advances by h_taken; self.stats [E, 4] as pfc_radau_step."""
+        with torch.cuda.stream(self.stream):
+            x = x0.to(device=self.dev, dtype=torch.float64).contiguous().clone()
+            tau = None if tau_ext is None else tau_ext.to(device=self.dev, dtype=torch.float64).contiguous()
+            t = self.t.clone()
+            h_taken = torch.zeros(self.E, dtype=torch.float64, device=self.dev)
+            self.ctx.radau_step_device(self.E, x.data_ptr(), None if tau is None else tau.data_ptr(), t.data_ptr(), h_taken.data_ptr(),
+                                       self.stats.data_ptr())
+            self.t = t
+            return x, h_taken
+
+    def integrate(self, x0, n_steps: int, tau_ext=None):
+        """n_steps accepted steps for every environment; returns (times [n_steps + 1, E], states [n_steps + 1, E, NX]) on the host."""
+        with torch.cuda.stream(self.stream):
+            x = torch.as_tensor(np.asarray(x0, dtype=np.float64)).to(self.dev).reshape(self.E, self.NX)
+            tau = None if tau_ext is None else torch.as_tensor(np.asarray(tau_ext, dtype=np.float64)).to(self.dev)
+            ts, xs = [self.t.cpu().numpy().copy()], [x.cpu().numpy().copy()]
+            for _ in range(n_steps):
+                x, _ = self.step(x, tau)
                 ts.append(self.t.cpu().numpy().copy())
                 xs.append(x.cpu().numpy().copy())
         return np.array(ts), np.array(xs)

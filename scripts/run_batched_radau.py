@@ -1,7 +1,13 @@
 #!/usr/bin/env python
 """Batched roll-out: n_env independent test/boxes.jl scenes advanced by the reference's adaptive Radau IIA scheme with every array on
-the GPU (pfc_b200.radau_batched).  Prints one JSON line: environment-steps per second, the split between Jacobian chunks, stage
-evaluations and the rest, and the CPU oracle's single-scene rate for the same integrator (one scene, one thread) for scale."""
+the GPU (pfc_b200.radau_batched).  Prints one JSON line.
+
+  --impl torch   (default) BatchedRadau, the Newton loop as torch ops between library calls: environment-steps per second, the split
+                 between Jacobian chunks, stage evaluations and the rest, and the CPU oracle's single-scene rate for scale.
+  --impl device  DeviceBatchedRadau, the whole step behind pfc_radau_step_device.
+  --impl both    both paths on the same seeded states after the same warm-up: per path ms per batched step, env-steps/s, stage states
+                 per environment per step, attempt rounds and host synchronisations per step; the device path's time split (CUDA events
+                 inside the library, in a separate pass); how far the two paths agree over the timed steps; the card and its power limit."""
 import argparse
 import json
 import os
@@ -21,7 +27,10 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--cpu-steps", type=int, default=10)
+    ap.add_argument("--impl", choices=("torch", "device", "both"), default="torch")
     args = ap.parse_args()
+    if args.impl != "torch":
+        return compare(args)
     import torch
     import pfc_b200  # noqa: F401
     from helpers import boxes_env_states, scene_boxes
@@ -89,6 +98,92 @@ def main():
     out["cpu_oracle_contact_only_env_steps_per_sec_estimate"] = 1.0 / ((rr.n_de_float + 7 * rr.n_de_chunk) / args.cpu_steps * 60e-6)
     out["note"] = "the CPU figures are one scene on one thread: the Python mirror (dominated by interpreter overhead) and an estimate from the " \
                   "oracle's measured 60 us per contact evaluation (Dual-6 chunk ~ 7x) ignoring rigid-body and linear-algebra time"
+    print(json.dumps(out))
+
+
+def _card():
+    import subprocess
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit", "--format=csv,noheader", "-i", "0"], capture_output=True, text=True)
+    return q.stdout.strip()
+
+
+def compare(args):
+    import torch
+    import pfc_b200  # noqa: F401
+    from helpers import boxes_env_states, scene_boxes
+    from pfc_b200 import capi
+    from pfc_b200.radau_batched import BatchedRadau, DeviceBatchedRadau
+
+    n_env, K = args.envs, args.steps
+    paths = ("torch", "device") if args.impl == "both" else ("device",)
+    m = scene_boxes(capi.Context(0), max_env=3 * n_env)[0]
+    x0 = boxes_env_states(m, n_env)
+    out = {"scene": "C3 batch of test/boxes.jl", "n_env": n_env, "h_max": 0.05, "warmup_steps": args.warmup, "timed_steps": K, "card": _card()}
+    runs = {}
+    for name in paths:
+        r = (BatchedRadau if name == "torch" else DeviceBatchedRadau)(m, n_env, h_max=0.05)
+        syncs = [0]
+        if name == "torch":   # host synchronisations of the eager loop: bool() of a device tensor, nonzero(), tolist()
+            real_bool, real_nonzero, real_tolist = torch.Tensor.__bool__, torch.nonzero, torch.Tensor.tolist
+
+            def counted(f):
+                def g(*a, **k):
+                    syncs[0] += 1
+                    return f(*a, **k)
+                return g
+        with torch.cuda.stream(r.stream):
+            x = torch.as_tensor(x0).to(r.dev)
+            for _ in range(args.warmup):
+                x, _ = r.step(x)
+            m.backend.sync()
+            c0, a0 = (r.n_calcxd_states, r.n_attempts) if name == "torch" else (0, 0)
+            hs, xs, evals, rounds = [], [], 0, 0
+            if name == "torch":
+                torch.Tensor.__bool__, torch.nonzero, torch.Tensor.tolist = counted(real_bool), counted(real_nonzero), counted(real_tolist)
+            try:
+                t0 = time.perf_counter()
+                for _ in range(K):
+                    x, h = r.step(x)
+                    hs.append(h)
+                    xs.append(x)
+                    if name == "device":
+                        evals = evals + r.stats[:, 3].sum(dtype=torch.int64)    # stays on the device: no read-back in the timed loop
+                        _, nr, ns = m.backend.radau_step_info()
+                        rounds += nr
+                        syncs[0] += ns
+                m.backend.sync()
+                wall = time.perf_counter() - t0
+            finally:
+                if name == "torch":
+                    torch.Tensor.__bool__, torch.nonzero, torch.Tensor.tolist = real_bool, real_nonzero, real_tolist
+            rec = {"ms_per_batched_step": wall / K * 1e3, "env_steps_per_sec": n_env * K / wall,
+                   "host_synchronisations_per_step": syncs[0] / K}
+            if name == "torch":
+                rec["stage_states_per_env_per_step"] = (r.n_calcxd_states - c0) / (n_env * K)
+                rec["attempt_rounds_per_step"] = (r.n_attempts - a0) / K
+            else:
+                rec["stage_states_per_env_per_step"] = int(evals) / (n_env * K)
+                rec["attempt_rounds_per_step"] = rounds / K
+                # the time split: CUDA events between the library's phases, in a separate pass of K steps (timing on)
+                m.backend.set_timing(True)
+                split = np.zeros(4)
+                xt = x.clone()
+                for _ in range(K):
+                    xt, _ = r.step(xt)
+                    split += m.backend.radau_step_info()[0]
+                m.backend.set_timing(False)
+                rec["device_ms_per_step"] = dict(zip(("jacobian", "stage_evaluations", "inverses", "newton_and_controller"), (split / K).tolist()))
+            runs[name] = (torch.stack(hs).cpu().numpy(), torch.stack(xs).cpu().numpy())
+        out[name] = rec
+    if len(paths) == 2:
+        (h_t, x_t), (h_d, x_d) = runs["torch"], runs["device"]
+        differ = (np.abs(h_d - h_t) > 1e-6 * h_t).any(axis=0)    # a different decision shows as a factor 0.1 or 2 in h
+        ok = ~differ
+        v_t, v_d = x_t[:, ok].reshape(K, ok.sum(), -1, 3), x_d[:, ok].reshape(K, ok.sum(), -1, 3)
+        den = np.maximum(np.abs(v_t).max(axis=3), 1e-6 * np.abs(v_t).max(axis=(2, 3))[:, :, None])
+        out["agreement"] = {"environments_with_different_decisions": int(differ.sum()),
+                            "max_relative_state_difference_per_3_vector": float((np.abs(v_d - v_t).max(axis=3) / den).max()),
+                            "max_relative_h_difference": float((np.abs(h_d - h_t) / h_t)[:, ok].max())}
     print(json.dumps(out))
 
 
