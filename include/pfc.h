@@ -170,9 +170,27 @@ int pfc_radau_init(pfc_ctx* ctx, int64_t n_env, int max_rule, double h0, double 
 int pfc_radau_step_device(pfc_ctx* ctx, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats);
 /* Same on host pointers (copies in and out are part of the call). */
 int pfc_radau_step(pfc_ctx* ctx, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats);
-/* Of the last pfc_radau_step[_device] call: counts[0] = rounds of attempts, counts[1] = host synchronisations; ms[0..3] = device time of
- * the Jacobian, the stage evaluations, the inverses, and the Newton + controller kernels (CUDA events; zeros unless pfc_set_timing is on).
- * Either pointer may be NULL. */
+/* A roll-out with a piecewise-constant tau_ext: every environment is advanced through the knot times t_knot[0..n_knot) (a HOST array,
+ * shared by the batch, strictly increasing with gaps of at least h_min = 1e-8; t_knot[0] - t[env] >= h_min), tau_ext[k][env][nv] (or NULL)
+ * acting on (t_knot[k-1], t_knot[k]].  Steps are pfc_radau_step's, from the controller state the context keeps, with one rule at the knots:
+ * when h >= (t_knot[k] - t) - h_min the step is a knot step of exactly t_knot[k] - t (a rejected one retries with a smaller, ordinary h);
+ * once accepted, t = t_knot[k] exactly, x (after principal_value!) is written to x_knot[k][env] (or nowhere if x_knot is NULL), and a
+ * controller proposal of at least the knot step's h is raised back to the h the knot step replaced.  So no ordinary step leaves less than
+ * h_min to a knot, and a roll-out through K knots equals K roll-outs through one knot each, bit for bit.  Environments go through their
+ * knots independently; a round of steps takes the Jacobian of the environments still under way only.  max_steps >= 1 bounds each
+ * environment's accepted steps: one that exhausts it stops where it is, its unreached x_knot rows are NaN, and the call returns PFC_OK.
+ * x[env][n_x] and t[env] in/out; stats[env][4] (or NULL) = {knots reached, accepted steps, rejected attempts, stage evaluations} of the call.
+ * PFC_E_ARG (nothing modified) for a bad knot array, max_steps < 1, an n_env other than pfc_radau_init's, or an environment that starts
+ * less than h_min before t_knot[0] (checked on the device before the first step); otherwise the errors of pfc_radau_step.  Device pointers
+ * except t_knot; one more host synchronisation per round of steps. */
+int pfc_radau_rollout_device(pfc_ctx* ctx, int64_t n_env, int n_knot, const double* t_knot, int64_t max_steps, double* x, const double* tau_ext,
+                             double* t, double* x_knot, int32_t* stats);
+/* Same on host pointers. */
+int pfc_radau_rollout(pfc_ctx* ctx, int64_t n_env, int n_knot, const double* t_knot, int64_t max_steps, double* x, const double* tau_ext, double* t,
+                      double* x_knot, int32_t* stats);
+/* Of the last pfc_radau_step[_device] or pfc_radau_rollout[_device] call (sums over a roll-out's steps): counts[0] = rounds of attempts,
+ * counts[1] = host synchronisations; ms[0..3] = device time of the Jacobian, the stage evaluations, the inverses, and the Newton +
+ * controller kernels (CUDA events; zeros unless pfc_set_timing is on).  Either pointer may be NULL. */
 int pfc_radau_step_info(pfc_ctx* ctx, double* ms, int64_t* counts);
 /* Debug / parity: the boundary arrays (X_r2_r1, twist_r2) the prologue computed and the per-instruction wrenches of the last
  * host-pointer evaluation; any pointer may be NULL. */

@@ -239,6 +239,20 @@ function radau_step_batch_gpu!(m::MechanismScenario, x::Matrix{Float64}, t::Vect
     return stats
 end
 
+"Every environment `x[:, env]` from `t[env]` through the shared knot times `t_knot` (pfc_radau_rollout, host arrays): `tau_ext[:, env, k]`
+acts on `(t_knot[k-1], t_knot[k]]`, `x_knot[:, env, k]` gets the state at knot k (NaN if the environment ran out of `max_steps` accepted
+steps first), `x` and `t` advance in place.  Returns `stats[:, env]` = knots reached, accepted steps, rejected attempts, stage evaluations.
+Written against include/pfc.h; not run (no Julia in the build environment)."
+function radau_rollout_batch_gpu!(m::MechanismScenario, x::Matrix{Float64}, t::Vector{Float64}, t_knot::Vector{Float64},
+                                  x_knot::Array{Float64,3}; tau_ext::Union{Nothing,Array{Float64,3}} = nothing, max_steps::Integer = 1000)
+    stats = zeros(Int32, 4, size(x, 2))
+    tau = tau_ext === nothing ? C_NULL : tau_ext
+    GC.@preserve x t t_knot x_knot tau_ext stats check(ccall((:pfc_radau_rollout, LIB), Cint,
+        (Ptr{Cvoid}, Int64, Cint, Ptr{Float64}, Int64, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+        CTX[m], size(x, 2), length(t_knot), t_knot, max_steps, x, tau, t, x_knot, stats))
+    return stats
+end
+
 "Moved vertices of mesh `id` (same connectivity): the device rebuilds the mesh's primitive records and refits its tree (pfc_refit_mesh)."
 function refit_mesh_gpu!(m::MechanismScenario, id::MeshID, point::Vector{SVector{3,Float64}})
     xyz = collect(Iterators.flatten(point))

@@ -22,7 +22,7 @@ _vp = C.c_void_p
 SYMBOLS = [
     "pfc_create", "pfc_destroy", "pfc_add_mesh", "pfc_add_instruction", "pfc_finalize", "pfc_eval_f64", "pfc_eval_f64_device",
     "pfc_eval_dual6", "pfc_set_debug", "pfc_get_pairs", "pfc_get_traction", "pfc_set_shard", "pfc_eval_sharded_begin", "pfc_eval_sharded_partials", "pfc_eval_sharded_step", "pfc_sync", "pfc_stream",
-    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
+    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_rollout", "pfc_radau_rollout_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
     "pfc_comm_unique_id", "pfc_comm_init_rank", "pfc_eval_sharded_f64_device", "pfc_group_create", "pfc_group_destroy", "pfc_group_size", "pfc_group_ctx",
     "pfc_group_add_mesh", "pfc_group_add_instruction", "pfc_group_finalize", "pfc_group_eval_f64",
 ]
@@ -73,6 +73,8 @@ def lib():
         L.pfc_radau_init.argtypes = [_vp, C.c_int64, C.c_int, C.c_double, C.c_double, C.c_double]
         L.pfc_radau_step.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
         L.pfc_radau_step_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
+        L.pfc_radau_rollout.argtypes = [_vp, C.c_int64, C.c_int, _d, C.c_int64, _vp, _vp, _vp, _vp, _vp]
+        L.pfc_radau_rollout_device.argtypes = [_vp, C.c_int64, C.c_int, _d, C.c_int64, _vp, _vp, _vp, _vp, _vp]
         L.pfc_radau_step_info.argtypes = [_vp, _vp, _vp]
         L.pfc_comm_unique_id.argtypes = [_vp]
         L.pfc_comm_init_rank.argtypes = [_vp, _vp, C.c_int, C.c_int]
@@ -291,9 +293,28 @@ class Context:
         """Device pointers given as integers (tau_ext / stats may be None); on self.stream."""
         _check(lib().pfc_radau_step_device(self._h, n_env, x, tau_ext, t, h_taken, stats))
 
+    def radau_rollout(self, x, t, t_knot, tau_ext=None, max_steps=1000):
+        """Every environment through the knot times t_knot [n_knot] (host arrays): tau_ext [n_knot][env][nv] or None ->
+        (x [env][n_x], t [env], x_knot [n_knot][env][n_x] (NaN rows for knots not reached), stats [env][4])."""
+        nx = self.nq + self.nv + 6 * self.n_bristle
+        x = _a(x).reshape(-1, nx).copy()
+        n_env = x.shape[0]
+        t = _a(t).reshape(n_env).copy()
+        t_knot = _a(t_knot).reshape(-1)
+        tau = None if tau_ext is None else _a(tau_ext).reshape(t_knot.shape[0], n_env, self.nv)
+        x_knot = np.zeros((t_knot.shape[0], n_env, nx))
+        stats = np.zeros((n_env, 4), np.int32)
+        _check(lib().pfc_radau_rollout(self._h, n_env, t_knot.shape[0], t_knot, int(max_steps), _p(x), _p(tau), _p(t), _p(x_knot), _p(stats)))
+        return x, t, x_knot, stats
+
+    def radau_rollout_device(self, n_env, t_knot, max_steps, x, tau_ext, t, x_knot, stats):
+        """t_knot is a host array; the rest are device pointers given as integers (tau_ext / x_knot / stats may be None); on self.stream."""
+        t_knot = _a(t_knot).reshape(-1)
+        _check(lib().pfc_radau_rollout_device(self._h, n_env, t_knot.shape[0], t_knot, int(max_steps), x, tau_ext, t, x_knot, stats))
+
     def radau_step_info(self):
         """(ms [Jacobian, stage evaluations, inverses, Newton + controller] -- needs set_timing(True) --, rounds, host synchronisations)
-        of the last Radau step."""
+        of the last Radau step or roll-out (sums over its steps)."""
         ms = np.zeros(4)
         counts = np.zeros(2, np.int64)
         _check(lib().pfc_radau_step_info(self._h, _p(ms), _p(counts)))

@@ -232,9 +232,13 @@ struct pfc_ctx {
         DevBuf<double> X, Xp, Fp, taup, xx0, jac, invc, shift, x, tau, t, h;
         DevBuf<int> index, state_list, env_list, state_pos, inv_base, counts, stats, flags, flags_stage, info;
         DevBuf<long long> np, np_stage;
-        int* h_counts = nullptr;   // pinned: counts[0..3] + the status word
-        int64_t rounds = 0, syncs = 0;   // of the last step
-        double ms[4] = {0, 0, 0, 0};     // of the last step with pfc_set_timing on: Jacobian, stage evaluations, inverses, Newton + controller
+        // roll-outs (pfc_radau_rollout): grown on first use
+        DevBuf<RadauEnv> env_c;
+        DevBuf<double> knots, x_c, tau_c, t_c, h_c, h_save, x_knot;
+        DevBuf<int> knot, steps, ro_stats, list, stats_c, ro_count;
+        int* h_counts = nullptr;   // pinned: counts[0..3] + the status word; [5..6] a roll-out's ro_count
+        int64_t rounds = 0, syncs = 0;   // of the last step or roll-out
+        double ms[4] = {0, 0, 0, 0};     // of the last step or roll-out with pfc_set_timing on: Jacobian, stage evaluations, inverses, Newton + controller
         std::vector<cudaEvent_t> ev_pool;
     } radau;
     bool timing = false;
@@ -1803,16 +1807,21 @@ static int radau_check(pfc_ctx* c, const char* who, int64_t n_env) {
     return PFC_OK;
 }
 
-// One accepted step for every environment.  Host round trips: one per attempt round (how many environments are pending) and one per Newton
-// iteration (how many stage states are still active); the error bits of every evaluation that counts ride along with them.
-static int radau_step_device(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
-    pfc_ctx::RadauState& r = c->radau;
-    const int nx = c->state.n_x, nv = c->state.nv, ni = c->scene.n_ins;
+static void radau_info_reset(pfc_ctx::RadauState& r) {
     r.rounds = 0; r.syncs = 0;
     for (double& v : r.ms) v = 0.0;
+}
+
+// One accepted step for every environment.  Host round trips: one per attempt round (how many environments are pending) and one per Newton
+// iteration (how many stage states are still active); the error bits of every evaluation that counts ride along with them.
+// The buffer set is the caller's: the context's own for pfc_radau_step, the compact sub-batch of a roll-out round; the work space is sized
+// for pfc_radau_init's n_env, which n_env never exceeds.  The step info (rounds, synchronisations, phase times) is added to.
+static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
+    pfc_ctx::RadauState& r = c->radau;
+    const int nx = c->state.n_x, nv = c->state.nv, ni = c->scene.n_ins;
     RadauBufs b{};
     b.n_env = n_env; b.nx = nx; b.nv = nv; b.n_ins = ni; b.s_max = r.s_max; b.max_rule = r.max_rule; b.h_max = r.h_max; b.tol_newton = r.tol_newton;
-    b.env = r.env.p; b.x = x; b.tau = tau_ext; b.t = t; b.h_taken = h_taken; b.stats = stats;
+    b.env = env; b.x = x; b.tau = tau_ext; b.t = t; b.h_taken = h_taken; b.stats = stats;
     b.X = r.X.p; b.Xp = r.Xp.p; b.Fp = r.Fp.p; b.taup = r.taup.p; b.xx0 = r.xx0.p; b.jac = r.jac.p; b.invc = r.invc.p; b.shift = r.shift.p;
     b.index = r.index.p; b.state_list = r.state_list.p; b.env_list = r.env_list.p; b.state_pos = r.state_pos.p; b.inv_base = r.inv_base.p;
     b.counts = r.counts.p; b.bodies = c->d_bodies.p; b.n_body = c->state.n_body;
@@ -1893,7 +1902,8 @@ int pfc_radau_step_device(pfc_ctx* c, int64_t n_env, double* x, const double* ta
     if (n_env == 0) return PFC_OK;
     if (!x || !t || !h_taken) return fail(PFC_E_ARG, "pfc_radau_step_device: NULL buffer");
     CU(cudaSetDevice(c->device));
-    return radau_step_device(c, n_env, x, tau_ext, t, h_taken, stats);
+    radau_info_reset(c->radau);
+    return radau_step_device(c, n_env, c->radau.env.p, x, tau_ext, t, h_taken, stats);
 }
 
 int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
@@ -1908,11 +1918,95 @@ int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, 
     CU(cudaMemcpyAsync(r.x.p, x, sizeof(double) * ne * nx, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemcpyAsync(r.t.p, t, sizeof(double) * ne, cudaMemcpyHostToDevice, c->stream));
     if (tau_ext) CU(cudaMemcpyAsync(r.tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
-    const int rc = radau_step_device(c, n_env, r.x.p, tau_ext ? r.tau.p : nullptr, r.t.p, r.h.p, r.stats.p);
+    radau_info_reset(r);
+    const int rc = radau_step_device(c, n_env, r.env.p, r.x.p, tau_ext ? r.tau.p : nullptr, r.t.p, r.h.p, r.stats.p);
     if (rc != PFC_OK) { cudaStreamSynchronize(c->stream); return rc; }
     CU(cudaMemcpyAsync(x, r.x.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(t, r.t.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(h_taken, r.h.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
+    if (stats) CU(cudaMemcpyAsync(stats, r.stats.p, sizeof(int32_t) * 4 * ne, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    return PFC_OK;
+}
+
+// ---- roll-outs through shared knot times: rounds of one step for every environment with a knot ahead and steps left ---------------
+static int radau_rollout_check(pfc_ctx* c, const char* who, int64_t n_env, int n_knot, const double* t_knot, int64_t max_steps) {
+    { const int rc = radau_check(c, who, n_env); if (rc != PFC_OK) return rc; }
+    if (n_knot < 1 || !t_knot) return fail(PFC_E_ARG, std::string(who) + ": at least one knot time");
+    for (int k = 0; k < n_knot; ++k) {
+        if (!std::isfinite(t_knot[k])) return fail(PFC_E_ARG, std::string(who) + ": non-finite knot time");
+        if (k > 0 && !(t_knot[k] - t_knot[k - 1] >= kRadauHMin)) return fail(PFC_E_ARG, std::string(who) + ": knot times must increase by at least h_min = 1e-8");
+    }
+    if (max_steps < 1) return fail(PFC_E_ARG, std::string(who) + ": max_steps must be at least 1");
+    return PFC_OK;
+}
+
+// Host round trips: one per round (how many environments take a step), besides the step's own.  The first selection also checks every
+// environment's distance to knot 0, before anything the caller sees is written.
+static int radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const double* t_knot, int64_t max_steps, double* x, const double* tau_ext,
+                                double* t, double* x_knot, int32_t* stats) {
+    pfc_ctx::RadauState& r = c->radau;
+    const size_t ne = size_t(n_env), nx = size_t(c->state.n_x), nv = size_t(c->state.nv);
+    CU(r.knots.ensure(size_t(n_knot))); CU(r.knot.ensure(ne)); CU(r.steps.ensure(ne)); CU(r.ro_stats.ensure(4 * ne)); CU(r.list.ensure(ne));
+    CU(r.env_c.ensure(ne)); CU(r.x_c.ensure(ne * nx)); CU(r.tau_c.ensure(ne * std::max<size_t>(nv, 1))); CU(r.t_c.ensure(ne)); CU(r.h_c.ensure(ne));
+    CU(r.h_save.ensure(ne)); CU(r.stats_c.ensure(4 * ne)); CU(r.ro_count.ensure(2));
+    RadauRolloutBufs b{};
+    b.n_env = n_env; b.max_steps = max_steps; b.nx = int(nx); b.nv = int(nv); b.n_knot = n_knot;
+    b.knots = r.knots.p; b.env = r.env.p; b.x = x; b.tau = tau_ext; b.t = t; b.x_knot = x_knot; b.knot = r.knot.p; b.steps = r.steps.p;
+    b.stats = r.ro_stats.p; b.list = r.list.p; b.env_c = r.env_c.p; b.x_c = r.x_c.p; b.tau_c = r.tau_c.p; b.t_c = r.t_c.p; b.h_c = r.h_c.p;
+    b.h_save = r.h_save.p; b.stats_c = r.stats_c.p; b.count = r.ro_count.p;
+    radau_info_reset(r);
+    CU(cudaMemcpyAsync(r.knots.p, t_knot, sizeof(double) * n_knot, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemsetAsync(r.knot.p, 0, sizeof(int) * ne, c->stream));
+    CU(cudaMemsetAsync(r.steps.p, 0, sizeof(int) * ne, c->stream));
+    CU(cudaMemsetAsync(r.ro_stats.p, 0, sizeof(int) * 4 * ne, c->stream));
+    for (int round = 0;; ++round) {
+        CU(launch_radau_select(b, round == 0, c->stream));
+        c->launches += 1;
+        CU(cudaMemcpyAsync(r.h_counts + 5, r.ro_count.p, 2 * sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+        CU(cudaStreamSynchronize(c->stream));
+        r.syncs += 1;
+        if (r.h_counts[6]) return fail(PFC_E_ARG, "pfc_radau_rollout: t_knot[0] - t < h_min for some environment");
+        if (round == 0 && x_knot) CU(cudaMemsetAsync(x_knot, 0xFF, sizeof(double) * n_knot * ne * nx, c->stream));   // all-ones bytes: a NaN
+        const long long n_active = r.h_counts[5];
+        if (n_active == 0) break;
+        { const int rc = radau_step_device(c, n_active, r.env_c.p, r.x_c.p, tau_ext ? r.tau_c.p : nullptr, r.t_c.p, r.h_c.p, r.stats_c.p); if (rc != PFC_OK) return rc; }
+        CU(launch_radau_finish(b, n_active, c->stream));
+        c->launches += 1;
+    }
+    if (stats) CU(cudaMemcpyAsync(stats, r.ro_stats.p, sizeof(int32_t) * 4 * ne, cudaMemcpyDeviceToDevice, c->stream));
+    return PFC_OK;
+}
+
+int pfc_radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const double* t_knot, int64_t max_steps, double* x, const double* tau_ext, double* t,
+                             double* x_knot, int32_t* stats) {
+    { const int rc = radau_rollout_check(c, "pfc_radau_rollout_device", n_env, n_knot, t_knot, max_steps); if (rc != PFC_OK) return rc; }
+    if (n_env == 0) return PFC_OK;
+    if (!x || !t) return fail(PFC_E_ARG, "pfc_radau_rollout_device: NULL buffer");
+    CU(cudaSetDevice(c->device));
+    return radau_rollout_device(c, n_env, n_knot, t_knot, max_steps, x, tau_ext, t, x_knot, stats);
+}
+
+int pfc_radau_rollout(pfc_ctx* c, int64_t n_env, int n_knot, const double* t_knot, int64_t max_steps, double* x, const double* tau_ext, double* t,
+                      double* x_knot, int32_t* stats) {
+    { const int rc = radau_rollout_check(c, "pfc_radau_rollout", n_env, n_knot, t_knot, max_steps); if (rc != PFC_OK) return rc; }
+    if (n_env == 0) return PFC_OK;
+    if (!x || !t) return fail(PFC_E_ARG, "pfc_radau_rollout: NULL buffer");
+    CU(cudaSetDevice(c->device));
+    pfc_ctx::RadauState& r = c->radau;
+    const size_t ne = size_t(n_env), nx = size_t(c->state.n_x), nv = size_t(c->state.nv), nk = size_t(n_knot);
+    CU(r.x.ensure(ne * nx)); CU(r.t.ensure(ne)); CU(r.stats.ensure(4 * ne));
+    if (tau_ext) CU(r.tau.ensure(std::max<size_t>(nk * ne * nv, 1)));
+    if (x_knot) CU(r.x_knot.ensure(nk * ne * nx));
+    CU(cudaMemcpyAsync(r.x.p, x, sizeof(double) * ne * nx, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(r.t.p, t, sizeof(double) * ne, cudaMemcpyHostToDevice, c->stream));
+    if (tau_ext) CU(cudaMemcpyAsync(r.tau.p, tau_ext, sizeof(double) * nk * ne * nv, cudaMemcpyHostToDevice, c->stream));
+    const int rc = radau_rollout_device(c, n_env, n_knot, t_knot, max_steps, r.x.p, tau_ext ? r.tau.p : nullptr, r.t.p, x_knot ? r.x_knot.p : nullptr,
+                                        r.stats.p);
+    if (rc != PFC_OK) { cudaStreamSynchronize(c->stream); return rc; }
+    CU(cudaMemcpyAsync(x, r.x.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaMemcpyAsync(t, r.t.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
+    if (x_knot) CU(cudaMemcpyAsync(x_knot, r.x_knot.p, sizeof(double) * nk * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     if (stats) CU(cudaMemcpyAsync(stats, r.stats.p, sizeof(int32_t) * 4 * ne, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaStreamSynchronize(c->stream));
     return PFC_OK;

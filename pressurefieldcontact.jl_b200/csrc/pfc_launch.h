@@ -146,4 +146,29 @@ cudaError_t launch_radau_gather(const RadauBufs& b, long long n_states, cudaStre
 cudaError_t launch_radau_newton(const RadauBufs& b, long long n_active, cudaStream_t stream);
 cudaError_t launch_radau_controller(const RadauBufs& b, cudaStream_t stream);
 
+// A roll-out through shared knot times (pfc_radau_rollout): per round of steps, the environments that still have a knot ahead and steps
+// left are gathered into compact arrays, take one step as a sub-batch (the RadauBufs sequence above on the compact arrays), and are
+// scattered back.
+struct RadauRolloutBufs {
+    long long n_env, max_steps;
+    int nx, nv, n_knot;
+    const double* knots;        // [knot] absolute times
+    RadauEnv* env;              // [env] controller state
+    double* x;                  // [env][nx]
+    const double* tau;          // [knot][env][nv] or nullptr
+    double* t;                  // [env]
+    double* x_knot;             // [knot][env][nx] or nullptr
+    int* knot;                  // [env] next knot
+    int* steps;                 // [env] accepted steps of this roll-out
+    int* stats;                 // [env][4] knots reached, accepted steps, rejected attempts, stage evaluations
+    int* list;                  // [slot] environment of the compact slot
+    RadauEnv* env_c; double* x_c; double* tau_c; double* t_c; double* h_c; double* h_save; int* stats_c;   // [slot] compact step arrays
+    int* count;                 // [2]: compact slots of the last selection; 1 if some environment starts within h_min of knot 0
+};
+// One CTA: lists the environments with knot < n_knot and steps < max_steps (environment order), gathers them and prepares the knot step
+// (radau_knot_begin).  check: also test t_knot[0] - t >= h_min for every environment (count[1]; nothing is gathered when it fails).
+cudaError_t launch_radau_select(const RadauRolloutBufs& b, int check, cudaStream_t stream);
+// After the compact step: radau_knot_end, the x_knot rows, the statistics and the write-back of the n_active slots.
+cudaError_t launch_radau_finish(const RadauRolloutBufs& b, long long n_active, cudaStream_t stream);
+
 }  // namespace pfc

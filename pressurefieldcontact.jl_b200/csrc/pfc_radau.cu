@@ -13,7 +13,9 @@
 // the plan kernel lists the pending environments' matrices and stage states; per Newton iteration the stage states of the still-active
 // environments are packed (gather), evaluated by calcXd! on the host side of the launch sequence, and radau_newton_kernel (one CTA per
 // active environment) does calcEw!, the mat-vecs with invC, updateStageX! and the convergence / divergence tests; radau_controller_kernel
-// (one thread per environment) applies calc_and_update_h! / update_rule! at the end of each round.
+// (one thread per environment) applies calc_and_update_h! / update_rule! at the end of each round.  A roll-out through knot times wraps that
+// step: radau_select_kernel gathers the environments still under way into compact arrays the step runs on, radau_finish_kernel scatters them
+// back and moves the environments that landed on their knot to the next one.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -285,7 +287,82 @@ __global__ void __launch_bounds__(128) radau_controller_kernel(RadauBufs b) {
     b.env[e] = ctl;
 }
 
+// roll-out round: the environments with a knot ahead and steps left, in environment order, gathered into the compact slots
+__global__ void __launch_bounds__(kPlanThreads) radau_select_kernel(RadauRolloutBufs b, int check) {
+    using Scan = cub::BlockScan<int, kPlanThreads>;
+    __shared__ typename Scan::TempStorage tmp;
+    int bad = 0;
+    if (check)
+        for (long long e = threadIdx.x; e < b.n_env; e += kPlanThreads) bad |= !(b.knots[0] - b.t[e] >= kRadauHMin);
+    if (__syncthreads_or(bad)) {
+        if (threadIdx.x == 0) { b.count[0] = 0; b.count[1] = 1; }
+        return;
+    }
+    int base = 0;
+    for (long long c0 = 0; c0 < b.n_env; c0 += kPlanThreads) {
+        const long long e = c0 + threadIdx.x;
+        int flag = 0;
+        if (e < b.n_env) flag = b.knot[e] < b.n_knot && b.steps[e] < b.max_steps;
+        int pos, agg;
+        Scan(tmp).ExclusiveSum(flag, pos, agg);
+        __syncthreads();
+        if (flag) {
+            const long long p = base + pos;
+            const int k = b.knot[e];
+            RadauEnv en = b.env[e];
+            const double t = b.t[e];
+            b.h_save[p] = radau_knot_begin(en, t, b.knots[k]);
+            b.list[p] = (int)e;
+            b.env_c[p] = en;
+            b.t_c[p] = t;
+            for (int n = 0; n < b.nx; ++n) b.x_c[p * b.nx + n] = b.x[e * b.nx + n];
+            if (b.tau) {
+                const double* row = b.tau + ((long long)k * b.n_env + e) * b.nv;
+                for (int n = 0; n < b.nv; ++n) b.tau_c[p * b.nv + n] = row[n];
+            }
+        }
+        base += agg;
+    }
+    if (threadIdx.x == 0) { b.count[0] = base; b.count[1] = 0; }
+}
+
+// one thread per compact slot: the step's end relative to the knot, then everything back to the environment's own arrays
+__global__ void __launch_bounds__(128) radau_finish_kernel(RadauRolloutBufs b, long long n_active) {
+    const long long p = blockIdx.x * (long long)blockDim.x + threadIdx.x;
+    if (p >= n_active) return;
+    const long long e = b.list[p];
+    const int k = b.knot[e];
+    RadauEnv en = b.env_c[p];
+    double t_new;
+    const bool hit = radau_knot_end(en, b.t[e], b.knots[k], b.h_c[p], b.h_save[p], &t_new);
+    b.t[e] = t_new;
+    b.env[e] = en;
+    b.steps[e] += 1;
+    if (hit) b.knot[e] = k + 1;
+    int* o = b.stats + 4 * e;
+    const int* s = b.stats_c + 4 * p;
+    o[0] += hit; o[1] += 1; o[2] += s[2]; o[3] += s[3];
+    const double* xs = b.x_c + p * b.nx;
+    double* xd = b.x + e * b.nx;
+    double* row = hit && b.x_knot ? b.x_knot + ((long long)k * b.n_env + e) * b.nx : nullptr;
+    for (int n = 0; n < b.nx; ++n) {
+        xd[n] = xs[n];
+        if (row) row[n] = xs[n];
+    }
+}
+
 }  // namespace
+
+cudaError_t launch_radau_select(const RadauRolloutBufs& b, int check, cudaStream_t stream) {
+    radau_select_kernel<<<1, kPlanThreads, 0, stream>>>(b, check);
+    return cudaGetLastError();
+}
+
+cudaError_t launch_radau_finish(const RadauRolloutBufs& b, long long n_active, cudaStream_t stream) {
+    if (n_active == 0) return cudaSuccess;
+    radau_finish_kernel<<<(unsigned)((n_active + 127) / 128), 128, 0, stream>>>(b, n_active);
+    return cudaGetLastError();
+}
 
 cudaError_t launch_radau_plan(const RadauBufs& b, int mode, cudaStream_t stream) {
     radau_plan_kernel<<<1, kPlanThreads, 0, stream>>>(b, mode);

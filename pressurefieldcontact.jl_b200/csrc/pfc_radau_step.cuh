@@ -151,4 +151,30 @@ PFC_RHD int radau_control(RadauEnv& e, int max_rule, double h_max, double* h_tak
     return e.h < kRadauHMin ? kRadauHTooSmall : kRadauRetry;
 }
 
+// Roll-outs through knot times (radau.py rollout_radau).  Before a step toward knot T from t: if h would end within h_min of T (or past
+// it), the step is a knot step of exactly T - t, so no ordinary step leaves a remainder below h_min.  Returns h_save, the h the controller
+// had (0 for an ordinary step).
+PFC_RHD double radau_knot_begin(RadauEnv& e, double t, double T) {
+    const double rem = T - t;
+    if (e.h >= rem - kRadauHMin) {
+        const double h_save = e.h;
+        e.h = rem;
+        return h_save;
+    }
+    return 0.0;
+}
+
+// After the accepted step of h_taken from t: true when it was the knot step (a rejected knot step is retried with a smaller, ordinary h).
+// *t_new is then T exactly, and a proposal of at least h_taken is raised back to h_save, so a short knot step does not shrink the next
+// ordinary one.  Otherwise *t_new = t + h_taken, as after any step.
+PFC_RHD bool radau_knot_end(RadauEnv& e, double t, double T, double h_taken, double h_save, double* t_new) {
+    if (h_save > 0.0 && h_taken == T - t) {
+        *t_new = T;
+        if (e.h >= h_taken && h_save > e.h) e.h = h_save;
+        return true;
+    }
+    *t_new = t + h_taken;
+    return false;
+}
+
 }  // namespace pfc

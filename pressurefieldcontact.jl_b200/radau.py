@@ -31,7 +31,7 @@ from __future__ import annotations
 import numpy as np
 
 __all__ = ["radau_table", "RadauTable", "RadauStep", "RadauRule", "RadauIntegrator", "makeRadauIntegrator", "solveRadau", "calcJacobian",
-           "update_h", "radau_rule_to_stage", "integrate_radau"]
+           "update_h", "radau_rule_to_stage", "integrate_radau", "rollout_radau"]
 
 
 def radau_rule_to_stage(n: int) -> int:   # load_table_from_file.jl:2
@@ -119,6 +119,7 @@ class RadauIntegrator:   # radau_struct.jl:108-125
         self.inv_C_stage = [np.zeros((NX, NX), dtype=np.complex128) for _ in range(n)]
         self.n_de_float = 0     # Float64 evaluations of de (stage evaluations)
         self.n_de_chunk = 0     # Dual-NC evaluations of de (Jacobian chunks)
+        self.n_rejected = 0     # attempts that did not converge
 
     def current_table(self) -> RadauTable:
         return self.table[self.rule.s - 1]
@@ -289,6 +290,7 @@ def solveRadau(rr: RadauIntegrator, x0: np.ndarray, t: float = 0.0):
         _update_rule(rr)
         if rr.step.exit_flag == 0:
             return rr.step.h_prev, rr.X_stage[table.n_stage - 1] * 1.0, t + rr.step.h_prev
+        rr.n_rejected += 1
         if rr.step.h < rr.step.h_min:
             raise RuntimeError("time step is too small, something is wrong")
 
@@ -308,3 +310,52 @@ def integrate_radau(rr: RadauIntegrator, x0, t_final: float = 1.0, max_steps: in
         if t_final < t:
             break
     return np.array(ts), np.array(xs)
+
+
+def rollout_radau(rr: RadauIntegrator, x0, t0: float, t_knots, de=None, max_steps: int = 1000, after_step=None, record=None):
+    """x0 at t0 through the knot times t_knots (strictly increasing, gaps and t_knots[0] - t0 at least h_min), one scene: the mirror of
+    pfc_radau_rollout.  de (optional) holds one ODE object per interval (t_knots[k-1], t_knots[k]], e.g. one per tau_ext of a control
+    sequence; rr.de_object otherwise.  The controller state of rr carries over from earlier steps and into later ones.
+
+    A step toward knot T from t is a knot step of exactly T - t when h >= (T - t) - h_min, so no ordinary step leaves less than h_min to
+    the knot.  A rejected knot step retries with a smaller, ordinary h.  Once the knot step is accepted, t = T exactly, x goes to
+    x_knot[k], and a controller proposal of at least the knot step's h is raised back to the h the knot step replaced.
+    after_step(x) is principal_value!; record (a list) gets (h_taken, t, x, stage evaluations) per accepted step.
+    Returns (x_knot [K, NX] with NaN rows for knots not reached within max_steps, x, t, stats = [knots, steps, rejected, evaluations])."""
+    t_knots = np.asarray(t_knots, dtype=np.float64).reshape(-1)
+    h_min = rr.step.h_min
+    if len(t_knots) == 0 or not np.isfinite(t_knots).all() or not (np.diff(t_knots) >= h_min).all() or not (t_knots[0] - t0 >= h_min):
+        raise ValueError("knot times must be finite and increase by at least h_min, from t0 on")
+    x = np.array(x0, dtype=np.float64)
+    t = float(t0)
+    x_knot = np.full((len(t_knots), len(x)), np.nan)
+    stats = [0, 0, 0, 0]
+    k = 0
+    while k < len(t_knots) and stats[1] < max_steps:
+        if de is not None:
+            rr.de_object = de[k]
+        T = float(t_knots[k])
+        rem = T - t
+        h_save = 0.0
+        if rr.step.h >= rem - h_min:
+            h_save = rr.step.h
+            rr.step.h, rr.step.h_inv = rem, 1.0 / rem
+        n_eval, n_rej = rr.n_de_float, rr.n_rejected
+        h_taken, x, _ = solveRadau(rr, x, t)
+        if after_step is not None:
+            after_step(x)
+        stats[1] += 1
+        stats[2] += rr.n_rejected - n_rej
+        stats[3] += rr.n_de_float - n_eval
+        if h_save > 0.0 and h_taken == rem:
+            t = T
+            x_knot[k] = x
+            k += 1
+            stats[0] += 1
+            if rr.step.h >= h_taken and h_save > rr.step.h:
+                rr.step.h, rr.step.h_inv = h_save, 1.0 / h_save
+        else:
+            t = t + h_taken
+        if record is not None:
+            record.append((h_taken, t, x.copy(), rr.n_de_float - n_eval))
+    return x_knot, x, t, stats

@@ -14,7 +14,8 @@ What runs where
 
 DeviceBatchedRadau is the same integrator behind the library's C ABI (pfc_radau_init / pfc_radau_step_device): the Newton iteration,
 error estimate and step-size / order control run in CUDA kernels, and the host only reads how many stage states are still active once per
-Newton iteration.  It has BatchedRadau's interface (step, integrate, t) so that the tests and scripts/run_batched_radau.py drive both.
+Newton iteration.  It has BatchedRadau's interface (step, integrate, t) so that the tests and scripts/run_batched_radau.py drive both,
+and rollout(): every environment through shared knot times with a piecewise-constant tau_ext (pfc_radau_rollout_device).
 
 BatchedRadau is caller-side code (the reference's is Julia); it exists to drive the device path end to end the way
 integrate_scenario_radau does and to measure batched roll-out throughput.
@@ -258,3 +259,20 @@ class DeviceBatchedRadau:
                 ts.append(self.t.cpu().numpy().copy())
                 xs.append(x.cpu().numpy().copy())
         return np.array(ts), np.array(xs)
+
+    def rollout(self, x0, t_knots, tau=None, max_steps: int = 1000):
+        """pfc_radau_rollout_device: every environment from x0 [E, NX] at self.t through the absolute knot times t_knots [K], with tau
+        [K, E, nv] (or None) acting on (t_knots[k-1], t_knots[k]].  Returns (x_knot [K, E, NX] with NaN rows for knots an environment did
+        not reach within max_steps, stats [E, 4] = knots reached, accepted steps, rejected attempts, stage evaluations), torch tensors on
+        the device; self.t advances to where each environment stopped."""
+        t_knots = np.asarray(t_knots, dtype=np.float64).reshape(-1)
+        with torch.cuda.stream(self.stream):
+            x = torch.as_tensor(x0).to(device=self.dev, dtype=torch.float64).reshape(self.E, self.NX).contiguous().clone()
+            tau_t = None if tau is None else torch.as_tensor(tau).to(device=self.dev, dtype=torch.float64).contiguous()
+            t = self.t.clone()
+            x_knot = torch.empty((len(t_knots), self.E, self.NX), dtype=torch.float64, device=self.dev)
+            stats = torch.zeros((self.E, 4), dtype=torch.int32, device=self.dev)
+            self.ctx.radau_rollout_device(self.E, t_knots, max_steps, x.data_ptr(), None if tau_t is None else tau_t.data_ptr(), t.data_ptr(),
+                                          x_knot.data_ptr(), stats.data_ptr())
+            self.t = t
+            return x_knot, stats
