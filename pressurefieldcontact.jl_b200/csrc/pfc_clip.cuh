@@ -158,24 +158,41 @@ template <class T> PFC_D Vec3<T> weight_poly(const Vec3<T>& p1, const Vec3<T>& p
     return mk<T>(c1 * p2.x - c2 * p1.x, c1 * p2.y - c2 * p1.y, c1 * p2.z - c2 * p1.z);
 }
 
-// Plane (4 coefficients) against a tetrahedron given by its 4 vertices; writes a 3- or 4-gon with
-// the plane's orientation into out and returns its size (0 when all vertices are on one side).
-template <class T> __device__ __noinline__ int plane_tet(const T* plane, const Vec3<T>* v, Vec3<T>* out) {
+// edge lists of plane_tet per case, 0-based (i1, i2) -> weightPoly(v[i1], v[i2], proj[i1], proj[i2])
+// lone vertex k:   plane_tet_intersection.jl:52-79 ; two-two split: :81-106
+constexpr signed char kPlaneTetTri[4][3][2] = {{{1, 0}, {3, 0}, {2, 0}}, {{0, 1}, {2, 1}, {3, 1}}, {{0, 2}, {3, 2}, {1, 2}}, {{0, 3}, {1, 3}, {2, 3}}};
+constexpr signed char kPlaneTetQuad[3][4][2] = {{{1, 2}, {1, 3}, {0, 3}, {0, 2}}, {{0, 1}, {0, 3}, {2, 3}, {2, 1}}, {{0, 2}, {0, 1}, {3, 1}, {3, 2}}};
+// The same lists as 4-bit fields i1 | i2 << 2 (case sel, edge k at bit 4 * (n_edges * sel + k)): a shift of a constant instead of a
+// table in local memory.
+constexpr unsigned long long plane_tet_edge_bits(bool quad) {
+    unsigned long long b = 0;
+    for (int s = 0; s < (quad ? 3 : 4); ++s)
+        for (int k = 0; k < (quad ? 4 : 3); ++k) {
+            const signed char* e = quad ? kPlaneTetQuad[s][k] : kPlaneTetTri[s][k];
+            b |= (unsigned long long)(e[0] | e[1] << 2) << (4 * ((quad ? 4 : 3) * s + k));
+        }
+    return b;
+}
+constexpr unsigned long long kPlaneTetTriBits = plane_tet_edge_bits(false), kPlaneTetQuadBits = plane_tet_edge_bits(true);
+template <class T> PFC_D T pick4(int i, const T& a, const T& b, const T& c, const T& d) { return i == 0 ? a : i == 1 ? b : i == 2 ? c : d; }
+
+// Plane (4 coefficients) against a tetrahedron whose vertex k is vert(k): hands the vertices of a 3- or 4-gon with the plane's
+// orientation to emit(j, vertex), j = 0, 1, ..., and returns its size (0 when all vertices are on one side).  Every array index is
+// a constant once the loops are unrolled, and vert is asked again for the two ends of each cut edge instead of holding all four
+// vertices: a caller that inlines this keeps what it needs in registers, and few of them.
+template <class T, class Vert, class Emit> PFC_D int plane_tet_inline(const T* plane, Vert&& vert, Emit&& emit) {
     T proj[4];
     int n_neg = 0, n_pos = 0;
     unsigned pos = 0, neg = 0;
 #pragma unroll
     for (int k = 0; k < 4; ++k) {
-        proj[k] = plane[0] * v[k].x + plane[1] * v[k].y + plane[2] * v[k].z + plane[3];
+        const Vec3<T> v = vert(k);
+        proj[k] = plane[0] * v.x + plane[1] * v.y + plane[2] * v.z + plane[3];
         const double p = val(proj[k]);
         if (p < 0.0) { ++n_neg; neg |= 1u << k; }
         if (0.0 < p) { ++n_pos; pos |= 1u << k; }
     }
     if (n_pos == 0 || n_neg == 0) return 0;
-    // edge lists per case, 0-based (i1, i2) -> weightPoly(v[i1], v[i2], proj[i1], proj[i2])
-    // lone vertex k:   plane_tet_intersection.jl:52-79 ; two-two split: :81-106
-    const signed char TRI[4][3][2] = {{{1, 0}, {3, 0}, {2, 0}}, {{0, 1}, {2, 1}, {3, 1}}, {{0, 2}, {3, 2}, {1, 2}}, {{0, 3}, {1, 3}, {2, 3}}};
-    const signed char QUAD[3][4][2] = {{{1, 2}, {1, 3}, {0, 3}, {0, 2}}, {{0, 1}, {0, 3}, {2, 3}, {2, 1}}, {{0, 2}, {0, 1}, {3, 1}, {3, 2}}};
     int cnt, sel;
     bool forward;
     if (n_pos == 1) { sel = __ffs(pos) - 1; cnt = 3; forward = true; }
@@ -189,13 +206,20 @@ template <class T> __device__ __noinline__ int plane_tet(const T* plane, const V
         cnt = 4;
         forward = (0.0 < val(proj[0]));
     }
-    for (int k = 0; k < cnt; ++k) {
-        const int i1 = (cnt == 3) ? TRI[sel][k][0] : QUAD[sel][k][0];
-        const int i2 = (cnt == 3) ? TRI[sel][k][1] : QUAD[sel][k][1];
-        const Vec3<T> p = weight_poly(v[i1], v[i2], proj[i1], proj[i2]);
-        out[forward ? k : cnt - 1 - k] = p;
-    }
+    const unsigned long long edges = (cnt == 3) ? kPlaneTetTriBits : kPlaneTetQuadBits;
+#pragma unroll
+    for (int j = 0; j < 4; ++j)   // output vertex j is edge k of the case's list
+        if (j < cnt) {
+            const int k = forward ? j : cnt - 1 - j;
+            const unsigned e = unsigned(edges >> (4 * (cnt * sel + k))) & 15u;
+            const int i1 = e & 3u, i2 = e >> 2;
+            emit(j, weight_poly(vert(i1), vert(i2), pick4(i1, proj[0], proj[1], proj[2], proj[3]), pick4(i2, proj[0], proj[1], proj[2], proj[3])));
+        }
     return cnt;
+}
+// The same for callers that do not inline it: tet vertices v[0 .. 4), the polygon written to out[0 .. size).
+template <class T> __device__ __noinline__ int plane_tet(const T* plane, const Vec3<T>* v, Vec3<T>* out) {
+    return plane_tet_inline(plane, [&](int k) { return v[k]; }, [&](int j, const Vec3<T>& p) { out[j] = p; });
 }
 
 }  // namespace pfc

@@ -685,9 +685,9 @@ __global__ void __launch_bounds__(kChunk, 2) narrow_large_kernel(SceneDev sc, La
             if (lane < 8) sm.tot[lane] = 0.0;
         }
         __syncthreads();
-        // ---- 1. start polygons
+        // ---- 1. start polygons, staged in doubles [16, 32) of slot tid (the compaction below writes doubles [0, 16) of a slot only)
         const unsigned i = seg_start[p] + (u - unit_start[p]) * kChunk + tid;
-        double zr[16];
+        double* zr = sm.poly + tid * kLPolyStride + 16;
         int n0 = 0;
         int3 pr = make_int3(0, 0, 0);
         if (i < seg_end[p]) {

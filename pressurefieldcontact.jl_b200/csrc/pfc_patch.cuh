@@ -285,7 +285,8 @@ PFC_D bool finish_polygon_slot(int n, const TetRec& tet_g, const Vec3<double>& n
 
 // ---- stage A split in two, for the tile kernel's compacted clip ---------------------------------------------------------
 // start_polygon_zeta: everything before the first face cut -- the start polygon (the triangle, or the plane/tet section) in
-// tetrahedral coordinates of tet 2, in REGISTERS (zr[4 * k + i]); returns its vertex count, 0 when the pair is rejected (same
+// tetrahedral coordinates of tet 2, written to zr[4 * k + i] (the tile kernel passes a shared-memory staging area: 16 doubles
+// held across its slot scan would cost it a local-memory frame); returns its vertex count, 0 when the pair is rejected (same
 // tests, same arithmetic as clip_pair).  pair_normal: the polygon normal, recomputed from the records after the clip.
 PFC_D int start_polygon_zeta(const SceneDev& sc, const InsDev& ins, int prim1, int prim2, const PatchCtx<double>& cx, double* zr) {
     const TetRec& t2 = sc.tets[ins.prim_base2 + prim2];
@@ -300,8 +301,9 @@ PFC_D int start_polygon_zeta(const SceneDev& sc, const InsDev& ins, int prim1, i
             const Vec3<double> p = apply_d(cx.x21, mk<double>(tri.v[3 * k], tri.v[3 * k + 1], tri.v[3 * k + 2]));
 #pragma unroll
             for (int i = 0; i < 4; ++i) {
-                zr[4 * k + i] = t2r.inv[4 * i] * p.x + t2r.inv[4 * i + 1] * p.y + t2r.inv[4 * i + 2] * p.z + t2r.inv[4 * i + 3];
-                if (!(zr[4 * k + i] <= 0.0)) all_non_pos &= ~(1u << i);
+                const double zz = t2r.inv[4 * i] * p.x + t2r.inv[4 * i + 1] * p.y + t2r.inv[4 * i + 2] * p.z + t2r.inv[4 * i + 3];
+                zr[4 * k + i] = zz;
+                if (!(zz <= 0.0)) all_non_pos &= ~(1u << i);
             }
         }
         return all_non_pos ? 0 : 3;
@@ -316,21 +318,17 @@ PFC_D int start_polygon_zeta(const SceneDev& sc, const InsDev& ins, int prim1, i
         plane[2] = cx.Ebar2 * t2.eps_r[2] - (g0 * Y.r[2] + g1 * Y.r[5] + g2 * Y.r[8]);
         plane[3] = cx.Ebar2 * t2.eps_r[3] - (g0 * Y.t[0] + g1 * Y.t[1] + g2 * Y.t[2] + g3);
     }
-    Vec3<double> v[4], poly[4];
+    // tet 1's vertices in r2 are recomputed where they are needed, and each vertex of the section goes to tetrahedral coordinates
+    // as soon as it exists: neither polygon is held in registers
+    const auto vert = [&](int k) { return apply_d(cx.x21, mk<double>(t1.v[3 * k], t1.v[3 * k + 1], t1.v[3 * k + 2])); };
+    const int n0 = plane_tet_inline(plane, vert, [&](int k, const Vec3<double>& p) {
 #pragma unroll
-    for (int k = 0; k < 4; ++k) v[k] = apply_d(cx.x21, mk<double>(t1.v[3 * k], t1.v[3 * k + 1], t1.v[3 * k + 2]));
-    const int n0 = plane_tet(plane, v, poly);
-    if (n0 < 3) return 0;
-#pragma unroll
-    for (int k = 0; k < 4; ++k)
-        if (k < n0) {
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-                const double zz = t2.inv[4 * i] * poly[k].x + t2.inv[4 * i + 1] * poly[k].y + t2.inv[4 * i + 2] * poly[k].z + t2.inv[4 * i + 3];
-                zr[4 * k + i] = zz * ((1.0e-14 < fabs(zz)) ? 1.0 : 0.0);   // zero_small_coordinates
-            }
+        for (int i = 0; i < 4; ++i) {
+            const double zz = t2.inv[4 * i] * p.x + t2.inv[4 * i + 1] * p.y + t2.inv[4 * i + 2] * p.z + t2.inv[4 * i + 3];
+            zr[4 * k + i] = zz * ((1.0e-14 < fabs(zz)) ? 1.0 : 0.0);   // zero_small_coordinates
         }
-    return n0;
+    });
+    return n0 < 3 ? 0 : n0;
 }
 
 PFC_D Vec3<double> pair_normal(const SceneDev& sc, const InsDev& ins, int prim1, int prim2, const PatchCtx<double>& cx) {

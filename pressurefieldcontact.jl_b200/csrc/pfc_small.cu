@@ -283,9 +283,10 @@ __global__ void __launch_bounds__(32 * NW, MINB) broad_tile_kernel(SceneDev sc, 
 // consecutive (environment, instruction) problems and every phase is flattened over all of them:
 //   1. 32 threads per problem fill the problem's shared context (transform, inverse, twist, constants), one element each;
 //   2. the tile's candidate pairs (about 118 for P = 4 boxes.jl instructions) are dealt one per thread and taken up to their
-//      start polygon in REGISTERS (start_polygon_zeta: about 3 of 10 pairs are rejected there); a block scan packs the
-//      survivors, in candidate order, into the shared-memory PolyRec slots (stride 35 doubles: conflict-free; no local
-//      memory); slot d is clipped IN PLACE by thread d, centroid -> a finished PolyRec.  The clip -- the most divergent part
+//      start polygon, staged in the free upper half of the thread's own slot (start_polygon_zeta: about 3 of 10 pairs are
+//      rejected there); a block scan packs the survivors, in candidate order, into the shared-memory PolyRec slots (stride 35
+//      doubles: conflict-free); slot d is clipped IN PLACE by thread d, centroid -> a finished PolyRec.  The kernel has no
+//      local-memory frame and no spills at 128 registers (tests/test_small_kernel_resources.py).  The clip -- the most divergent part
 //      of the step -- so starts with all lanes of the leading warps busy, and a tile with more than 128 candidates (19 % of
 //      the settled boxes.jl stacks) needs one clip / quadrature / summation round instead of two because its survivors fit
 //      the 128 slots (164 -> 144 us on 4096 environments).  When the survivors of a round do not fit, the round after the
@@ -326,7 +327,8 @@ template <int P> struct TileSmem {   // P problems, P warps
     long long next_tile;    // drawn from the ticket counter by thread 0
     double fpv[P][8];
 };
-static_assert(sizeof(TileSmem<4>) <= 45 * 1024, "5 CTAs per SM need <= 45 KB each");
+// 4 CTAs per SM (the launch's grid and the register budget assume it): 228 KB of shared memory per SM, 1 KB reserved per CTA
+static_assert(sizeof(TileSmem<4>) <= 56 * 1024, "4 CTAs per SM need <= 56 KB each");
 
 template <int P, int MINB>
 __global__ void __launch_bounds__(32 * P, MINB) narrow_tile_kernel(SceneDev sc, EvalIO io, int cap, const unsigned* __restrict__ pairs_in, unsigned* __restrict__ ticket) {
@@ -342,6 +344,10 @@ __global__ void __launch_bounds__(32 * P, MINB) narrow_tile_kernel(SceneDev sc, 
     for (long long tile = blockIdx.x; tile < n_tile;) {
         // ---- 1. problem contexts: warp q fills problem q, one element per lane
         {
+            // (lane and warp numbers made opaque per tile: this phase's index and address arithmetic is redone for each tile instead
+            // of being hoisted out of the tile loop, where its results would be held -- spilled -- across the clip and the quadrature)
+            int lane = tid & 31, wib = tid >> 5;
+            asm volatile("" : "+r"(lane), "+r"(wib));
             const long long prob = tile * P + wib;
             const long long env = prob < n_prob ? prob / sc.n_small : 0;
             const int k = prob < n_prob ? sc.small_ins[prob - env * sc.n_small] : 0;
@@ -364,25 +370,26 @@ __global__ void __launch_bounds__(32 * P, MINB) narrow_tile_kernel(SceneDev sc, 
         }
         __syncthreads();
         if (tid == 0) sm.next_tile = (long long)gridDim.x + atomicAdd(ticket, 1u);   // read after the tile's last barrier
-        int pre[P + 1];
-        pre[0] = 0;
+        int n_cand = 0;
 #pragma unroll
-        for (int q = 0; q < P; ++q) pre[q + 1] = pre[q] + sm.n_cand[q];
-        const int n_cand = pre[P];
+        for (int q = 0; q < P; ++q) n_cand += sm.n_cand[q];
         for (int j = lane; j < P * 8; j += 32) sm.wtot[wib][j >> 3][j & 7] = 0.0;   // this warp's running sums (warp-private)
         int filled = 0;          // occupied polygon slots (block-uniform)
         int c0 = 0;              // first candidate of the next round (block-uniform)
         while (true) {
-            // ---- 2a. one candidate pair per thread up to its start polygon (registers)
+            // ---- 2a. one candidate pair per thread up to its start polygon, staged in doubles [16, 32) of slot tid: until the clip
+            // an occupied slot holds its start polygon in doubles [0, 16) only, and the compaction below writes nothing else
             if (c0 < n_cand) {
                 const int c = c0 + tid;
-                double zr[16];
+                double* zr = sm.poly + tid * kPolyStride + 16;
                 int n0 = 0, q = 0;
                 unsigned e = 0;
                 if (c < n_cand) {
-                    int first = 0;   // first candidate of problem q (pre[] by a run-time index would go to local memory)
+                    // first candidate of problem q: the prefix sums are taken again from shared memory (a per-thread copy held over the
+                    // tile costs registers the clip needs)
+                    int first = 0, end = 0;
 #pragma unroll
-                    for (int r = 1; r < P; ++r) { const bool ge = c >= pre[r]; q += ge; first = ge ? pre[r] : first; }
+                    for (int r = 1; r < P; ++r) { end += sm.n_cand[r - 1]; const bool ge = c >= end; q += ge; first = ge ? end : first; }
                     e = pairs_in[(size_t)cap * sm.ei[q] + (c - first)];
                     n0 = start_polygon_zeta(sc, sc.ins[sm.ins[q]], dec_a(e), dec_b(e), sm.cx[q], zr);
                 }
