@@ -66,27 +66,29 @@ PFC_D void broad_phase_xform(const Xform<double>& x21, double* Rab, double* tab)
 // What limited the first version of this kernel (one group of 16 lanes per problem, node records read from global memory) was
 // not the FP64 pipe but the L1 data pipe: every lane gathered its two 128 B node records with its own vector loads, so one warp-wide load instruction touched 32 different lines and cost 32 wavefronts
 // for 16 useful bytes each (ncu: l1tex__data_pipe_lsu_wavefronts ~ 66 % of peak, profiles/r1_v7_*).  Here
-//   * the persistent CTA stages the node records of all small instructions ONCE in shared memory at an odd stride
-//     (17 doubles): a lane-private record read is then conflict-free, 2 wavefronts per 64-bit load instead of 32;
+//   * the persistent CTA stages the node records of all small instructions ONCE in shared memory, as the float records of the
+//     filtered SAT (FiltNode, 80 B: five 16 B loads per record);
 //   * each warp owns a tile of P consecutive problems whose frontiers form ONE flattened array (problem-major, DFS order
 //     inside a problem), and every level runs in two phases:
-//       A. the OPEN node pairs (a compact work list of frontier slots) are tested one per lane, lanes dense: 15-axis SAT
-//          (pfc_sat.cuh: the reference's arithmetic, operation by operation) -> a result code per slot;
+//       A. the OPEN node pairs (a compact work list of frontier slots) are tested one per lane, lanes dense: the filtered 15-axis
+//          SAT in float (pfc_sat.cuh: sat_filter, a certified error bound) -> a result code per slot; the few slots it cannot
+//          decide are compacted and tested again, one per lane, with the reference's FP64 arithmetic, operation by operation, on
+//          the global node records;
 //       B. an ordered rebuild over the whole frontier (integer work only): finished pairs are copied, hits are replaced by
 //          their children in the reference's visiting order, a warp scan gives the positions; the open children form the
 //          next work list.
 //     When no pair is open the frontier is exactly the reference's recursion order: no atomics, no sort, bit-exact lists.
 // Warps never synchronise with each other after the staging barrier.
-constexpr int kNodeStride = 17;        // doubles per staged node record (16 + 1 pad: odd, so lane-private records do not collide)
-constexpr int kNodeTabMax = 320;       // nodes staged at most (43.5 KB); larger scenes read the records from global memory
+constexpr int kNodeTabMax = 320;       // nodes staged at most (25 KB of FiltNode); larger scenes test every pair exactly from global memory
 template <int P> struct BroadTileLayout {
-    // per warp: double xf[P][12] | long long ei[P] | unsigned front[2][P * cap] | int pre[2][P + 1] | int ins[P] | u16 olist[2][P * cap] | u8 res[P * cap]
+    // per warp: double xf[P][12] | long long ei[P] | FiltXf fxf[P] | unsigned front[2][P * cap] | int pre[2][P + 1] | int ins[P] |
+    // u16 olist[2][P * cap] | u8 res[P * cap]
     __host__ __device__ static size_t warp_bytes(int cap) {
-        const size_t b = sizeof(double) * P * 12 + sizeof(long long) * P + sizeof(unsigned) * 2 * P * cap + sizeof(int) * (2 * (P + 1) + P) +
-                         sizeof(unsigned short) * 2 * P * cap + (size_t)P * cap;
+        const size_t b = sizeof(double) * P * 12 + sizeof(long long) * P + sizeof(FiltXf) * P + sizeof(unsigned) * 2 * P * cap +
+                         sizeof(int) * (2 * (P + 1) + P) + sizeof(unsigned short) * 2 * P * cap + (size_t)P * cap;
         return (b + 15) / 16 * 16;
     }
-    __host__ __device__ static size_t bytes(int cap, int n_warps, int n_stage) { return sizeof(double) * kNodeStride * n_stage + warp_bytes(cap) * n_warps; }
+    __host__ __device__ static size_t bytes(int cap, int n_warps, int n_stage) { return sizeof(FiltNode) * n_stage + warp_bytes(cap) * n_warps; }
 };
 
 template <int P, int NW, int MINB>
@@ -95,20 +97,19 @@ __global__ void __launch_bounds__(32 * NW, MINB) broad_tile_kernel(SceneDev sc, 
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
     if (blockIdx.x == 0 && threadIdx.x == 0) pairs_out[(size_t)cap * io.n_env * sc.n_ins] = 0u;   // the narrow tile kernel's tile ticket
-    // ---- node table: staged once per (persistent) CTA
-    double* ntab_s = reinterpret_cast<double*>(smem_raw);
-    for (int j = threadIdx.x; j < n_stage * 16; j += 32 * NW) {
-        const int node = j >> 4, w = j & 15;
-        ntab_s[node * kNodeStride + w] = reinterpret_cast<const double*>(sc.nodes + sc.small_node_lo + node)[w];
-    }
+    // ---- node table of the filtered SAT (float records, kind / right for the rebuild): staged once per (persistent) CTA
+    FiltNode* ftab_s = reinterpret_cast<FiltNode*>(smem_raw);
+    for (int j = threadIdx.x; j < n_stage; j += 32 * NW) filt_node_from(sc.nodes[sc.small_node_lo + j], ftab_s[j]);
     __syncthreads();
-    const double* ntab = n_stage > 0 ? ntab_s - (size_t)kNodeStride * sc.small_node_lo : reinterpret_cast<const double*>(sc.nodes);
-    const int nstride = n_stage > 0 ? kNodeStride : 16;
+    const FiltNode* ftab = ftab_s - sc.small_node_lo;
+    const bool staged = n_stage > 0;   // otherwise every pair takes the exact test and the rebuild reads the FP64 records
+    auto right_of = [&](int node) { return staged ? ftab[node].right : sc.nodes[node].right; };
 
-    unsigned char* wbase = smem_raw + sizeof(double) * kNodeStride * n_stage + BroadTileLayout<P>::warp_bytes(cap) * wib;
+    unsigned char* wbase = smem_raw + sizeof(FiltNode) * n_stage + BroadTileLayout<P>::warp_bytes(cap) * wib;
     double* xf = reinterpret_cast<double*>(wbase);
     long long* s_ei = reinterpret_cast<long long*>(xf + P * 12);
-    unsigned* front = reinterpret_cast<unsigned*>(s_ei + P);
+    FiltXf* fxf = reinterpret_cast<FiltXf*>(s_ei + P);
+    unsigned* front = reinterpret_cast<unsigned*>(fxf + P);
     int* pre = reinterpret_cast<int*>(front + 2 * (size_t)P * cap);   // pre[b][q + 1]: end of problem q's segment in frontier b
     int* s_ins = pre + 2 * (P + 1);
     unsigned short* olist = reinterpret_cast<unsigned short*>(s_ins + P);
@@ -135,6 +136,8 @@ __global__ void __launch_bounds__(32 * NW, MINB) broad_tile_kernel(SceneDev sc, 
         const int n_valid = (int)((n_prob - tile * P) < P ? (n_prob - tile * P) : P);
         for (int j = lane; j <= P; j += T) pre[j] = j < n_valid ? j : n_valid;
         __syncwarp();
+        if (lane < n_valid) filt_xf_from(xf + 12 * lane, xf + 12 * lane + 9, fxf[lane]);
+        __syncwarp();
         int cur = 0, n_open = n_valid;
         int flags = 0;
         bool tile_overflow = false;   // warp-uniform
@@ -157,17 +160,43 @@ __global__ void __launch_bounds__(32 * NW, MINB) broad_tile_kernel(SceneDev sc, 
             }
             const int total = pc[P];
             if (n_open == 0) break;
-            // ---- A. SAT on the open node pairs, one per lane
-            for (int j = lane; j < n_open; j += T) {
-                const int c = olc[j];
+            // ---- A1. filtered SAT on the open node pairs, one per lane (pfc_sat.cuh: float, certified bound); the slots it cannot decide
+            // are listed in oln, which is free until the rebuild
+            int n_und = 0;   // warp-uniform
+            for (int j0 = 0; j0 < n_open; j0 += T) {
+                const int j = j0 + lane;
+                int c = 0;
+                bool und = false;
+                if (j < n_open) {
+                    c = olc[j];
+                    und = true;
+                    if (staged) {
+                        int q = 0;
+#pragma unroll
+                        for (int r = 1; r < P; ++r) q += (c >= pc[r]);
+                        const unsigned e = fc[c];
+                        const InsDev& ins = sc.ins[s_ins[q]];
+                        const FiltNode a = ftab[ins.node_base1 + dec_a(e)], b = ftab[ins.node_base2 + dec_b(e)];
+                        const int f = sat_filter(a, b, fxf[q]);
+                        und = f == kSatUndecided;
+                        if (!und) res[c] = (unsigned char)(f == kSatSeparated ? 0 : ((a.kind < 0) ? ((b.kind < 0) ? 1 : 2) : ((b.kind < 0) ? 3 : 4)));
+                    }
+                }
+                const unsigned m = __ballot_sync(0xffffffffu, und);
+                if (und) oln[n_und + __popc(m & ((1u << lane) - 1u))] = (unsigned short)c;
+                n_und += __popc(m);
+            }
+            __syncwarp();
+            // ---- A2. the reference's FP64 test on the undecided slots, from the global node records
+            for (int k = lane; k < n_und; k += T) {
+                const int c = oln[k];
                 int q = 0;
 #pragma unroll
                 for (int r = 1; r < P; ++r) q += (c >= pc[r]);
                 const unsigned e = fc[c];
-                const int ia = dec_a(e), ib = dec_b(e);
                 const InsDev& ins = sc.ins[s_ins[q]];
-                const NodeRec& a = *reinterpret_cast<const NodeRec*>(ntab + (size_t)nstride * (ins.node_base1 + ia));
-                const NodeRec& b = *reinterpret_cast<const NodeRec*>(ntab + (size_t)nstride * (ins.node_base2 + ib));
+                const NodeRec& a = sc.nodes[ins.node_base1 + dec_a(e)];
+                const NodeRec& b = sc.nodes[ins.node_base2 + dec_b(e)];
                 // (the general path for every node: skipping the identity products of axis-aligned nodes, as the large path's traversal does,
                 // makes the lanes of a work list diverge by node kind here -- measured 88 us against 84 us on 4096 environments)
                 SatA A;
@@ -193,9 +222,7 @@ __global__ void __launch_bounds__(32 * NW, MINB) broad_tile_kernel(SceneDev sc, 
                         if (code) {
                             const int ia = dec_a(e), ib = dec_b(e);
                             const InsDev& ins = sc.ins[s_ins[q]];
-                            const NodeRec& a = *reinterpret_cast<const NodeRec*>(ntab + (size_t)nstride * (ins.node_base1 + ia));
-                            const NodeRec& b = *reinterpret_cast<const NodeRec*>(ntab + (size_t)nstride * (ins.node_base2 + ib));
-                            const int al = ia + 1, ar = a.right, bl = ib + 1, br = b.right;   // pre-order: child 1 is the next record
+                            const int al = ia + 1, ar = right_of(ins.node_base1 + ia), bl = ib + 1, br = right_of(ins.node_base2 + ib);   // pre-order: child 1 is the next record
                             if (code == 1) { cnt = 1; ch0 = kDone | enc(ar, br); }
                             else if (code == 2) { cnt = ocnt = 2; ch0 = enc(ia, bl); ch1 = enc(ia, br); }
                             else if (code == 3) { cnt = ocnt = 2; ch0 = enc(al, ib); ch1 = enc(ar, ib); }
@@ -219,10 +246,11 @@ __global__ void __launch_bounds__(32 * NW, MINB) broad_tile_kernel(SceneDev sc, 
                 // only instructions whose slot is smaller than n_leaf1 * n_leaf2 (mid-size trees) can overflow it: the tile is given up --
                 // the host moves the instruction to the large path and repeats the evaluation
                 tile_overflow |= __any_sync(0xffffffffu, cnt > 0 && at + cnt > fcap);
-                if (c < total) {   // the last slot of problem q closes its segment (pc[] by a run-time index would go to local memory)
+                if (c < total) {   // the last slot of problem q closes its segment.  pc[] is read with compile-time indices only: end_q is the
+                    // first segment end above c (an 'r == q + 1' select chain is folded back into pc[q + 1], which puts pc[] in local memory)
                     int end_q = pc[P];
 #pragma unroll
-                    for (int r = 1; r < P; ++r) if (r == q + 1) end_q = pc[r];
+                    for (int r = P - 1; r >= 1; --r) end_q = c < pc[r] ? pc[r] : end_q;
                     if (c + 1 == end_q) pn[q + 1] = min(at + cnt, fcap);
                 }
                 carry += chunk_total;
@@ -251,9 +279,9 @@ __global__ void __launch_bounds__(32 * NW, MINB) broad_tile_kernel(SceneDev sc, 
                 int q = 0;
 #pragma unroll
                 for (int r = 1; r < P; ++r) q += (c >= pc[r]);
-                int beg_q = 0;
+                int beg_q = 0;   // the last segment start at or below c (compile-time indices, as above)
 #pragma unroll
-                for (int r = 1; r < P; ++r) if (r == q) beg_q = pc[r];
+                for (int r = 1; r < P; ++r) beg_q = c >= pc[r] ? pc[r] : beg_q;
                 const int i = c - beg_q;
                 const unsigned e = fc[c];
                 if (i < cap) pairs_out[(size_t)cap * s_ei[q] + i] = e;
