@@ -70,6 +70,21 @@ int pfc_add_instruction(pfc_ctx* ctx, int mesh_1, int mesh_2, double chi, int mo
 /* finalize! -- src/mechanism_scenario.jl:206-231: uploads the static scene and sizes the per-batch buffers for max_env environments. */
 int pfc_finalize(pfc_ctx* ctx, int64_t max_env);
 
+/* Per-environment contact parameters, after pfc_finalize (domain randomization, system identification, parameter sweeps as one batch).
+ * params[env][ins][8] = {chi, Ebar_1, Ebar_2, q0, q1, q2, q3, q4}: q = {mu_s, mu_d, v_c, -, -} for a regularized instruction,
+ * {tau, k_bar, mu_s, mu_d, magic} for a bristle one (pfc_add_instruction's order); Ebar_1 / Ebar_2 take the place of the Ebar that
+ * pfc_add_mesh gave mesh_1 / mesh_2 (Ebar_1 is ignored when mesh_1 is a triangle mesh); entries marked - are ignored.  Host pointer,
+ * copied.  While a table is set, environment e of every evaluation (pfc_eval_f64[_device], pfc_eval_dual6, pfc_eval_state_f64[_device],
+ * pfc_calcxd_*, pfc_radau_step[_device], pfc_radau_rollout[_device], pfc_get_traction) gives the bits of a context whose scene was built
+ * with row e's values, evaluated on the same batch.  (In a scene whose number of small instructions is not a multiple of 4, a narrow
+ * tile holds problems of neighbouring environments and a wrench's last bits depend on their contact patches, with or without a table:
+ * bit-for-bit equality then needs the environments that share e's tiles to carry row e too; otherwise e agrees to rounding.)  Those
+ * entry points (and pfc_radau_init) require n_env to equal the table's.  The candidate-pair lists do not
+ * depend on these values.  n_env = 0 clears the table.  PFC_E_ARG, with the table in force unchanged, before pfc_finalize, for n_env
+ * outside 0..max_env, a NULL params with n_env > 0, or a non-finite entry that the instruction's model uses.  The sharded and group
+ * evaluations (pfc_eval_sharded_*, pfc_group_eval_f64) return PFC_E_ARG while a table is set. */
+int pfc_set_contact_params(pfc_ctx* ctx, int64_t n_env, const double* params);
+
 /* forceAllElasticIntersections!, Float64 mode -- src/contact_algorithms_non_friction.jl:60-84, for n_env independent states of the scene.
  *   X_r2_r1 [env][ins][16]  b.x_r2_r1.mat (:112)          twist_r2 [env][ins][6]  b.twist_r2_r1_r2 (:128)
  *   s       [env][bristle][6] bristle state (tm.s)         sdot     [env][bristle][6] tm.s-dot   (both may be NULL without bristles)

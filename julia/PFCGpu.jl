@@ -187,6 +187,19 @@ function finalize_floating_gpu!(m::MechanismScenario)
     return nothing
 end
 
+"Per-environment contact parameters (pfc_set_contact_params): `params[:, ins, env]` = (chi, Ebar_1, Ebar_2, q0..q4) with q = (mu_s, mu_d,
+v_c, -, -) for a regularized instruction and (tau, k_bar, mu_s, mu_d, magic) for a bristle one; every batched call then takes
+n_env = size(params, 3).  `nothing` clears the table."
+function set_contact_params!(m::MechanismScenario, params::Union{Array{Float64,3},Nothing})
+    if params === nothing
+        check(ccall((:pfc_set_contact_params, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}), CTX[m], 0, C_NULL))
+    else
+        size(params, 1) == 8 || error("params must be 8 x n_ins x n_env")
+        GC.@preserve params check(ccall((:pfc_set_contact_params, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}), CTX[m], size(params, 3), params))
+    end
+    return nothing
+end
+
 "forceAllElasticIntersections! for a batch of states `x[:, env]`: generalized forces `f[:, env]` and `sdot` (pfc_eval_state_f64)."
 function force_all_batch_gpu!(f::Matrix{Float64}, sdot::Matrix{Float64}, m::MechanismScenario, x::Matrix{Float64})
     GC.@preserve x f sdot check(ccall((:pfc_eval_state_f64, LIB), Cint,

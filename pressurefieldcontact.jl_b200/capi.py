@@ -20,7 +20,7 @@ _vp = C.c_void_p
 
 # every symbol include/pfc.h declares
 SYMBOLS = [
-    "pfc_create", "pfc_destroy", "pfc_add_mesh", "pfc_add_instruction", "pfc_finalize", "pfc_eval_f64", "pfc_eval_f64_device",
+    "pfc_create", "pfc_destroy", "pfc_add_mesh", "pfc_add_instruction", "pfc_finalize", "pfc_set_contact_params", "pfc_eval_f64", "pfc_eval_f64_device",
     "pfc_eval_dual6", "pfc_set_debug", "pfc_get_pairs", "pfc_get_traction", "pfc_set_shard", "pfc_eval_sharded_begin", "pfc_eval_sharded_partials", "pfc_eval_sharded_step", "pfc_sync", "pfc_stream",
     "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_rollout", "pfc_radau_rollout_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
     "pfc_comm_unique_id", "pfc_comm_init_rank", "pfc_eval_sharded_f64_device", "pfc_group_create", "pfc_group_destroy", "pfc_group_size", "pfc_group_ctx",
@@ -47,6 +47,7 @@ def lib():
                                    C.POINTER(C.c_int)]
         L.pfc_add_instruction.argtypes = [_vp, C.c_int, C.c_int, C.c_double, C.c_int, _d, C.c_int, C.POINTER(C.c_int)]
         L.pfc_finalize.argtypes = [_vp, C.c_int64]
+        L.pfc_set_contact_params.argtypes = [_vp, C.c_int64, _vp]
         L.pfc_eval_f64.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
         L.pfc_eval_f64_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
         L.pfc_eval_dual6.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp]
@@ -161,6 +162,17 @@ class Context:
 
     def finalize(self, max_env: int = 1):
         _check(lib().pfc_finalize(self._h, max_env))
+
+    def set_contact_params(self, params):
+        """Per-environment contact parameters: params[env][ins][8] = (chi, Ebar_1, Ebar_2, q0..q4), q = (mu_s, mu_d, v_c, -, -) for a
+        regularized instruction and (tau, k_bar, mu_s, mu_d, magic) for a bristle one; None clears the table (pfc_set_contact_params)."""
+        if params is None:
+            _check(lib().pfc_set_contact_params(self._h, 0, None))
+            return
+        p = _a(params)
+        if p.ndim != 3 or p.shape[1:] != (self.n_ins, 8):
+            raise ValueError(f"params must have shape [n_env, {self.n_ins}, 8], got {p.shape}")
+        _check(lib().pfc_set_contact_params(self._h, p.shape[0], _p(p)))
 
     def set_debug(self, keep_pairs: bool = True):
         _check(lib().pfc_set_debug(self._h, int(keep_pairs)))

@@ -230,6 +230,7 @@ struct pfc_ctx {
         double h_max = 0.0, tol_newton = 0.0;
         DevBuf<RadauEnv> env;
         DevBuf<double> X, Xp, Fp, taup, xx0, jac, invc, shift, x, tau, t, h;
+        DevBuf<InsParam> paramp, params_c;   // contact-parameter rows gathered per stage state / per compact roll-out slot: grown on first use
         DevBuf<int> index, state_list, env_list, state_pos, inv_base, counts, stats, flags, flags_stage, info;
         DevBuf<long long> np, np_stage;
         // roll-outs (pfc_radau_rollout): grown on first use
@@ -244,6 +245,10 @@ struct pfc_ctx {
     bool timing = false;
     cudaEvent_t ev[8] = {};
     bool ev_valid = false;
+    // per-environment contact parameters (pfc_set_contact_params): rows [env][ins]; params_n_env = 0 while no table is set
+    DevBuf<InsParam> d_params;
+    int64_t params_n_env = 0;
+    const InsParam* last_params = nullptr;   // the table the last evaluation read (pfc_get_traction re-runs its narrow phase)
 };
 
 namespace {
@@ -433,6 +438,19 @@ int pfc_add_instruction(pfc_ctx* c, int mesh_1, int mesh_2, double chi, int mode
     return PFC_OK;
 }
 
+// The contact parameters of an instruction as the kernels use them, from the values a scene is built with (pfc_add_mesh's Ebar,
+// pfc_add_instruction's chi and params): for pfc_finalize's scene table and for every row of a per-environment table alike, so equal
+// values give equal bits.  Ebar1 is 0 for a triangle mesh_1.
+static InsParam derive_contact_params(int model, double chi, double Ebar1, double Ebar2, const double* q) {
+    InsParam d{};
+    d.chi = chi; d.Ebar1 = Ebar1; d.Ebar2 = Ebar2;
+    if (model == 0) { d.p[0] = q[0]; d.p[1] = q[1]; d.p[2] = q[2]; d.p[3] = 2 * q[2]; d.p[4] = 3 * q[2];
+        d.p[5] = (d.p[1] - d.p[0]) / (d.p[4] - d.p[3]); d.p[6] = 1.0 / d.p[2]; }
+    else { d.p[0] = q[0]; d.p[1] = q[1]; d.p[2] = q[2]; d.p[3] = q[3]; d.p[4] = 2 * q[2]; d.p[5] = 3 * q[2]; d.p[6] = q[4];
+        d.p[7] = (d.p[3] - d.p[2]) / (d.p[5] - d.p[4]); }
+    return d;
+}
+
 // Which path every instruction takes, and the device tables that follow from it.
 //   small  n_leaf1 * n_leaf2 <= 512: broad and narrow phase on chip, two launches per batch; the pair list cannot outgrow its slot.
 //   mid    both trees <= kMidLeaves leaves (gripper pads, coarse spheres): the same two kernels with a frontier / pair-list slot of
@@ -461,11 +479,11 @@ static int build_tables(pfc_ctx* c) {
         const bool fits_slot = m1.n_prim * m2.n_prim <= kSmallCap;
         const bool mid = !fits_slot && m1.n_prim <= mid_leaves && m2.n_prim <= mid_leaves && !c->force_large[k];
         d.small = (fits_slot || mid) ? 1 : 0;
-        d.chi = h.chi; d.Ebar1 = m1.kind == 1 ? m1.Ebar : 0.0; d.Ebar2 = m2.Ebar;
-        if (h.model == 0) { d.p[0] = h.params[0]; d.p[1] = h.params[1]; d.p[2] = h.params[2]; d.p[3] = 2 * h.params[2]; d.p[4] = 3 * h.params[2];
-            d.p[5] = (d.p[1] - d.p[0]) / (d.p[4] - d.p[3]); d.p[6] = 1.0 / d.p[2]; }
-        else { d.p[0] = h.params[0]; d.p[1] = h.params[1]; d.p[2] = h.params[2]; d.p[3] = h.params[3]; d.p[4] = 2 * h.params[2]; d.p[5] = 3 * h.params[2]; d.p[6] = h.params[4];
-            d.p[7] = (d.p[3] - d.p[2]) / (d.p[5] - d.p[4]); }
+        {
+            const InsParam cp = derive_contact_params(h.model, h.chi, m1.kind == 1 ? m1.Ebar : 0.0, m2.Ebar, h.params);
+            d.chi = cp.chi; d.Ebar1 = cp.Ebar1; d.Ebar2 = cp.Ebar2;
+            for (int j = 0; j < 8; ++j) d.p[j] = cp.p[j];
+        }
         d.path_base1 = m1.path_base; d.path_base2 = m2.path_base;
         if (d.small) {
             small.push_back(int32_t(k));
@@ -618,9 +636,9 @@ int pfc_finalize(pfc_ctx* c, int64_t max_env) {
 // phase left.  dual: Jacobian mode (every scalar of X / twist / s / wrench / sdot is 7 doubles).  skip_large: a sharded context keeps its
 // large bristle instructions on the partial-sum protocol.  Synchronises the stream once (see exact_bristle_eval).
 static int eval_bristle_exact(pfc_ctx* c, long long n_env, const double* X, const double* twist, const double* s, double* wrench, double* sdot,
-                              const long long* n_pairs, int* flags, int dual, bool skip_large, int* nl, cudaStream_t stream = nullptr) {
+                              const long long* n_pairs, int* flags, const InsParam* params, int dual, bool skip_large, int* nl, cudaStream_t stream = nullptr) {
     if (c->exact_scene.n_bris == 0) return PFC_OK;
-    ExactIO xio{n_env, X, twist, s, wrench, sdot, n_pairs, flags};
+    ExactIO xio{n_env, X, twist, s, wrench, sdot, n_pairs, flags, params};
     ExactPairs ps{};
     ps.small_pairs = c->d_small_pairs.p; ps.small_cap = small_cap(c->small_max_pairs);
     if (c->large_scene.n_large > 0 && c->has_large_bristle && !skip_large) large_exact_view(c->large_buf, c->large_scene, n_env, ps);
@@ -693,7 +711,7 @@ static int eval_device_once(pfc_ctx* c, const EvalIO& io_in) {
     }
     if (beside) {
         CU(cudaStreamWaitEvent(c->stream2, c->ev_fork, 0));
-        int rc = eval_bristle_exact(c, io.n_env, io.X, io.twist, io.s, io.wrench, io.sdot, io.n_pairs, io.flags, 0, false, &nl, c->stream2);
+        int rc = eval_bristle_exact(c, io.n_env, io.X, io.twist, io.s, io.wrench, io.sdot, io.n_pairs, io.flags, io.params, 0, false, &nl, c->stream2);
         if (rc != PFC_OK) return rc;
         CU(cudaEventRecord(c->ev_join, c->stream2));
     }
@@ -705,7 +723,7 @@ static int eval_device_once(pfc_ctx* c, const EvalIO& io_in) {
     if (beside) {
         CU(cudaStreamWaitEvent(c->stream, c->ev_join, 0));
     } else {   // bristle instructions (small and large): reference-order pipeline
-        int rc = eval_bristle_exact(c, io.n_env, io.X, io.twist, io.s, io.wrench, io.sdot, io.n_pairs, io.flags, 0, false, &nl);
+        int rc = eval_bristle_exact(c, io.n_env, io.X, io.twist, io.s, io.wrench, io.sdot, io.n_pairs, io.flags, io.params, 0, false, &nl);
         if (rc != PFC_OK) return rc;
     }
     if (c->n_mid > 0) {
@@ -713,7 +731,7 @@ static int eval_device_once(pfc_ctx* c, const EvalIO& io_in) {
         c->mid_check_pending = true;
     }
     c->launches += nl;
-    c->last_X = io.X; c->last_tw = io.twist;
+    c->last_X = io.X; c->last_tw = io.twist; c->last_params = io.params;
     // the pair lists now belong to this evaluation: pfc_eval_dual6(X_bp = NULL) may reuse them only together with the library's own
     // count / flag arrays (set again by the host-pointer entry points after a successful evaluation)
     c->lists_n_env = -1;
@@ -784,6 +802,7 @@ static unsigned long long eval_key(int kind, const pfc_ctx* c, const EvalIO& io)
     mix((unsigned long long)kind); mix((unsigned long long)io.n_env); mix((unsigned long long)(uintptr_t)io.X); mix((unsigned long long)(uintptr_t)io.twist);
     mix((unsigned long long)(uintptr_t)io.s); mix((unsigned long long)(uintptr_t)io.wrench); mix((unsigned long long)(uintptr_t)io.sdot);
     mix((unsigned long long)(uintptr_t)io.n_pairs); mix((unsigned long long)(uintptr_t)io.flags); mix((unsigned long long)c->shard_rank * 64 + c->shard_world);
+    mix((unsigned long long)(uintptr_t)io.params);   // (a table's buffer, or none: a graph never replays with another table)
     return h ? h : 1;
 }
 
@@ -858,17 +877,61 @@ static void copy_out_finish(pfc_ctx* c) {
     c->arena_out.clear();
 }
 
+// ---- per-environment contact parameters ------------------------------------------------------------------------------------
+// the table of the context (nullptr while none is set) and the batch size it imposes on every evaluation
+static const InsParam* ctx_params(const pfc_ctx* c) { return c->params_n_env > 0 ? c->d_params.p : nullptr; }
+static int params_check(const pfc_ctx* c, const char* who, int64_t n_env) {
+    if (c->params_n_env > 0 && n_env != c->params_n_env)
+        return fail(PFC_E_ARG, std::string(who) + ": n_env differs from the batch of the contact-parameter table (pfc_set_contact_params)");
+    return PFC_OK;
+}
+
+int pfc_set_contact_params(pfc_ctx* c, int64_t n_env, const double* params) {
+    if (!c || !c->finalized) return fail(PFC_E_ARG, "pfc_set_contact_params: call after pfc_finalize");
+    if (n_env < 0 || n_env > c->max_env) return fail(PFC_E_ARG, "pfc_set_contact_params: n_env must be in 0..max_env");
+    if (n_env > 0 && !params) return fail(PFC_E_ARG, "pfc_set_contact_params: params is NULL");
+    CU(cudaSetDevice(c->device));
+    if (n_env == 0) {   // back to the scene's own values (the buffer is kept for the next table)
+        c->params_n_env = 0;
+        return PFC_OK;
+    }
+    const size_t ni = c->ins.size();
+    std::vector<InsParam> rows(size_t(n_env) * ni);
+    for (int64_t e = 0; e < n_env; ++e)
+        for (size_t k = 0; k < ni; ++k) {
+            const double* v = params + 8 * (size_t(e) * ni + k);
+            const HostIns& h = c->ins[k];
+            const bool tet1 = c->mesh[h.mesh_1].kind == 1;
+            const int n_q = h.model == 0 ? 3 : 5;   // the entries the instruction's model uses
+            bool finite = std::isfinite(v[0]) && std::isfinite(v[2]) && (!tet1 || std::isfinite(v[1]));
+            for (int j = 0; j < n_q; ++j) finite = finite && std::isfinite(v[3 + j]);
+            if (!finite)
+                return fail(PFC_E_ARG, "pfc_set_contact_params: non-finite entry (environment " + std::to_string(e) + ", instruction " + std::to_string(k) + ")");
+            rows[size_t(e) * ni + k] = derive_contact_params(h.model, v[0], tet1 ? v[1] : 0.0, v[2], v + 3);
+        }
+    // in stream order behind the evaluations already queued (they read the previous table), and complete before `rows` goes
+    if (rows.size() > c->d_params.n) {
+        c->params_n_env = 0;   // (growing frees the previous table: should the allocation fail, no table is left in force)
+        CU(c->d_params.ensure(rows.size()));
+    }
+    CU(cudaMemcpyAsync(c->d_params.p, rows.data(), sizeof(InsParam) * rows.size(), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    c->params_n_env = n_env;
+    return PFC_OK;
+}
+
 int pfc_eval_f64_device(pfc_ctx* c, int64_t n_env, const double* X, const double* twist, const double* s, double* wrench, double* sdot,
                         int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized) return fail(PFC_E_ARG, "pfc_eval_f64_device: context not finalized");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_eval_f64_device: negative n_env");
+    { const int rc = params_check(c, "pfc_eval_f64_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!X || !twist || !wrench || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_eval_f64_device: NULL buffer");
     if (c->n_bristle > 0 && (!s || !sdot)) return fail(PFC_E_ARG, "pfc_eval_f64_device: bristle instructions need s and sdot");
     CU(cudaSetDevice(c->device));
     EvalIO io{};
     io.n_env = n_env; io.X = X; io.twist = twist; io.s = s; io.wrench = wrench; io.sdot = sdot;
-    io.n_pairs = reinterpret_cast<long long*>(n_pairs); io.flags = flags;
+    io.n_pairs = reinterpret_cast<long long*>(n_pairs); io.flags = flags; io.params = ctx_params(c);
     return eval_device(c, io);
 }
 
@@ -876,6 +939,7 @@ int pfc_eval_f64(pfc_ctx* c, int64_t n_env, const double* X, const double* twist
                  int32_t* flags) {
     if (!c || !c->finalized) return fail(PFC_E_ARG, "pfc_eval_f64: context not finalized");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_eval_f64: negative n_env");
+    { const int rc = params_check(c, "pfc_eval_f64", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!X || !twist || !wrench) return fail(PFC_E_ARG, "pfc_eval_f64: NULL buffer");
     if (c->n_bristle > 0 && (!s || !sdot)) return fail(PFC_E_ARG, "pfc_eval_f64: bristle instructions need s and sdot");
@@ -888,7 +952,7 @@ int pfc_eval_f64(pfc_ctx* c, int64_t n_env, const double* X, const double* twist
     const size_t bX = sizeof(double) * 16 * ne * ni, bT = sizeof(double) * 6 * ne * ni, bS = sizeof(double) * 6 * ne * nb;
     const size_t bW = bT, bD = bS, bN = sizeof(long long) * ne * ni, bF = (sizeof(int32_t) * ne * ni + 7) & ~size_t(7);
     EvalIO io{};
-    io.n_env = n_env;
+    io.n_env = n_env; io.params = ctx_params(c);
     std::vector<int32_t> fl_local;
     int32_t* fl = flags;
     if (!fl) { fl_local.resize(ne * ni); fl = fl_local.data(); }
@@ -914,7 +978,7 @@ int pfc_eval_f64(pfc_ctx* c, int64_t n_env, const double* X, const double* twist
         unsigned long long key = 1469598103934665603ull;
         auto mix = [&](unsigned long long v) { key ^= v; key *= 1099511628211ull; };
         mix(6ull); mix((unsigned long long)n_env); mix((unsigned long long)(uintptr_t)h_in); mix((unsigned long long)(uintptr_t)h_out);
-        mix((unsigned long long)(uintptr_t)di); mix((unsigned long long)(uintptr_t)dn);
+        mix((unsigned long long)(uintptr_t)di); mix((unsigned long long)(uintptr_t)dn); mix((unsigned long long)(uintptr_t)io.params);
         { const int rc = run_host_call(c, c->graph_pack, key, enqueue); if (rc != PFC_OK) return rc; }
         CU(cudaStreamSynchronize(c->stream));
         std::memcpy(wrench, h_out, bW);
@@ -961,7 +1025,7 @@ static int sharded_enqueue(pfc_ctx* c, const EvalIO& io) {
     // every rank lists and evaluates them completely -- identical bits on every rank, nothing to exchange.
     CU(large_broad_phase(c->scene, c->large_scene, io, c->large_buf, c->stream, &nl, c->shard_rank, c->shard_world));
     CU(large_narrow_stage(c->scene, c->large_scene, io, c->large_buf, c->shard_world > 1, 0, c->stream, &nl));
-    int rc = eval_bristle_exact(c, io.n_env, io.X, io.twist, io.s, io.wrench, io.sdot, io.n_pairs, io.flags, 0, false, &nl);
+    int rc = eval_bristle_exact(c, io.n_env, io.X, io.twist, io.s, io.wrench, io.sdot, io.n_pairs, io.flags, nullptr, 0, false, &nl);
     if (rc != PFC_OK) return rc;
     if (c->n_mid > 0) {
         CU(cudaMemcpyAsync(c->h_ins_overflow, c->d_ins_overflow.p, sizeof(int) * c->h_ins.size(), cudaMemcpyDeviceToHost, c->stream));
@@ -979,6 +1043,7 @@ static int sharded_enqueue(pfc_ctx* c, const EvalIO& io) {
 int pfc_eval_sharded_begin(pfc_ctx* c, int64_t n_env, const double* X, const double* twist, const double* s, double* wrench, double* sdot,
                            int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized) return fail(PFC_E_ARG, "pfc_eval_sharded_begin: context not finalized");
+    if (c->params_n_env > 0) return fail(PFC_E_ARG, "pfc_eval_sharded_begin: per-environment contact parameters are not supported by the sharded protocol");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_eval_sharded_begin: negative n_env");
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!X || !twist || !wrench || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_eval_sharded_begin: NULL buffer");
@@ -1061,6 +1126,7 @@ int pfc_comm_init_rank(pfc_ctx* c, const void* id128, int rank, int world) {
 
 int pfc_eval_sharded_f64_device(pfc_ctx* c, int64_t n_env, const double* X, const double* twist, const double* s, double* wrench, double* sdot,
                                 int64_t* n_pairs, int32_t* flags) {
+    if (c && c->params_n_env > 0) return fail(PFC_E_ARG, "pfc_eval_sharded_f64_device: per-environment contact parameters are not supported by the sharded protocol");
     if (!c || !c->comm) return fail(PFC_E_ARG, "pfc_eval_sharded_f64_device: pfc_comm_init_rank (or pfc_group_create) first");
     int rc = pfc_eval_sharded_begin(c, n_env, X, twist, s, wrench, sdot, n_pairs, flags);
     if (rc != PFC_OK || n_env == 0) return rc;
@@ -1131,6 +1197,8 @@ int pfc_group_eval_f64(pfc_group* g, int64_t n_env, const double* X, const doubl
     pfc_ctx* c0 = g->ctx[0];
     if (!c0->finalized) return fail(PFC_E_ARG, "pfc_group_eval_f64: pfc_group_finalize first");
     if (c0->n_bristle > 0 && (!s || !sdot)) return fail(PFC_E_ARG, "pfc_group_eval_f64: bristle instructions need s and sdot");
+    for (pfc_ctx* c : g->ctx)
+        if (c->params_n_env > 0) return fail(PFC_E_ARG, "pfc_group_eval_f64: per-environment contact parameters are not supported by the group protocol");
     if (g->ctx.size() == 1 || c0->large_scene.n_large == 0)   // nothing to split: the plain evaluation on the first device
         return pfc_eval_f64(c0, n_env, X, twist, s, wrench, sdot, n_pairs, flags);
     NcclApi& n = nccl_api();
@@ -1204,6 +1272,7 @@ int pfc_eval_dual6(pfc_ctx* c, int64_t n_env, const double* X_bp, const double* 
                    double* sdot7, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized) return fail(PFC_E_ARG, "pfc_eval_dual6: context not finalized");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_eval_dual6: negative n_env");
+    { const int rc = params_check(c, "pfc_eval_dual6", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!X7 || !twist7 || !wrench7) return fail(PFC_E_ARG, "pfc_eval_dual6: NULL buffer");
     if (c->n_bristle > 0 && (!s7 || !sdot7)) return fail(PFC_E_ARG, "pfc_eval_dual6: bristle instructions need s7 and sdot7");
@@ -1241,9 +1310,10 @@ int pfc_eval_dual6(pfc_ctx* c, int64_t n_env, const double* X_bp, const double* 
         }
         CU(launch_eval_dual6(c->scene, n_env, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->d_w7.p, nb ? c->d_sd7.p : nullptr, np_d, fl_d,
                              c->d_small_pairs.p, small_cap(c->small_max_pairs), c->large_scene.n_large > 0 ? c->large_buf : nullptr, c->d_large_index.p,
-                             c->large_scene.n_large, c->stream, c->d_dual_ticket.p));
+                             c->large_scene.n_large, ctx_params(c), c->stream, c->d_dual_ticket.p));
         {   // bristle instructions on Duals, in the reference's operation order
-            int rc = eval_bristle_exact(c, n_env, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->d_w7.p, nb ? c->d_sd7.p : nullptr, np_d, fl_d, 1, false, &nl);
+            int rc = eval_bristle_exact(c, n_env, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->d_w7.p, nb ? c->d_sd7.p : nullptr, np_d, fl_d, ctx_params(c),
+                                        1, false, &nl);
             if (rc != PFC_OK) return rc;
         }
         c->launches += nl + 1;
@@ -1305,7 +1375,7 @@ int pfc_get_traction(pfc_ctx* c, int64_t env, int ins, double* out, int64_t cap_
     DevBuf<double> d_out; DevBuf<int> d_n;
     CU(d_out.ensure(size_t(8) * cap)); CU(d_n.ensure(1));
     EvalIO io{};
-    io.X = c->last_X; io.twist = c->last_tw;
+    io.X = c->last_X; io.twist = c->last_tw; io.params = c->last_params;
     const int* d_pairs = c->d_dbg_pairs.p + 2 * int64_t(c->dbg_cap) * ei;
     DevBuf<int> d_tmp;
     if (!c->h_ins[ins].small) {  // large instruction: fetch its sorted pair list and stage it as (a, b) ints
@@ -1386,7 +1456,8 @@ static int status_end(pfc_ctx* c, int64_t n_env, bool copy_status = true) {
     return PFC_OK;
 }
 
-static int eval_state_device(pfc_ctx* c, int64_t n_env, const double* x, double* f_gen, double* sdot, long long* n_pairs, int* flags, int* status = nullptr) {
+static int eval_state_device(pfc_ctx* c, int64_t n_env, const double* x, double* f_gen, double* sdot, long long* n_pairs, int* flags, const InsParam* params,
+                             int* status = nullptr) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle);
     CU(c->d_X.ensure(16 * ne * ni)); CU(c->d_tw.ensure(6 * ne * ni)); CU(c->d_w.ensure(6 * ne * ni));
     if (nb) CU(c->d_s.ensure(6 * ne * nb));
@@ -1398,7 +1469,7 @@ static int eval_state_device(pfc_ctx* c, int64_t n_env, const double* x, double*
     CU(launch_state_prologue(c->state, n_env, int(ni), int(nb), x, dX, dtw, ds, c->stream, &nl));
     EvalIO io{};
     io.n_env = n_env; io.X = dX; io.twist = dtw; io.s = ds; io.wrench = dw;
-    io.sdot = sdot; io.n_pairs = n_pairs; io.flags = flags;
+    io.sdot = sdot; io.n_pairs = n_pairs; io.flags = flags; io.params = params;
     int rc = eval_device(c, io);
     if (rc != PFC_OK) return rc;
     CU(launch_state_epilogue(c->state, n_env, int(ni), x, dw, f_gen, c->stream, &nl, flags, status));
@@ -1409,16 +1480,18 @@ static int eval_state_device(pfc_ctx* c, int64_t n_env, const double* x, double*
 int pfc_eval_state_f64_device(pfc_ctx* c, int64_t n_env, const double* x, double* f_generalized, double* sdot, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_bodies) return fail(PFC_E_ARG, "pfc_eval_state_f64_device: pfc_finalize and pfc_set_bodies first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_eval_state_f64_device: negative n_env");
+    { const int rc = params_check(c, "pfc_eval_state_f64_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !f_generalized || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_eval_state_f64_device: NULL buffer");
     if (c->n_bristle > 0 && !sdot) return fail(PFC_E_ARG, "pfc_eval_state_f64_device: bristle instructions need sdot");
     CU(cudaSetDevice(c->device));
-    return eval_state_device(c, n_env, x, f_generalized, sdot, reinterpret_cast<long long*>(n_pairs), flags);
+    return eval_state_device(c, n_env, x, f_generalized, sdot, reinterpret_cast<long long*>(n_pairs), flags, ctx_params(c));
 }
 
 int pfc_eval_state_f64(pfc_ctx* c, int64_t n_env, const double* x, double* f_generalized, double* sdot, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_bodies) return fail(PFC_E_ARG, "pfc_eval_state_f64: pfc_finalize and pfc_set_bodies first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_eval_state_f64: negative n_env");
+    { const int rc = params_check(c, "pfc_eval_state_f64", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !f_generalized) return fail(PFC_E_ARG, "pfc_eval_state_f64: NULL buffer");
     if (c->n_bristle > 0 && !sdot) return fail(PFC_E_ARG, "pfc_eval_state_f64: bristle instructions need sdot");
@@ -1434,7 +1507,7 @@ int pfc_eval_state_f64(pfc_ctx* c, int64_t n_env, const double* x, double* f_gen
         // slower -- 379 vs 325 us for 4096 environments: half-size grids no longer fill the GPU and the extra launches / events cost more
         // than the ~50 us of copies they hide.)
         CU(cudaMemcpyAsync(c->d_x.p, x, sizeof(double) * ne * nx, cudaMemcpyHostToDevice, c->stream));
-        int rc = eval_state_device(c, n_env, c->d_x.p, c->d_fgen.p, nb ? c->d_sd.p : nullptr, c->d_np.p, c->d_fl.p, c->d_status.p);
+        int rc = eval_state_device(c, n_env, c->d_x.p, c->d_fgen.p, nb ? c->d_sd.p : nullptr, c->d_np.p, c->d_fl.p, ctx_params(c), c->d_status.p);
         if (rc != PFC_OK) return rc;
         CU(cudaMemcpyAsync(f_generalized, c->d_fgen.p, sizeof(double) * ne * nv, cudaMemcpyDeviceToHost, c->stream));
         if (nb) CU(cudaMemcpyAsync(sdot, c->d_sd.p, sizeof(double) * 6 * ne * nb, cudaMemcpyDeviceToHost, c->stream));
@@ -1447,6 +1520,7 @@ int pfc_eval_state_f64(pfc_ctx* c, int64_t n_env, const double* x, double* f_gen
     auto mix = [&](unsigned long long v) { key ^= v; key *= 1099511628211ull; };
     mix(5ull); mix((unsigned long long)n_env); mix((unsigned long long)(uintptr_t)x); mix((unsigned long long)(uintptr_t)f_generalized);
     mix((unsigned long long)(uintptr_t)sdot); mix((unsigned long long)(uintptr_t)n_pairs); mix((unsigned long long)(uintptr_t)flags);
+    mix((unsigned long long)(uintptr_t)ctx_params(c));
     { const int rc = run_host_call(c, c->graph_host, key, enqueue); if (rc != PFC_OK) return rc; }
     return status_end(c, n_env, false);
 }
@@ -1493,7 +1567,8 @@ int pfc_set_dynamics(pfc_ctx* c, int n_body, const double* spatial_inertia, cons
     return PFC_OK;
 }
 
-static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* xdot, long long* n_pairs, int* flags, int* status = nullptr) {
+static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, double* xdot, long long* n_pairs, int* flags,
+                         int* status = nullptr) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle);
     CU(c->d_X.ensure(16 * ne * ni)); CU(c->d_tw.ensure(6 * ne * ni)); CU(c->d_w.ensure(6 * ne * ni));
     if (nb) { CU(c->d_s.ensure(6 * ne * nb)); CU(c->d_sd.ensure(6 * ne * nb)); }
@@ -1501,7 +1576,7 @@ static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const doubl
     CU(launch_state_prologue(c->state, n_env, int(ni), int(nb), x, c->d_X.p, c->d_tw.p, nb ? c->d_s.p : nullptr, c->stream, &nl));
     EvalIO io{};
     io.n_env = n_env; io.X = c->d_X.p; io.twist = c->d_tw.p; io.s = nb ? c->d_s.p : nullptr; io.wrench = c->d_w.p;
-    io.sdot = nb ? c->d_sd.p : nullptr; io.n_pairs = n_pairs; io.flags = flags;
+    io.sdot = nb ? c->d_sd.p : nullptr; io.n_pairs = n_pairs; io.flags = flags; io.params = params;
     int rc = eval_device(c, io);
     if (rc != PFC_OK) return rc;
     CU(launch_state_dynamics(c->state, c->dyn, n_env, int(ni), int(nb), x, c->d_w.p, tau_ext, nb ? c->d_sd.p : nullptr, xdot, c->stream, &nl, flags, status));
@@ -1512,15 +1587,17 @@ static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const doubl
 int pfc_calcxd_f64_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* xdot, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: negative n_env");
+    { const int rc = params_check(c, "pfc_calcxd_f64_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: NULL buffer");
     CU(cudaSetDevice(c->device));
-    return calcxd_device(c, n_env, x, tau_ext, xdot, reinterpret_cast<long long*>(n_pairs), flags);
+    return calcxd_device(c, n_env, x, tau_ext, ctx_params(c), xdot, reinterpret_cast<long long*>(n_pairs), flags);
 }
 
 int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* xdot, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_f64: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_f64: negative n_env");
+    { const int rc = params_check(c, "pfc_calcxd_f64", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot) return fail(PFC_E_ARG, "pfc_calcxd_f64: NULL buffer");
     CU(cudaSetDevice(c->device));
@@ -1533,7 +1610,7 @@ int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau
     }
     CU(cudaMemsetAsync(c->d_xdot.p, 0, sizeof(double) * ne * nx, c->stream));
     CU(status_begin(c));
-    int rc = calcxd_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = calcxd_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(xdot, c->d_xdot.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     if (n_pairs) CU(cudaMemcpyAsync(n_pairs, c->d_np.p, sizeof(long long) * ne * ni, cudaMemcpyDeviceToHost, c->stream));
@@ -1544,18 +1621,18 @@ int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau
 // The Float64 part the seed chunks of a Jacobian share: candidate-pair lists, the wrenches of the regularized instructions (problems whose
 // inputs do not depend on a chunk's seeds copy them) and, for the small instructions, the pairs that survive the Float64 clip.
 // Expects the Float64 boundary arrays in c->d_X / c->d_tw.
-static int dual_shared_f64(pfc_ctx* c, int64_t n_env, long long* n_pairs, int* flags, DualShared* sh, int* nl) {
+static int dual_shared_f64(pfc_ctx* c, int64_t n_env, long long* n_pairs, int* flags, const InsParam* params, DualShared* sh, int* nl) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins);
     CU(c->d_w.ensure(6 * ne * ni));
     EvalIO io{};
-    io.n_env = n_env; io.X = c->d_X.p; io.twist = c->d_tw.p; io.wrench = c->d_w.p; io.n_pairs = n_pairs; io.flags = flags;
+    io.n_env = n_env; io.X = c->d_X.p; io.twist = c->d_tw.p; io.wrench = c->d_w.p; io.n_pairs = n_pairs; io.flags = flags; io.params = params;
     sh->surv_pairs = nullptr; sh->surv_n = nullptr; sh->w_f64 = c->d_w.p;
     if (c->scene.n_small > 0) {
         const int cap = small_cap(c->small_max_pairs);
         CU(c->d_small_pairs.ensure(size_t(cap) * ne * ni + kSmallPairsSlack));
         CU(launch_eval_small_f64(c->scene, io, c->small_max_pairs, c->d_small_pairs.p, c->stream, nl, nullptr));
         CU(c->d_surv.ensure(size_t(cap) * ne * ni)); CU(c->d_surv_n.ensure(ne * ni));
-        CU(launch_dual_prefilter(c->scene, n_env, c->d_X.p, n_pairs, c->d_small_pairs.p, cap, c->d_surv.p, c->d_surv_n.p, c->stream));
+        CU(launch_dual_prefilter(c->scene, n_env, c->d_X.p, n_pairs, c->d_small_pairs.p, cap, c->d_surv.p, c->d_surv_n.p, params, c->stream));
         *nl += 1;
         sh->surv_pairs = c->d_surv.p; sh->surv_n = c->d_surv_n.p;
     }
@@ -1575,8 +1652,8 @@ static int dual_shared_f64(pfc_ctx* c, int64_t n_env, long long* n_pairs, int* f
 // calcXd! in Jacobian mode for the same scenes: x (Float64) with Dual seeds on x[seed_start .. seed_start + 6) -> x_dot as 7 doubles per
 // entry (value, then d x_dot / d x[seed_start + k]).  Device pipeline: Float64 prologue + broad phase (the reference always traverses
 // with m.float), Dual prologue, Dual narrow phase / friction (pfc_dual.cu), Dual J' w and rigid-body terms.
-static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, int seed_start, double* xdot7, long long* n_pairs,
-                                    int* flags, int* status) {
+static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, int seed_start, double* xdot7,
+                                    long long* n_pairs, int* flags, int* status) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle);
     CU(c->d_X.ensure(16 * ne * ni)); CU(c->d_tw.ensure(6 * ne * ni));
     CU(c->d_X7.ensure(112 * ne * ni)); CU(c->d_tw7.ensure(42 * ne * ni)); CU(c->d_w7.ensure(42 * ne * ni)); CU(c->d_dual_ticket.ensure(1));
@@ -1585,14 +1662,15 @@ static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, 
     // Float64 boundary arrays -> candidate-pair lists, Float64 wrenches, survivors of the Float64 clip
     CU(launch_state_prologue(c->state, n_env, int(ni), int(nb), x, c->d_X.p, c->d_tw.p, nb ? c->d_s.p : nullptr, c->stream, &nl));
     DualShared shared{};
-    { const int rc = dual_shared_f64(c, n_env, n_pairs, flags, &shared, &nl); if (rc != PFC_OK) return rc; }
+    { const int rc = dual_shared_f64(c, n_env, n_pairs, flags, params, &shared, &nl); if (rc != PFC_OK) return rc; }
     // Dual boundary arrays, Dual contact wrenches, Dual rigid-body terms
     CU(launch_state_prologue_dual6(c->state, n_env, int(ni), int(nb), x, seed_start, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->stream, &nl));
     CU(launch_eval_dual6(c->scene, n_env, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->d_w7.p, nb ? c->d_sd7.p : nullptr, n_pairs, flags,
                          c->d_small_pairs.p, small_cap(c->small_max_pairs), c->large_scene.n_large > 0 ? c->large_buf : nullptr, c->d_large_index.p,
-                         c->large_scene.n_large, c->stream, c->d_dual_ticket.p, 0, &shared));
+                         c->large_scene.n_large, params, c->stream, c->d_dual_ticket.p, 0, &shared));
     {
-        int rc = eval_bristle_exact(c, n_env, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->d_w7.p, nb ? c->d_sd7.p : nullptr, n_pairs, flags, 1, false, &nl);
+        int rc = eval_bristle_exact(c, n_env, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->d_w7.p, nb ? c->d_sd7.p : nullptr, n_pairs, flags, params, 1, false,
+                                    &nl);
         if (rc != PFC_OK) return rc;
     }
     CU(launch_state_dynamics_dual6(c->state, c->dyn, n_env, int(ni), int(nb), x, seed_start, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr, xdot7,
@@ -1600,9 +1678,9 @@ static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, 
     c->launches += nl + 1;
     return PFC_OK;
 }
-static int calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, int seed_start, double* xdot7, long long* n_pairs,
-                               int* flags, int* status) {
-    PFC_REQUEUE_LOOP({ const int rc_ = calcxd_dual6_device_once(c, n_env, x, tau_ext, seed_start, xdot7, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
+static int calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, int seed_start, double* xdot7,
+                               long long* n_pairs, int* flags, int* status) {
+    PFC_REQUEUE_LOOP({ const int rc_ = calcxd_dual6_device_once(c, n_env, x, tau_ext, params, seed_start, xdot7, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
     return PFC_OK;
 }
 
@@ -1610,16 +1688,18 @@ int pfc_calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const do
                             int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: negative n_env");
+    { const int rc = params_check(c, "pfc_calcxd_dual6_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot7 || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: NULL buffer");
     if (seed_start < 0 || seed_start >= c->state.n_x) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: seed_start out of range");
     CU(cudaSetDevice(c->device));
-    return calcxd_dual6_device(c, n_env, x, tau_ext, seed_start, xdot7, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
+    return calcxd_dual6_device(c, n_env, x, tau_ext, ctx_params(c), seed_start, xdot7, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
 }
 
 int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, int seed_start, double* xdot7, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_dual6: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_dual6: negative n_env");
+    { const int rc = params_check(c, "pfc_calcxd_dual6", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot7) return fail(PFC_E_ARG, "pfc_calcxd_dual6: NULL buffer");
     if (seed_start < 0 || seed_start >= c->state.n_x) return fail(PFC_E_ARG, "pfc_calcxd_dual6: seed_start out of range");
@@ -1633,7 +1713,7 @@ int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* t
     }
     CU(cudaMemsetAsync(c->d_xdot.p, 0, sizeof(double) * 7 * ne * nx, c->stream));
     CU(status_begin(c));
-    int rc = calcxd_dual6_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, seed_start, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = calcxd_dual6_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), seed_start, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(xdot7, c->d_xdot.p, sizeof(double) * 7 * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     if (n_pairs) CU(cudaMemcpyAsync(n_pairs, c->d_np.p, sizeof(long long) * ne * ni, cudaMemcpyDeviceToHost, c->stream));
@@ -1648,8 +1728,8 @@ int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* t
 // seed chunks are a grid axis of the Dual kernels ("environment" (g, env) = chunk g of real environment env) as far as the work space
 // allows, and the rigid-body kernel writes the partials straight into jac[env][row][col].  Scenes with bristle instructions go chunk by
 // chunk (their reference-order pipeline is sized per real environment) but still share the broad phase.
-static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* jac, double* xdot, long long* n_pairs,
-                                int* flags, int* status) {
+static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, double* jac, double* xdot,
+                                long long* n_pairs, int* flags, int* status) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle), nx = size_t(c->state.n_x);
     const int n_chunk = int((nx + 5) / 6);
     // chunks per pass: all of them if the Dual boundary arrays (196 doubles per (chunk, environment, instruction)) stay below 1 GiB
@@ -1662,17 +1742,17 @@ static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, cons
     int nl = 0;
     CU(launch_state_prologue(c->state, n_env, int(ni), int(nb), x, c->d_X.p, c->d_tw.p, nb ? c->d_s.p : nullptr, c->stream, &nl));
     DualShared shared{};
-    { const int rc = dual_shared_f64(c, n_env, n_pairs, flags, &shared, &nl); if (rc != PFC_OK) return rc; }
+    { const int rc = dual_shared_f64(c, n_env, n_pairs, flags, params, &shared, &nl); if (rc != PFC_OK) return rc; }
     for (int g0 = 0; g0 < n_chunk; g0 += G) {
         const int g = std::min(G, n_chunk - g0);
         const long long n_virtual = n_env * g;
         CU(launch_state_prologue_dual6(c->state, n_virtual, int(ni), int(nb), x, 6 * g0, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->stream, &nl, n_env));
         CU(launch_eval_dual6(c->scene, n_virtual, c->d_X7.p, c->d_tw7.p, nb ? c->d_s7.p : nullptr, c->d_w7.p, nb ? c->d_sd7.p : nullptr, n_pairs, flags,
                              c->d_small_pairs.p, small_cap(c->small_max_pairs), c->large_scene.n_large > 0 ? c->large_buf : nullptr, c->d_large_index.p,
-                             c->large_scene.n_large, c->stream, c->d_dual_ticket.p, n_env, &shared));
+                             c->large_scene.n_large, params, c->stream, c->d_dual_ticket.p, n_env, &shared));
         nl += 1;
         if (nb) {
-            int rc = eval_bristle_exact(c, n_env, c->d_X7.p, c->d_tw7.p, c->d_s7.p, c->d_w7.p, c->d_sd7.p, n_pairs, flags, 1, false, &nl);
+            int rc = eval_bristle_exact(c, n_env, c->d_X7.p, c->d_tw7.p, c->d_s7.p, c->d_w7.p, c->d_sd7.p, n_pairs, flags, params, 1, false, &nl);
             if (rc != PFC_OK) return rc;
         }
         CU(launch_state_dynamics_dual6(c->state, c->dyn, n_virtual, int(ni), int(nb), x, 6 * g0, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr,
@@ -1681,9 +1761,9 @@ static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, cons
     c->launches += nl;
     return PFC_OK;
 }
-static int jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* jac, double* xdot, long long* n_pairs, int* flags,
-                           int* status) {
-    PFC_REQUEUE_LOOP({ const int rc_ = jacobian_device_once(c, n_env, x, tau_ext, jac, xdot, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
+static int jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, double* jac, double* xdot,
+                           long long* n_pairs, int* flags, int* status) {
+    PFC_REQUEUE_LOOP({ const int rc_ = jacobian_device_once(c, n_env, x, tau_ext, params, jac, xdot, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
     return PFC_OK;
 }
 
@@ -1691,15 +1771,17 @@ int pfc_calcxd_jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const
                                int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: negative n_env");
+    { const int rc = params_check(c, "pfc_calcxd_jacobian_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !jac || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: NULL buffer");
     CU(cudaSetDevice(c->device));
-    return jacobian_device(c, n_env, x, tau_ext, jac, xdot, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
+    return jacobian_device(c, n_env, x, tau_ext, ctx_params(c), jac, xdot, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
 }
 
 int pfc_calcxd_jacobian(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* jac, double* xdot, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: negative n_env");
+    { const int rc = params_check(c, "pfc_calcxd_jacobian", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !jac) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: NULL buffer");
     CU(cudaSetDevice(c->device));
@@ -1711,7 +1793,7 @@ int pfc_calcxd_jacobian(pfc_ctx* c, int64_t n_env, const double* x, const double
         CU(cudaMemcpyAsync(c->d_tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
     }
     CU(status_begin(c));
-    int rc = jacobian_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, c->d_jac.p, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = jacobian_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), c->d_jac.p, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(jac, c->d_jac.p, sizeof(double) * ne * nx * nx, cudaMemcpyDeviceToHost, c->stream));
     if (xdot) CU(cudaMemcpyAsync(xdot, c->d_xdot.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
@@ -1778,6 +1860,7 @@ int pfc_radau_inv_c_device(pfc_ctx* c, int64_t n_mat, int n, const double* neg_J
 int pfc_radau_init(pfc_ctx* c, int64_t n_env, int max_rule, double h0, double h_max, double tol_newton) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_radau_init: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_radau_init: negative n_env");
+    { const int rc = params_check(c, "pfc_radau_init", n_env); if (rc != PFC_OK) return rc; }
     if (max_rule < 1 || max_rule > kRadauMaxRule) return fail(PFC_E_ARG, "pfc_radau_init: max_rule must be 1, 2 or 3");
     if (c->state.n_x < 1 || c->state.n_x > 96) return fail(PFC_E_ARG, "pfc_radau_init: the state must have 1 to 96 entries");
     if (!(std::isfinite(h0) && h0 > 0.0) || !(std::isfinite(h_max) && h_max > 0.0)) return fail(PFC_E_ARG, "pfc_radau_init: h0 and h_max must be finite and positive");
@@ -1804,7 +1887,7 @@ static int radau_check(pfc_ctx* c, const char* who, int64_t n_env) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, std::string(who) + ": pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (c->radau.n_env < 0) return fail(PFC_E_ARG, std::string(who) + ": pfc_radau_init first");
     if (n_env != c->radau.n_env) return fail(PFC_E_ARG, std::string(who) + ": n_env differs from the one given to pfc_radau_init");
-    return PFC_OK;
+    return params_check(c, who, n_env);
 }
 
 static void radau_info_reset(pfc_ctx::RadauState& r) {
@@ -1816,7 +1899,9 @@ static void radau_info_reset(pfc_ctx::RadauState& r) {
 // iteration (how many stage states are still active); the error bits of every evaluation that counts ride along with them.
 // The buffer set is the caller's: the context's own for pfc_radau_step, the compact sub-batch of a roll-out round; the work space is sized
 // for pfc_radau_init's n_env, which n_env never exceeds.  The step info (rounds, synchronisations, phase times) is added to.
-static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
+// params: the contact-parameter rows [env][ins] of these environments (or nullptr); they travel like tau_ext, gathered per stage state.
+static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x, const double* tau_ext, const InsParam* params, double* t, double* h_taken,
+                             int32_t* stats) {
     pfc_ctx::RadauState& r = c->radau;
     const int nx = c->state.n_x, nv = c->state.nv, ni = c->scene.n_ins;
     RadauBufs b{};
@@ -1825,6 +1910,10 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
     b.X = r.X.p; b.Xp = r.Xp.p; b.Fp = r.Fp.p; b.taup = r.taup.p; b.xx0 = r.xx0.p; b.jac = r.jac.p; b.invc = r.invc.p; b.shift = r.shift.p;
     b.index = r.index.p; b.state_list = r.state_list.p; b.env_list = r.env_list.p; b.state_pos = r.state_pos.p; b.inv_base = r.inv_base.p;
     b.counts = r.counts.p; b.bodies = c->d_bodies.p; b.n_body = c->state.n_body;
+    if (params) {
+        CU(r.paramp.ensure(std::max<size_t>(size_t(r.n_env) * r.s_max * ni, 1)));
+        b.params = params; b.paramp = r.paramp.p;
+    }
     // phase timing (pfc_set_timing): events around every phase, read after the step's last synchronisation
     std::vector<std::pair<int, int>> marks;   // (phase, index of its start event; the end event follows)
     std::vector<cudaEvent_t>& pool = r.ev_pool;
@@ -1850,7 +1939,7 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
     CU(cudaMemsetAsync(r.counts.p, 0, 4 * sizeof(int), c->stream));
     // calcJacobian! once per step: xx_0 and -J (a retry reuses them, radau_solve.jl:23-28)
     CU(mark(0, true));
-    { const int rc = jacobian_device(c, n_env, x, tau_ext, r.jac.p, r.xx0.p, r.np.p, r.flags.p, nullptr); if (rc != PFC_OK) return rc; }
+    { const int rc = jacobian_device(c, n_env, x, tau_ext, params, r.jac.p, r.xx0.p, r.np.p, r.flags.p, nullptr); if (rc != PFC_OK) return rc; }
     CU(launch_radau_prepare(b, r.flags.p, c->d_status.p, c->stream));
     CU(mark(0, false));
     c->launches += 1;
@@ -1874,7 +1963,8 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
             CU(mark(1, true));
             CU(launch_radau_gather(b, n_states, c->stream));
             CU(cudaMemsetAsync(r.Fp.p, 0, sizeof(double) * size_t(n_states) * nx, c->stream));
-            { const int rc = calcxd_device(c, n_states, r.Xp.p, tau_ext ? r.taup.p : nullptr, r.Fp.p, r.np_stage.p, r.flags_stage.p, c->d_status.p); if (rc != PFC_OK) return rc; }
+            { const int rc = calcxd_device(c, n_states, r.Xp.p, tau_ext ? r.taup.p : nullptr, params ? r.paramp.p : nullptr, r.Fp.p, r.np_stage.p, r.flags_stage.p,
+                                          c->d_status.p); if (rc != PFC_OK) return rc; }
             CU(mark(1, false));
             CU(mark(3, true));
             CU(launch_radau_newton(b, n_active, c->stream));
@@ -1903,7 +1993,7 @@ int pfc_radau_step_device(pfc_ctx* c, int64_t n_env, double* x, const double* ta
     if (!x || !t || !h_taken) return fail(PFC_E_ARG, "pfc_radau_step_device: NULL buffer");
     CU(cudaSetDevice(c->device));
     radau_info_reset(c->radau);
-    return radau_step_device(c, n_env, c->radau.env.p, x, tau_ext, t, h_taken, stats);
+    return radau_step_device(c, n_env, c->radau.env.p, x, tau_ext, ctx_params(c), t, h_taken, stats);
 }
 
 int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
@@ -1919,7 +2009,7 @@ int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, 
     CU(cudaMemcpyAsync(r.t.p, t, sizeof(double) * ne, cudaMemcpyHostToDevice, c->stream));
     if (tau_ext) CU(cudaMemcpyAsync(r.tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
     radau_info_reset(r);
-    const int rc = radau_step_device(c, n_env, r.env.p, r.x.p, tau_ext ? r.tau.p : nullptr, r.t.p, r.h.p, r.stats.p);
+    const int rc = radau_step_device(c, n_env, r.env.p, r.x.p, tau_ext ? r.tau.p : nullptr, ctx_params(c), r.t.p, r.h.p, r.stats.p);
     if (rc != PFC_OK) { cudaStreamSynchronize(c->stream); return rc; }
     CU(cudaMemcpyAsync(x, r.x.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(t, r.t.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
@@ -1950,11 +2040,14 @@ static int radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const dou
     CU(r.knots.ensure(size_t(n_knot))); CU(r.knot.ensure(ne)); CU(r.steps.ensure(ne)); CU(r.ro_stats.ensure(4 * ne)); CU(r.list.ensure(ne));
     CU(r.env_c.ensure(ne)); CU(r.x_c.ensure(ne * nx)); CU(r.tau_c.ensure(ne * std::max<size_t>(nv, 1))); CU(r.t_c.ensure(ne)); CU(r.h_c.ensure(ne));
     CU(r.h_save.ensure(ne)); CU(r.stats_c.ensure(4 * ne)); CU(r.ro_count.ensure(2));
+    const InsParam* params = ctx_params(c);
+    if (params) CU(r.params_c.ensure(ne * size_t(c->scene.n_ins)));
     RadauRolloutBufs b{};
     b.n_env = n_env; b.max_steps = max_steps; b.nx = int(nx); b.nv = int(nv); b.n_knot = n_knot;
     b.knots = r.knots.p; b.env = r.env.p; b.x = x; b.tau = tau_ext; b.t = t; b.x_knot = x_knot; b.knot = r.knot.p; b.steps = r.steps.p;
     b.stats = r.ro_stats.p; b.list = r.list.p; b.env_c = r.env_c.p; b.x_c = r.x_c.p; b.tau_c = r.tau_c.p; b.t_c = r.t_c.p; b.h_c = r.h_c.p;
     b.h_save = r.h_save.p; b.stats_c = r.stats_c.p; b.count = r.ro_count.p;
+    b.params = params; b.params_c = params ? r.params_c.p : nullptr; b.n_ins = c->scene.n_ins;
     radau_info_reset(r);
     CU(cudaMemcpyAsync(r.knots.p, t_knot, sizeof(double) * n_knot, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemsetAsync(r.knot.p, 0, sizeof(int) * ne, c->stream));
@@ -1970,7 +2063,8 @@ static int radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const dou
         if (round == 0 && x_knot) CU(cudaMemsetAsync(x_knot, 0xFF, sizeof(double) * n_knot * ne * nx, c->stream));   // all-ones bytes: a NaN
         const long long n_active = r.h_counts[5];
         if (n_active == 0) break;
-        { const int rc = radau_step_device(c, n_active, r.env_c.p, r.x_c.p, tau_ext ? r.tau_c.p : nullptr, r.t_c.p, r.h_c.p, r.stats_c.p); if (rc != PFC_OK) return rc; }
+        { const int rc = radau_step_device(c, n_active, r.env_c.p, r.x_c.p, tau_ext ? r.tau_c.p : nullptr, params ? r.params_c.p : nullptr, r.t_c.p, r.h_c.p,
+                                           r.stats_c.p); if (rc != PFC_OK) return rc; }
         CU(launch_radau_finish(b, n_active, c->stream));
         c->launches += 1;
     }

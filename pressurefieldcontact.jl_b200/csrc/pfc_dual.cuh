@@ -17,6 +17,7 @@ struct DualIO {
     int* flags;             // [env][ins]
     long long n_real;       // whole-Jacobian mode: the n_env "environments" are n_env / n_real seed chunks of n_real real ones
                             // (chunk-major); pair lists, counts and flags exist once per REAL environment.  Otherwise = n_env.
+    const InsParam* params; // [real env][ins] contact parameters, or nullptr for the scene's own
 };
 
 // pair list access for both paths

@@ -50,6 +50,7 @@ struct DualTileSmem {
     long long ei[kDP], er[kDP];   // problem index among the (chunk, env, ins) entries / among the real (env, ins) ones; ei = -1: nothing to do
     const unsigned* pl_s[kDP];
     const int3* pl_l[kDP];
+    const double* fp[kDP];        // friction parameters of problem q (InsDev::p, or its environment's row of the parameter table)
     int ins[kDP], seeded[kDP], pflags[kDP], prefiltered[kDP], copied[kDP];
     int pre[kDP + 1];             // candidates before problem q
     int surv_a[kDT], surv_b[kDT];
@@ -80,7 +81,8 @@ PFC_D int block_scan_excl(int v, int* warp_tot, int& total) {
 // packed in candidate order, are what every seed chunk of the Jacobian works on (two thirds of the candidates clip to nothing).  One warp
 // per problem, 32 candidates per pass.
 __global__ void __launch_bounds__(128) dual_prefilter_kernel(SceneDev sc, long long n_env, const double* __restrict__ X, const long long* __restrict__ n_pairs,
-                                                             const unsigned* __restrict__ pairs, int cap, unsigned* __restrict__ surv, int* __restrict__ surv_n) {
+                                                             const unsigned* __restrict__ pairs, int cap, unsigned* __restrict__ surv, int* __restrict__ surv_n,
+                                                             const InsParam* __restrict__ params) {
     const int lane = threadIdx.x & 31;
     const long long n_prob = n_env * sc.n_ins;
     for (long long ei = (long long)blockIdx.x * 4 + (threadIdx.x >> 5); ei < n_prob; ei += (long long)gridDim.x * 4) {
@@ -100,7 +102,9 @@ __global__ void __launch_bounds__(128) dual_prefilter_kernel(SceneDev sc, long l
         }
         cx.x12 = inverse(cx.x21);
         cx.w_ang = mk<double>(0.0, 0.0, 0.0); cx.w_lin = cx.w_ang;
-        cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; cx.n_quad = ins.n_quad;
+        if (params) { cx.chi = params[ei].chi; cx.Ebar1 = params[ei].Ebar1; cx.Ebar2 = params[ei].Ebar2; }
+        else { cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; }
+        cx.n_quad = ins.n_quad;
         const unsigned* in = pairs + (size_t)cap * ei;
         unsigned* out = surv + (size_t)cap * ei;
         int kept = 0;
@@ -135,6 +139,7 @@ __global__ void __launch_bounds__(kDT) eval_dual6_tile_kernel(SceneDev sc, DualI
                 const InsDev& ins = sc.ins[k];
                 if (ins.model == PFC_MODEL_REGULARIZED) {   // bristle: pfc_exact.cu
                     active = true;
+                    const InsParam* cp = io.params ? io.params + er : nullptr;   // the real environment's contact parameters, if it has its own
                     const double* Xp = io.X7 + 112 * ei;
                     const double* tw = io.twist7 + 42 * ei;
                     bool mine_x = false, mine_t = false;   // does the transform / the twist depend on the seeds?  (lanes share the 18 x 6 partials)
@@ -158,7 +163,9 @@ __global__ void __launch_bounds__(kDT) eval_dual6_tile_kernel(SceneDev sc, DualI
                         cx.x12 = inverse(cx.x21);
                         cx.w_ang = mk<D2>(ld(tw), ld(tw + 7), ld(tw + 14));
                         cx.w_lin = mk<D2>(ld(tw + 21), ld(tw + 28), ld(tw + 35));
-                        cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; cx.n_quad = ins.n_quad;
+                        if (cp) { cx.chi = cp->chi; cx.Ebar1 = cp->Ebar1; cx.Ebar2 = cp->Ebar2; }
+                        else { cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; }
+                        cx.n_quad = ins.n_quad;
                     }
                     __syncwarp();
                     if (lane == 0) {
@@ -173,7 +180,7 @@ __global__ void __launch_bounds__(kDT) eval_dual6_tile_kernel(SceneDev sc, DualI
                             cxv.w_lin = mk<double>(c0.w_lin.x.v, c0.w_lin.y.v, c0.w_lin.z.v);
                             cxv.chi = c0.chi; cxv.Ebar1 = c0.Ebar1; cxv.Ebar2 = c0.Ebar2; cxv.n_quad = c0.n_quad;
                         }
-                        sm.ei[q] = ei; sm.er[q] = er; sm.ins[q] = k; sm.seeded[q] = seeded; sm.pflags[q] = 0;
+                        sm.ei[q] = ei; sm.er[q] = er; sm.ins[q] = k; sm.seeded[q] = seeded; sm.pflags[q] = 0; sm.fp[q] = cp ? cp->p : ins.p;
                         const bool pf = ins.small && ps.surv_pairs;       // survivors of the Float64 clip are listed already
                         const bool cp = seeded == 0 && ps.w_f64;          // nothing to differentiate and the values exist: copy them
                         sm.prefiltered[q] = pf ? 1 : 0; sm.copied[q] = cp ? 1 : 0;
@@ -183,7 +190,7 @@ __global__ void __launch_bounds__(kDT) eval_dual6_tile_kernel(SceneDev sc, DualI
                     }
                 }
             }
-            if (!active && lane == 0) { sm.ei[q] = -1; sm.er[q] = 0; sm.ins[q] = 0; sm.seeded[q] = 0; sm.pflags[q] = 0; sm.pre[q + 1] = 0; sm.pl_s[q] = nullptr; sm.pl_l[q] = nullptr; sm.prefiltered[q] = 0; sm.copied[q] = 0; }
+            if (!active && lane == 0) { sm.fp[q] = nullptr; sm.ei[q] = -1; sm.er[q] = 0; sm.ins[q] = 0; sm.seeded[q] = 0; sm.pflags[q] = 0; sm.pre[q + 1] = 0; sm.pl_s[q] = nullptr; sm.pl_l[q] = nullptr; sm.prefiltered[q] = 0; sm.copied[q] = 0; }
             for (int j = lane; j <= kTotStride; j += 32) sm.tot[q][j] = 0.0;
         }
         __syncthreads();
@@ -239,7 +246,7 @@ __global__ void __launch_bounds__(kDT) eval_dual6_tile_kernel(SceneDev sc, DualI
                     if (sm.seeded[sq] == 2) {          // the transform carries partials: the whole pair on Dual<2>, this item's 2 partials
                         const PatchCtx<D2>& cx = sm.cx[sq][chunk];
                         Accum<D2, 6> acc;
-                        acc.fp = ins.p; acc.w_ang = cx.w_ang; acc.w_lin = cx.w_lin; acc.dump = nullptr; acc.dump_cap = 0;
+                        acc.fp = sm.fp[sq]; acc.w_ang = cx.w_ang; acc.w_lin = cx.w_lin; acc.dump = nullptr; acc.dump_cap = 0;
                         acc.reset(ACC_REGULARIZED);
                         integrate_pair(sc, ins, sm.surv_a[lo], sm.surv_b[lo], cx, acc, flags);
 #pragma unroll
@@ -254,7 +261,7 @@ __global__ void __launch_bounds__(kDT) eval_dual6_tile_kernel(SceneDev sc, DualI
                         for (int c3 = 0; c3 < 3; ++c3) {
                             const PatchCtx<D2>& cx = sm.cx[sq][c3];
                             TwistAcc<2> acc;
-                            acc.fp = ins.p; acc.w_ang = cx.w_ang; acc.w_lin = cx.w_lin; acc.n_points = 0;
+                            acc.fp = sm.fp[sq]; acc.w_ang = cx.w_ang; acc.w_lin = cx.w_lin; acc.n_points = 0;
 #pragma unroll
                             for (int j = 0; j < 6; ++j) acc.a[j] = D2(0.0);
                             if (hit) {
@@ -272,7 +279,7 @@ __global__ void __launch_bounds__(kDT) eval_dual6_tile_kernel(SceneDev sc, DualI
                     } else {                            // nothing does: the Float64 evaluation
                         const PatchCtx<double>& cx = sm.cxv[sq];
                         Accum<double, 6> acc;
-                        acc.fp = ins.p; acc.w_ang = cx.w_ang; acc.w_lin = cx.w_lin; acc.dump = nullptr; acc.dump_cap = 0;
+                        acc.fp = sm.fp[sq]; acc.w_ang = cx.w_ang; acc.w_lin = cx.w_lin; acc.dump = nullptr; acc.dump_cap = 0;
                         acc.reset(ACC_REGULARIZED);
                         integrate_pair(sc, ins, sm.surv_a[lo], sm.surv_b[lo], cx, acc, flags);
 #pragma unroll
@@ -329,8 +336,9 @@ const int3* large_sorted_ptr(const LargeBuffers* b);
 
 cudaError_t launch_eval_dual6(const SceneDev& sc, long long n_env, const double* X7, const double* twist7, const double* s7, double* wrench7, double* sdot7,
                               const long long* n_pairs, int* flags, const unsigned* small_pairs, int small_cap, const LargeBuffers* lb,
-                              const int32_t* large_index, int n_large, cudaStream_t stream, unsigned* ticket, long long n_real, const DualShared* shared) {
-    DualIO io{n_env, X7, twist7, s7, wrench7, sdot7, n_pairs, flags, n_real > 0 ? n_real : n_env};
+                              const int32_t* large_index, int n_large, const InsParam* params, cudaStream_t stream, unsigned* ticket, long long n_real,
+                              const DualShared* shared) {
+    DualIO io{n_env, X7, twist7, s7, wrench7, sdot7, n_pairs, flags, n_real > 0 ? n_real : n_env, params};
     PairSource ps{small_pairs, small_cap, lb ? large_sorted_ptr(lb) : nullptr, lb ? large_seg_start_ptr(lb) : nullptr, large_index, n_large,
                   shared ? shared->surv_pairs : nullptr, shared ? shared->surv_n : nullptr, shared ? shared->w_f64 : nullptr};
     const long long n_prob = n_env * sc.n_ins;
@@ -357,13 +365,13 @@ cudaError_t launch_eval_dual6(const SceneDev& sc, long long n_env, const double*
 
 
 cudaError_t launch_dual_prefilter(const SceneDev& sc, long long n_env, const double* X, const long long* n_pairs, const unsigned* small_pairs, int small_cap,
-                                  unsigned* surv_pairs, int* surv_n, cudaStream_t stream) {
+                                  unsigned* surv_pairs, int* surv_n, const InsParam* params, cudaStream_t stream) {
     const long long n_prob = n_env * sc.n_ins;
     if (n_prob == 0) return cudaSuccess;
     int n_sm = 148;
     { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev); }
     const unsigned blocks = (unsigned)std::min<long long>((n_prob + 3) / 4, (long long)n_sm * 8);
-    dual_prefilter_kernel<<<blocks, 128, 0, stream>>>(sc, n_env, X, n_pairs, small_pairs, small_cap, surv_pairs, surv_n);
+    dual_prefilter_kernel<<<blocks, 128, 0, stream>>>(sc, n_env, X, n_pairs, small_pairs, small_cap, surv_pairs, surv_n, params);
     return cudaGetLastError();
 }
 

@@ -72,7 +72,10 @@ template <class T> __device__ inline void load_ctx(const SceneDev& sc, const Exa
     for (int j = 0; j < 16; ++j) cx.X21[j] = ldT<T>(io.X, 16 * uw.ei + j);
     for (int j = 0; j < 6; ++j) cx.twist[j] = ldT<T>(io.twist, 6 * uw.ei + j);
     make_x12(cx);
-    cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; cx.n_quad = ins.n_quad;
+    const InsParam* cp = io.params ? io.params + uw.ei : nullptr;
+    if (cp) { cx.chi = cp->chi; cx.Ebar1 = cp->Ebar1; cx.Ebar2 = cp->Ebar2; }
+    else { cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; }
+    cx.n_quad = ins.n_quad;
 }
 
 template <class T>
@@ -183,7 +186,8 @@ __global__ void __launch_bounds__(32 * WPB) exact_bristle_kernel(SceneDev sc, Ex
         long long u0, u1;   // this problem's units
         if (ins.small) { u0 = pb * U_s; u1 = u0 + U_s; }
         else { const long long p = env * ps.n_large + es.large_index[k]; u0 = W_small + ps.unit_start[p]; u1 = W_small + ps.unit_start[p + 1]; }
-        const BristleP bf = {ins.p[0], ins.p[1], ins.p[2], ins.p[3], ins.p[4], ins.p[5], ins.p[6]};
+        const double* fp = io.params ? io.params[ei].p : ins.p;
+        const BristleP bf = {fp[0], fp[1], fp[2], fp[3], fp[4], fp[5], fp[6]};
         const long long sb = 6 * ((long long)sc.n_bristle * env + ins.bristle_id);
         if (lane < 6) { sm.s[lane] = ldT<T>(io.s, sb + lane); sm.twist[lane] = ldT<T>(io.twist, 6 * ei + lane); }
         long long n_points = 0;

@@ -25,6 +25,7 @@ struct ExactIO {
     double* sdot;          // [env][bristle][6]
     const long long* n_pairs;   // [env][ins] (small instructions)
     int* flags;            // [env][ins]
+    const InsParam* params;     // [env][ins] contact parameters, or nullptr for the scene's own
 };
 // candidate-pair lists of the Float64 broad phase
 struct ExactPairs {

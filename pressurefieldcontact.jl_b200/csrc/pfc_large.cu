@@ -674,14 +674,19 @@ __global__ void __launch_bounds__(kChunk, 2) narrow_large_kernel(SceneDev sc, La
             const double* X = io.X + 16 * ei;
             const double* twist = io.twist + 6 * ei;
             PatchCtx<double>& cx = sm.cx;
-            if (lane < 8) sm.fpv[lane] = ins.p[lane];
+            const InsParam* cp = io.params ? io.params + ei : nullptr;   // this environment's contact parameters, if it has its own
+            if (lane < 8) sm.fpv[lane] = cp ? cp->p[lane] : ins.p[lane];
             if (lane < 9) { const int i = lane / 3, j = lane % 3; cx.x21.r[lane] = X[4 * j + i]; }
             else if (lane < 12) cx.x21.t[lane - 9] = X[12 + lane - 9];
             else if (lane < 21) { const int e = lane - 12, i = e / 3, j = e % 3; cx.x12.r[e] = X[4 * i + j]; }
             else if (lane < 24) { const int i = lane - 21; cx.x12.t[i] = -(X[4 * i] * X[12] + X[4 * i + 1] * X[13] + X[4 * i + 2] * X[14]); }
             else if (lane < 27) (&cx.w_ang.x)[lane - 24] = twist[lane - 24];
             else if (lane < 30) (&cx.w_lin.x)[lane - 27] = twist[lane - 24];
-            else if (lane == 30) { cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; cx.n_quad = ins.n_quad; }
+            else if (lane == 30) {
+                if (cp) { cx.chi = cp->chi; cx.Ebar1 = cp->Ebar1; cx.Ebar2 = cp->Ebar2; }
+                else { cx.chi = ins.chi; cx.Ebar1 = ins.Ebar1; cx.Ebar2 = ins.Ebar2; }
+                cx.n_quad = ins.n_quad;
+            }
             if (lane < 8) sm.tot[lane] = 0.0;
         }
         __syncthreads();

@@ -48,11 +48,12 @@ cudaError_t large_get_pairs(LargeBuffers* b, int prob, int* out, long long cap, 
 // What the seed chunks of one Jacobian share (all optional): survivors of the Float64 clip of the small instructions' candidates
 // (launch_dual_prefilter) and the Float64 wrenches of the same evaluation.
 struct DualShared { const unsigned* surv_pairs; const int* surv_n; const double* w_f64; };
+// params: [real env][ins] contact parameters, or nullptr for the scene's own
 cudaError_t launch_dual_prefilter(const SceneDev& sc, long long n_env, const double* X, const long long* n_pairs, const unsigned* small_pairs, int small_cap,
-                                  unsigned* surv_pairs, int* surv_n, cudaStream_t stream);
+                                  unsigned* surv_pairs, int* surv_n, const InsParam* params, cudaStream_t stream);
 cudaError_t launch_eval_dual6(const SceneDev& sc, long long n_env, const double* X7, const double* twist7, const double* s7, double* wrench7, double* sdot7,
                               const long long* n_pairs, int* flags, const unsigned* small_pairs, int small_cap, const LargeBuffers* lb,
-                              const int32_t* large_index, int n_large, cudaStream_t stream, unsigned* ticket, long long n_real = 0,
-                              const DualShared* shared = nullptr);
+                              const int32_t* large_index, int n_large, const InsParam* params, cudaStream_t stream, unsigned* ticket,
+                              long long n_real = 0, const DualShared* shared = nullptr);
 
 }  // namespace pfc

@@ -37,6 +37,7 @@ struct EvalIO {
     int* flags;           // [env][ins]
     int* dbg_pairs;       // optional [env*n_ins][dbg_cap][2] (prim ids, DFS order) or nullptr
     int dbg_cap;
+    const InsParam* params;   // [env][ins] contact parameters, or nullptr for the scene's own
 };
 
 constexpr int kSmallCap = 512;      // frontier / pair capacity of the fused small path
@@ -125,6 +126,8 @@ struct RadauBufs {
     double* X;                  // [env][s_max][nx] stage states
     double* Xp; double* Fp;     // [state][nx] packed stage states / their derivatives
     double* taup;               // [state][nv] (with tau)
+    const InsParam* params;     // [env][n_ins] contact parameters, or nullptr for the scene's own
+    InsParam* paramp;           // [state][n_ins] (with params): the environment's rows, gathered next to taup
     const double* xx0;          // [env][nx] calcXd!(x)
     double* jac;                // [env][nx][nx] d xdot / d x, negated in place into -J
     double* invc;               // [matrix][nx][nx] complex: (h^-1 lambda_i I - J)^-1, matrices in the order of the round's plan
@@ -157,16 +160,19 @@ struct RadauRolloutBufs {
     double* x;                  // [env][nx]
     const double* tau;          // [knot][env][nv] or nullptr
     double* t;                  // [env]
+    const InsParam* params;     // [env][n_ins] contact parameters, or nullptr for the scene's own
     double* x_knot;             // [knot][env][nx] or nullptr
     int* knot;                  // [env] next knot
     int* steps;                 // [env] accepted steps of this roll-out
     int* stats;                 // [env][4] knots reached, accepted steps, rejected attempts, stage evaluations
     int* list;                  // [slot] environment of the compact slot
     RadauEnv* env_c; double* x_c; double* tau_c; double* t_c; double* h_c; double* h_save; int* stats_c;   // [slot] compact step arrays
+    InsParam* params_c;         // [slot][n_ins] (with params)
+    int n_ins;
     int* count;                 // [2]: compact slots of the last selection; 1 if some environment starts within h_min of knot 0
 };
-// One CTA: lists the environments with knot < n_knot and steps < max_steps (environment order), gathers them and prepares the knot step
-// (radau_knot_begin).  check: also test t_knot[0] - t >= h_min for every environment (count[1]; nothing is gathered when it fails).
+// One CTA: lists the environments with knot < n_knot and steps < max_steps (environment order), gathers them (with their parameter rows)
+// and prepares the knot step (radau_knot_begin).  check: also test t_knot[0] - t >= h_min for every environment (count[1]; nothing is gathered when it fails).
 cudaError_t launch_radau_select(const RadauRolloutBufs& b, int check, cudaStream_t stream);
 // After the compact step: radau_knot_end, the x_knot rows, the statistics and the write-back of the n_active slots.
 cudaError_t launch_radau_finish(const RadauRolloutBufs& b, long long n_active, cudaStream_t stream);

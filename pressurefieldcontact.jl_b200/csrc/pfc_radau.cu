@@ -159,7 +159,8 @@ __global__ void radau_prepare_kernel(RadauBufs b, const int* __restrict__ flags,
     if (bad) atomicOr(status, bad);
 }
 
-// one CTA per packed state: its stage vector (x0 at the first iteration of an attempt, which also initialises the stage) and tau_ext
+// one CTA per packed state: its stage vector (x0 at the first iteration of an attempt, which also initialises the stage), tau_ext and the
+// environment's contact parameters
 __global__ void __launch_bounds__(64) radau_gather_kernel(RadauBufs b) {
     const long long p = blockIdx.x;
     const int code = b.state_list[p], e = code >> 3, st = code & 7;
@@ -173,6 +174,11 @@ __global__ void __launch_bounds__(64) radau_gather_kernel(RadauBufs b) {
     }
     if (b.tau)
         for (int n = threadIdx.x; n < b.nv; n += blockDim.x) b.taup[p * b.nv + n] = b.tau[(long long)e * b.nv + n];
+    if (b.params) {
+        const double* src = reinterpret_cast<const double*>(b.params + (long long)e * b.n_ins);
+        double* dst = reinterpret_cast<double*>(b.paramp + p * b.n_ins);
+        for (int n = threadIdx.x; n < b.n_ins * (int)(sizeof(InsParam) / sizeof(double)); n += blockDim.x) dst[n] = src[n];
+    }
 }
 
 // one Newton iteration of one environment (radau.py _simple_newton loop body); every element summed by one thread in a fixed order
@@ -320,6 +326,8 @@ __global__ void __launch_bounds__(kPlanThreads) radau_select_kernel(RadauRollout
                 const double* row = b.tau + ((long long)k * b.n_env + e) * b.nv;
                 for (int n = 0; n < b.nv; ++n) b.tau_c[p * b.nv + n] = row[n];
             }
+            if (b.params)
+                for (int n = 0; n < b.n_ins; ++n) b.params_c[p * b.n_ins + n] = b.params[e * b.n_ins + n];
         }
         base += agg;
     }

@@ -59,6 +59,13 @@ struct InsDev {
     double p[8];
 };
 
+// The contact parameters of one instruction in one environment (pfc_set_contact_params): the fields InsDev ends with, derived by the same
+// host code.  A table of rows [env][ins], passed to the kernels as an optional pointer (nullptr: every environment uses the InsDev values).
+struct InsParam {
+    double chi, Ebar1, Ebar2;
+    double p[8];
+};
+
 // flags written per (env, instruction)
 enum { kFlagContact = 1, kFlagNonFinite = 2, kFlagBadArity = 4, kFlagOverflow = 8 };  // == PFC_FLAG_* of include/pfc.h
 
