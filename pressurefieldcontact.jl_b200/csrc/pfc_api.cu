@@ -742,6 +742,41 @@ static int eval_device_once(pfc_ctx* c, const EvalIO& io_in) {
     return PFC_OK;
 }
 
+// One call through the graph cache g.  When the call (key) has a graph captured since the last reallocation, the graph is launched;
+// when it has run eagerly once since then, it is captured and launched; otherwise enqueue() queues it on c->stream and g remembers it,
+// so that the next identical call is captured.  reuse = false skips the first two.  A graph that cannot be captured or launched
+// disables g: the context stays with plain launches.  Returns enqueue()'s error or PFC_OK; *replayed tells whether a graph ran the call.
+static int run_cached(pfc_ctx* c, pfc_ctx::GraphCache& g, unsigned long long key, bool reuse, const std::function<int()>& enqueue, bool* replayed) {
+    *replayed = false;
+    const unsigned long long gen = alloc_generation().load();
+    if (reuse && g.key == key && g.gen == gen) {
+        if (g.exec) {
+            if (cudaGraphLaunch(g.exec, c->stream) == cudaSuccess) { c->launches += g.launches; *replayed = true; return PFC_OK; }
+            cudaGetLastError(); cudaGraphExecDestroy(g.exec); g.exec = nullptr; g.disabled = true;
+        } else if (g.seen) {   // second identical call: capture it
+            cudaGraph_t graph = nullptr;
+            const long long l0 = c->launches;
+            if (cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
+                const int rc = enqueue();
+                const cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
+                const bool ok = rc == PFC_OK && e == cudaSuccess && graph && alloc_generation().load() == gen &&
+                                cudaGraphInstantiate(&g.exec, graph, 0) == cudaSuccess && cudaGraphLaunch(g.exec, c->stream) == cudaSuccess;
+                if (graph) cudaGraphDestroy(graph);
+                if (ok) { g.launches = int(c->launches - l0); *replayed = true; return PFC_OK; }
+                cudaGetLastError();
+                if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
+                g.disabled = true;
+                c->launches = l0;
+            } else { cudaGetLastError(); g.disabled = true; }
+        }
+    }
+    const int rc = enqueue();
+    if (rc != PFC_OK) return rc;
+    if (g.exec && (g.key != key || g.gen != alloc_generation().load())) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
+    g.key = key; g.gen = alloc_generation().load(); g.seen = true;   // everything this call needs is allocated now
+    return PFC_OK;
+}
+
 // Scenes with large or bristle instructions queue dozens of short kernels per evaluation (breadth-first levels, radix passes, ...): once
 // the same evaluation -- same entry point, batch size and buffers, nothing reallocated since -- has run eagerly, its launch sequence is
 // captured into a CUDA graph and replayed (one launch instead of ~45; the kernels read every data-dependent size from the device).
@@ -750,43 +785,13 @@ static int run_evaluation(pfc_ctx* c, unsigned long long key, const std::functio
     pfc_ctx::GraphCache& g = c->graph;
     const bool want_graph = !g.disabled && !c->timing && !c->keep_pairs && (c->large_buf || c->exact_buf);
     for (int attempt = 0;; ++attempt) {
-        const unsigned long long gen = alloc_generation().load();
         bool replayed = false;
-        if (want_graph && attempt == 0 && g.key == key && g.gen == gen) {
-            if (g.exec) {
-                if (cudaGraphLaunch(g.exec, c->stream) == cudaSuccess) { replayed = true; c->launches += g.launches; }
-                else { cudaGetLastError(); cudaGraphExecDestroy(g.exec); g.exec = nullptr; g.disabled = true; }
-            } else if (g.seen) {   // second identical evaluation: capture it
-                cudaGraph_t graph = nullptr;
-                const long long l0 = c->launches;
-                if (cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-                    const int rc = enqueue();
-                    const cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
-                    if (rc == PFC_OK && e == cudaSuccess && graph && alloc_generation().load() == gen &&
-                        cudaGraphInstantiate(&g.exec, graph, 0) == cudaSuccess && cudaGraphLaunch(g.exec, c->stream) == cudaSuccess) {
-                        g.launches = int(c->launches - l0);
-                        replayed = true;
-                    } else {
-                        cudaGetLastError();
-                        if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
-                        g.disabled = true;   // this context's evaluations do not capture: stay eager
-                        c->launches = l0;
-                    }
-                    if (graph) cudaGraphDestroy(graph);
-                } else { cudaGetLastError(); g.disabled = true; }
-            }
-        }
+        const int rc = want_graph ? run_cached(c, g, key, attempt == 0, enqueue, &replayed) : enqueue();
+        if (rc != PFC_OK) return rc;
         if (replayed) {
             large_mark_pending(c->large_buf);
             exact_mark_pending(c->exact_buf);
             if (c->n_mid > 0) c->mid_check_pending = true;
-        } else {
-            const int rc = enqueue();
-            if (rc != PFC_OK) return rc;
-            if (want_graph) {
-                if (g.key != key || g.gen != alloc_generation().load()) { if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; } g.seen = false; }
-                g.key = key; g.gen = alloc_generation().load(); g.seen = true;
-            }
         }
         const int fit = evaluation_fits(c);
         if (fit < 0) return fit;
@@ -817,36 +822,10 @@ static int eval_device(pfc_ctx* c, const EvalIO& io) {
 // launches.)  Scenes with large / mid-size / bristle instructions are left to run_evaluation: their evaluations synchronise to check
 // buffer sizes.  enqueue() queues the whole call on c->stream (no synchronisation) and returns PFC_OK.
 static int run_host_call(pfc_ctx* c, pfc_ctx::GraphCache& g, unsigned long long key, const std::function<int()>& enqueue) {
-    static const bool host_graph_off = getenv("PFC_NO_HOST_GRAPH") != nullptr;   // (experiment switch)
-    const bool graphable = !host_graph_off && !g.disabled && !c->timing && !c->keep_pairs && !c->large_buf && !c->exact_buf && c->n_mid == 0;
+    const bool graphable = !g.disabled && !c->timing && !c->keep_pairs && !c->large_buf && !c->exact_buf && c->n_mid == 0;
     if (!graphable) return enqueue();
-    const unsigned long long gen = alloc_generation().load();
-    if (g.key == key && g.gen == gen) {
-        if (g.exec) {
-            if (cudaGraphLaunch(g.exec, c->stream) == cudaSuccess) { c->launches += g.launches; return PFC_OK; }
-            cudaGetLastError(); cudaGraphExecDestroy(g.exec); g.exec = nullptr; g.disabled = true;
-        } else if (g.seen) {
-            cudaGraph_t graph = nullptr;
-            const long long l0 = c->launches;
-            if (cudaStreamBeginCapture(c->stream, cudaStreamCaptureModeThreadLocal) == cudaSuccess) {
-                const int rc = enqueue();
-                const cudaError_t e = cudaStreamEndCapture(c->stream, &graph);
-                bool ok = rc == PFC_OK && e == cudaSuccess && graph && alloc_generation().load() == gen && cudaGraphInstantiate(&g.exec, graph, 0) == cudaSuccess &&
-                          cudaGraphLaunch(g.exec, c->stream) == cudaSuccess;
-                if (graph) cudaGraphDestroy(graph);
-                if (ok) { g.launches = int(c->launches - l0); return PFC_OK; }
-                cudaGetLastError();
-                if (g.exec) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
-                g.disabled = true;
-                c->launches = l0;
-            } else { cudaGetLastError(); g.disabled = true; }
-        }
-    }
-    const int rc = enqueue();
-    if (rc != PFC_OK) return rc;
-    if (g.exec && (g.key != key || g.gen != alloc_generation().load())) { cudaGraphExecDestroy(g.exec); g.exec = nullptr; }
-    g.key = key; g.gen = alloc_generation().load(); g.seen = true;   // everything this call needs is allocated now: the next identical one is captured
-    return PFC_OK;
+    bool replayed;
+    return run_cached(c, g, key, true, enqueue, &replayed);
 }
 
 // ---- small host-pointer calls: copies through a pinned arena ----------------------------------------------------------------

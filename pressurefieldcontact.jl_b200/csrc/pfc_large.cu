@@ -190,6 +190,10 @@ PFC_D unsigned item_hash(int prob, int a, int b) {
     return h;
 }
 
+// the level size (node pairs) from which broad_bfs_kernel reserves output space once per warp instead of once per CTA: the
+// measurements are in the kernel
+constexpr unsigned kBfsPerWarpFrom = 1u << 20;
+
 __global__ void __launch_bounds__(256, 2) broad_bfs_kernel(SceneDev sc, const ProbRec* __restrict__ ptab, const Seed* __restrict__ in, Seed* out,
                                                         int level, int split_level, unsigned cap_frontier, int3* pairs, unsigned cap_pairs, Counters* cnt,
                                                         unsigned hrank, unsigned hworld, unsigned per_warp_from) {
@@ -282,10 +286,9 @@ __global__ void dfs_queue_init_kernel(Counters* cnt, int level, unsigned cap_fro
 PFC_D unsigned ld_volatile_u32(const unsigned* p) { return *reinterpret_cast<const volatile unsigned*>(p); }
 
 // K1b: warp-cooperative stack-based traversal of the seeds, with work donation
-template <int MINB>
-__global__ void __launch_bounds__(kDfsWarps * 32, MINB) broad_dfs_kernel(SceneDev sc, const ProbRec* __restrict__ ptab, Seed* seeds, unsigned cap_seeds,
-                                                                   int3* pairs, unsigned cap_pairs, Counters* cnt, unsigned hrank,
-                                                                   unsigned hworld) {
+__global__ void __launch_bounds__(kDfsWarps * 32, 1) broad_dfs_kernel(SceneDev sc, const ProbRec* __restrict__ ptab, Seed* seeds, unsigned cap_seeds,
+                                                                int3* pairs, unsigned cap_pairs, Counters* cnt, unsigned hrank,
+                                                                unsigned hworld) {
     __shared__ int2 stack_mem[kDfsWarps][kStackCap];   // per-warp circular stack: entry i lives at (base + i) & (kStackCap - 1)
     const unsigned epoch = cnt->epoch;
     const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
@@ -961,14 +964,13 @@ cudaError_t large_broad_phase(const SceneDev& sc, const LargeScene& ls, const Ev
     int n_sm = 148;
     { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev); }
     // the traversal kernel is persistent: every block must be resident, because idle warps wait for donated work
-    static const int dfs_minb = getenv("PFC_DFS_MINB") ? atoi(getenv("PFC_DFS_MINB")) : 1;   // (experiment switch)
     int dfs_blocks_per_sm = 0;
     {
         struct Tag {};
         std::lock_guard<std::mutex> g(launch_mutex());
         LaunchSlot& sl = launch_slot<Tag>();
         if (sl.blocks == 0) {
-            LCU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sl.blocks, dfs_minb == 4 ? broad_dfs_kernel<4> : (dfs_minb == 3 ? broad_dfs_kernel<3> : broad_dfs_kernel<1>), kDfsWarps * 32, 0));
+            LCU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&sl.blocks, broad_dfs_kernel, kDfsWarps * 32, 0));
             if (sl.blocks < 1) sl.blocks = 1;
         }
         dfs_blocks_per_sm = sl.blocks;
@@ -993,8 +995,8 @@ cudaError_t large_broad_phase(const SceneDev& sc, const LargeScene& ls, const Ev
     { double f = (double)n_prob; const double target = 1.0 * dfs_blocks * kDfsWarps; while (f < target && levels < 12) { f *= 4.0; ++levels; } }
     // split over several GPUs: a contact patch is small against the meshes, so a few sub-trees carry nearly all of the work; three more
     // breadth-first levels make the hash-partitioned pieces ~64x finer, which is what balances the ranks
-    static const int split_extra = getenv("PFC_SPLIT_EXTRA") ? atoi(getenv("PFC_SPLIT_EXTRA")) : 3;   // (experiment switch)
-    if (hash_world > 1) levels = std::min(levels + split_extra, 16);
+    constexpr int kSplitExtra = 3;
+    if (hash_world > 1) levels = std::min(levels + kSplitExtra, 16);
     const int split_level = levels - 1;             // the level whose children are dealt to the ranks by hash
     // (a level descends both trees until one of them is at a leaf, then the other alone: a leaf pair at depths (d1, d2) is reached at
     // level max(d1, d2), so max_depth + 1 levels test every pair of the recursion)
@@ -1016,23 +1018,15 @@ cudaError_t large_broad_phase(const SceneDev& sc, const LargeScene& ls, const Ev
     // ---- traversal
     init_frontier_kernel<<<std::min<unsigned>((n_prob + 255) / 256, 1024), 256, 0, stream>>>(sc, ls, io.n_env, io.X, b->frontier[0], b->ptab, b->cnt);
     int src = 0;
-    static const unsigned per_warp_from = getenv("PFC_BFS_PER_WARP_FROM") ? (unsigned)atoll(getenv("PFC_BFS_PER_WARP_FROM")) : (1u << 20);   // (experiment switch)
     for (int l = 0; l < levels; ++l) {
         broad_bfs_kernel<<<n_sm * 8, 256, 0, stream>>>(sc, b->ptab, b->frontier[src], b->frontier[src ^ 1], l, split_level, (unsigned)b->cap_frontier, b->pairs,
-                                                     (unsigned)b->cap_pairs, b->cnt, (unsigned)hash_rank, (unsigned)hash_world, per_warp_from);
+                                                     (unsigned)b->cap_pairs, b->cnt, (unsigned)hash_rank, (unsigned)hash_world, kBfsPerWarpFrom);
         src ^= 1;
     }
     // what the levels left (nothing, when they ran to the leaves) is traversed with per-warp stacks; the split has been made by then
     dfs_queue_init_kernel<<<1, 1, 0, stream>>>(b->cnt, levels, (unsigned)b->cap_frontier);
-    if (dfs_minb == 4)
-        broad_dfs_kernel<4><<<dfs_blocks, kDfsWarps * 32, 0, stream>>>(sc, b->ptab, b->frontier[src], (unsigned)b->cap_frontier, b->pairs, (unsigned)b->cap_pairs,
-                                                                     b->cnt, 0u, 1u);
-    else if (dfs_minb == 3)
-        broad_dfs_kernel<3><<<dfs_blocks, kDfsWarps * 32, 0, stream>>>(sc, b->ptab, b->frontier[src], (unsigned)b->cap_frontier, b->pairs, (unsigned)b->cap_pairs,
-                                                                     b->cnt, 0u, 1u);
-    else
-        broad_dfs_kernel<1><<<dfs_blocks, kDfsWarps * 32, 0, stream>>>(sc, b->ptab, b->frontier[src], (unsigned)b->cap_frontier, b->pairs, (unsigned)b->cap_pairs,
-                                                                     b->cnt, 0u, 1u);
+    broad_dfs_kernel<<<dfs_blocks, kDfsWarps * 32, 0, stream>>>(sc, b->ptab, b->frontier[src], (unsigned)b->cap_frontier, b->pairs, (unsigned)b->cap_pairs,
+                                                              b->cnt, 0u, 1u);
     LCU(cudaMemcpyAsync(b->h_cnt, b->cnt, sizeof(Counters), cudaMemcpyDeviceToHost, stream));   // read by large_check() after the caller's synchronisation
     b->check_pending = true;
     if (n_launches) *n_launches += 3 + levels;

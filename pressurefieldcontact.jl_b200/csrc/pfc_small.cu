@@ -430,11 +430,14 @@ cudaError_t launch_broad_tile(const SceneDev& sc, const EvalIO& io, int cap, uns
     return cudaGetLastError();
 }
 
-template <int P, int MINB>
+// 4 problems per tile whatever the batch size: a tile of 4 is one environment's instructions, whose light (box on plane) and heavy
+// (box on box) pair lists balance each other over the CTA's 128 threads.  Measured: 4096 environments 137 / 170 / 200 us for
+// 4 / 2 / 1 problems per tile; 512 environments 30 / 48 / 52 us.
 cudaError_t launch_narrow_tile(const SceneDev& sc, const EvalIO& io, int cap, const unsigned* pairs, cudaStream_t stream) {
+    constexpr int P = 4;
     struct Tag {};
     const bool per_env = io.params != nullptr;
-    auto kern = per_env ? narrow_tile_params_kernel<P, MINB> : narrow_tile_kernel<P, MINB>;
+    auto kern = per_env ? narrow_tile_params_kernel<P, 4> : narrow_tile_kernel<P, 4>;   // 4 CTAs per SM
     const size_t smem = sizeof(TileSmem<P>);
     int cached_blocks;
     {
@@ -460,11 +463,10 @@ cudaError_t launch_broad(const SceneDev& sc, const EvalIO& io, int cap, unsigned
     // 2 problems 102 us, 4 problems 85 us.)  Small batches: a warp's tile of 4 problems takes ~42 us whatever the load (level after level of
     // dependent phases), so when the problems do not fill the resident warps 4 at a time, smaller tiles shorten the critical path:
     // 512 environments 27.6 / 29.7 / 42.0 us for 1 / 2 / 4 problems per warp, 1024 environments 46.0 / 37.9 / 42.1 us.
-    static const int broad_p_env = getenv("PFC_BROAD_P") ? atoi(getenv("PFC_BROAD_P")) : 0;   // (experiment switch)
     const long long n_prob = io.n_env * sc.n_small;
     int n_sm = 148;
     { int dev = 0; cudaGetDevice(&dev); cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev); }
-    int p = broad_p_env ? broad_p_env : (n_prob <= 16LL * n_sm ? 1 : (n_prob <= 32LL * n_sm ? 2 : 4));
+    int p = n_prob <= 16LL * n_sm ? 1 : (n_prob <= 32LL * n_sm ? 2 : 4);
     if (cap > 256) p = 1;   // slots of kMidCap entries (mid-size trees): the frontiers of one problem per warp are what fits in shared memory
     if (p == 1) return launch_broad_tile<1, 8, 2>(sc, io, cap, pairs, stream);
     if (p == 2) return launch_broad_tile<2, 8, 2>(sc, io, cap, pairs, stream);
@@ -488,18 +490,7 @@ cudaError_t launch_eval_small_f64(const SceneDev& sc, const EvalIO& io, int max_
     if (after_broad) cudaEventRecord(after_broad, stream);   // the pair lists exist: what only needs them may start on another stream
     // regularized instructions: the tile kernel (4 problems per CTA, 4 CTAs per SM).  Bristle instructions are skipped here: they are
     // evaluated in the reference's operation order by pfc_exact.cu from the pair lists the broad kernel left
-    {
-        // 4 problems per tile whatever the batch size: a tile of 4 is one environment's instructions, whose light (box on plane) and heavy
-        // (box on box) pair lists balance each other over the CTA's 128 threads.  Measured: 4096 environments 137 / 170 / 200 us for
-        // 4 / 2 / 1 problems per tile; 512 environments 30 / 48 / 52 us.
-        static const int tile_p = getenv("PFC_TILE_P") ? atoi(getenv("PFC_TILE_P")) : 4;   // (experiment switch)
-        if (tile_p == 1) e = launch_narrow_tile<1, 16>(sc, io, cap, pairs, stream);
-        else if (tile_p == 2) e = launch_narrow_tile<2, 8>(sc, io, cap, pairs, stream);
-        else {
-            static const int minb = getenv("PFC_TILE_MINB") ? atoi(getenv("PFC_TILE_MINB")) : 4;   // (experiment switch)
-            e = minb == 5 ? launch_narrow_tile<4, 5>(sc, io, cap, pairs, stream) : launch_narrow_tile<4, 4>(sc, io, cap, pairs, stream);
-        }
-    }
+    e = launch_narrow_tile(sc, io, cap, pairs, stream);
     if (ev) cudaEventRecord(ev[2], stream);
     if (n_launches) *n_launches += 2;
     return e;

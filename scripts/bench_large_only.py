@@ -22,8 +22,7 @@ def main():
         dist.init_process_group("nccl", device_id=torch.device("cuda", local_rank))
     out = bench.measure_large_scenes(local_rank, rank, world)
     if rank == 0:
-        print(json.dumps({"n_gpus": world, "split_extra": os.environ.get("PFC_SPLIT_EXTRA", "default"),
-                          "ms_per_eval": {k: v.get("ms_per_eval", v.get("error")) for k, v in out.items()}}))
+        print(json.dumps({"n_gpus": world, "ms_per_eval": {k: v.get("ms_per_eval", v.get("error")) for k, v in out.items()}}))
     if world > 1:
         dist.destroy_process_group()
 

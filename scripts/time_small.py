@@ -55,8 +55,7 @@ def main():
     ctx.sync()
     tot = float(np.median([a.elapsed_time(b) for a, b in zip(e0, e1)]))
     wh = w.cpu().numpy()
-    print(json.dumps({"n_env": n_env, "tile_p": os.environ.get("PFC_TILE_P", "default"), "variant": os.environ.get("PFC_VARIANT", ""),
-                      "broad_us": 1e3 * float(np.median([a for a, _ in split])), "narrow_us": 1e3 * float(np.median([b for _, b in split])), "step_us": 1e3 * tot,
+    print(json.dumps({"n_env": n_env, "broad_us": 1e3 * float(np.median([a for a, _ in split])), "narrow_us": 1e3 * float(np.median([b for _, b in split])), "step_us": 1e3 * tot,
                       "wrench_sha": hashlib.sha256(wh.tobytes()).hexdigest()[:16], "contacts": int((fl.cpu().numpy() & 1).sum())}))
 
 

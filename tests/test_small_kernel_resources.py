@@ -1,8 +1,9 @@
 """CPU-only: the small path's kernels keep what they need in registers and shared memory.
 
 pfc_small.cu is compiled for sm_100a with -Xptxas -v and the report is read back:
-  * narrow_tile_kernel<4, 4> (the tile kernel every batch runs) fits 128 registers with no stack frame and no spill traffic.  It runs
-    at 4 CTAs x 128 threads per SM, so 128 registers is the whole register file, and a spill or a local-memory array silently puts
+  * narrow_tile_kernel<4, 4> (the tile kernel every batch runs) and narrow_tile_params_kernel<4, 4> (its twin from the same source,
+    run by every batch with a contact-parameter table) fit 128 registers with no stack frame and no spill traffic.  They run at
+    4 CTAs x 128 threads per SM, so 128 registers is the whole register file, and a spill or a local-memory array silently puts
     L1 / L2 round trips on the critical path of every tile;
   * every broad_tile_kernel variant stays free of spills.
 Skipped when nvcc is not installed."""
@@ -54,9 +55,10 @@ def _kernels(res, pattern):
 
 
 def test_narrow_tile_kernel_has_no_local_memory(resources):
-    (name, r), = _kernels(resources, r"narrow_tile_kernelILi4ELi4E").items()
-    assert r["regs"] <= 128, r
-    assert r["stack"] == 0 and r["spill_st"] == 0 and r["spill_ld"] == 0, r
+    for kernel in ("narrow_tile_kernel", "narrow_tile_params_kernel"):
+        (name, r), = _kernels(resources, kernel + r"ILi4ELi4E").items()
+        assert r["regs"] <= 128, (name, r)
+        assert r["stack"] == 0 and r["spill_st"] == 0 and r["spill_ld"] == 0, (name, r)
 
 
 def test_broad_tile_kernels_do_not_spill(resources):
