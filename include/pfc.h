@@ -127,6 +127,22 @@ int pfc_eval_state_f64_device(pfc_ctx* ctx, int64_t n_env, const double* x, doub
  * [angular; linear] ordering (newBodyFromInertia, src/body_inertia.jl:2-9; ignored for world-attached bodies); gravity[3] in the world frame
  * (src/mechanism_scenario.jl:184).  The mass matrix of such a scene is block diagonal and constant, so it is factored once, here. */
 int pfc_set_dynamics(pfc_ctx* ctx, int n_body, const double* spatial_inertia, const double* gravity);
+/* Per-environment body parameters, after pfc_set_dynamics (domain randomization and system identification of mass, centre of mass,
+ * rotational inertia and gravity as one batch).  spatial_inertia[env][body][36] in pfc_set_dynamics' layout (rows of world-attached
+ * bodies are ignored and not validated), gravity[env][3] in the world frame.  Host pointers, copied; each row is checked and factored
+ * as pfc_set_dynamics does it.  While a table is set, environment e of pfc_calcxd_f64[_device], pfc_calcxd_dual6[_device],
+ * pfc_calcxd_jacobian[_device], pfc_radau_step[_device] and pfc_radau_rollout[_device] gives the bits of a context whose
+ * pfc_set_dynamics got row e, evaluated on the same batch.  For calcXd! and its Jacobian this holds in every scene (the contact wrenches do
+ * not read inertia).  For Radau steps and roll-outs the environments follow different trajectories, so the caveat of
+ * pfc_set_contact_params applies: in a scene whose number of small instructions is not a multiple of 4, bit-for-bit equality needs the
+ * environments that share e's narrow tiles to follow e's trajectory; otherwise e agrees to rounding.  Those entry points (and
+ * pfc_radau_init) require n_env to equal the table's; the evaluations that do not read inertia or gravity (pfc_eval_*,
+ * pfc_eval_state_f64[_device], sharded and group calls, pfc_get_*) ignore the table.  With a contact-parameter table set as well, row e of
+ * each applies.  n_env = 0 clears the table, and so does a later pfc_set_bodies or pfc_set_dynamics (its rows were checked against the
+ * previous mechanism).  PFC_E_ARG, with the table in force unchanged, before pfc_set_dynamics, for n_env outside 0..max_env, a NULL
+ * pointer with n_env > 0, a non-finite entry, or a non-symmetric or non-positive-definite inertia (the message names the environment
+ * and the body). */
+int pfc_set_body_params(pfc_ctx* ctx, int64_t n_env, const double* spatial_inertia, const double* gravity);
 /* x[env][n_x] -> xdot[env][n_x] = [q_dot; v_dot; s_dot] (copyto!, src/extensions.jl:40-50).  tau_ext[env][nv] = external generalized
  * forces (the controller's tau_ext, :46-47) or NULL.  Host pointers; n_pairs / flags [env][ins] may be NULL. */
 int pfc_calcxd_f64(pfc_ctx* ctx, int64_t n_env, const double* x, const double* tau_ext, double* xdot, int64_t* n_pairs, int32_t* flags);

@@ -200,6 +200,22 @@ function set_contact_params!(m::MechanismScenario, params::Union{Array{Float64,3
     return nothing
 end
 
+"Per-environment body parameters (pfc_set_body_params), after `finalize_floating_gpu!`: `H[:, body, env]` = the body's 6x6 spatial inertia
+as `finalize_floating_gpu!` lays it out (`vec(transpose(M))`, M = [moment cx; cx' mass I] about the body origin in the body frame; columns of
+the root are ignored), `g[:, env]` = gravity in the world frame; the calcXd!, Jacobian and Radau calls then take n_env = size(H, 3).
+`nothing` clears the table."
+function set_body_params!(m::MechanismScenario, H::Union{Array{Float64,3},Nothing}, g::Union{Matrix{Float64},Nothing}=nothing)
+    if H === nothing
+        check(ccall((:pfc_set_body_params, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}), CTX[m], 0, C_NULL, C_NULL))
+    else
+        nb = length(collect(bodies(m.float.state.mechanism)))
+        (size(H, 1) == 36 && size(H, 2) == nb) || error("H must be 36 x n_body x n_env")
+        (g !== nothing && size(g) == (3, size(H, 3))) || error("g must be 3 x n_env")
+        GC.@preserve H g check(ccall((:pfc_set_body_params, LIB), Cint, (Ptr{Cvoid}, Int64, Ptr{Float64}, Ptr{Float64}), CTX[m], size(H, 3), H, g))
+    end
+    return nothing
+end
+
 "forceAllElasticIntersections! for a batch of states `x[:, env]`: generalized forces `f[:, env]` and `sdot` (pfc_eval_state_f64)."
 function force_all_batch_gpu!(f::Matrix{Float64}, sdot::Matrix{Float64}, m::MechanismScenario, x::Matrix{Float64})
     GC.@preserve x f sdot check(ccall((:pfc_eval_state_f64, LIB), Cint,

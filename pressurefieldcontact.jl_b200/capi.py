@@ -22,7 +22,7 @@ _vp = C.c_void_p
 SYMBOLS = [
     "pfc_create", "pfc_destroy", "pfc_add_mesh", "pfc_add_instruction", "pfc_finalize", "pfc_set_contact_params", "pfc_eval_f64", "pfc_eval_f64_device",
     "pfc_eval_dual6", "pfc_set_debug", "pfc_get_pairs", "pfc_get_traction", "pfc_set_shard", "pfc_eval_sharded_begin", "pfc_eval_sharded_partials", "pfc_eval_sharded_step", "pfc_sync", "pfc_stream",
-    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_rollout", "pfc_radau_rollout_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
+    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_set_body_params", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_rollout", "pfc_radau_rollout_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
     "pfc_comm_unique_id", "pfc_comm_init_rank", "pfc_eval_sharded_f64_device", "pfc_group_create", "pfc_group_destroy", "pfc_group_size", "pfc_group_ctx",
     "pfc_group_add_mesh", "pfc_group_add_instruction", "pfc_group_finalize", "pfc_group_eval_f64",
 ]
@@ -63,6 +63,7 @@ def lib():
         L.pfc_eval_state_f64_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
         L.pfc_get_boundary.argtypes = [_vp, C.c_int64, _vp, _vp, _vp]
         L.pfc_set_dynamics.argtypes = [_vp, C.c_int, _d, _d]
+        L.pfc_set_body_params.argtypes = [_vp, C.c_int64, _vp, _vp]
         L.pfc_calcxd_f64.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
         L.pfc_calcxd_f64_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
         L.pfc_calcxd_dual6.argtypes = [_vp, C.c_int64, _vp, _vp, C.c_int, _vp, _vp, _vp]
@@ -211,7 +212,7 @@ class Context:
         jt, q0a, v0a, mb = _a(joint_type, np.int32), _a(q0, np.int32), _a(v0, np.int32), _a(mesh_body, np.int32)
         pose_a = None if pose is None else _a(pose).reshape(len(jt), 12)
         _check(lib().pfc_set_bodies(self._h, len(jt), jt, q0a, v0a, _p(pose_a), mb, int(nq), int(nv)))
-        self.nq, self.nv = int(nq), int(nv)
+        self.nq, self.nv, self.n_body = int(nq), int(nv), len(jt)
 
     def eval_state_f64(self, x):
         """x[env][nq + nv + 6 n_bristle] (host) -> dict(f_generalized[env][nv], sdot, n_pairs, flags)."""
@@ -236,6 +237,20 @@ class Context:
         """spatial_inertia[n_body][6][6] about the body origins in the body frames ([angular; linear]); gravity[3] in the world."""
         H = _a(spatial_inertia).reshape(-1, 36)
         _check(lib().pfc_set_dynamics(self._h, H.shape[0], H, _a(gravity).reshape(3)))
+
+    def set_body_params(self, spatial_inertia, gravity=None):
+        """Per-environment body parameters: spatial_inertia[env][body][6][6] in set_dynamics' layout (rows of world-attached bodies are
+        ignored), gravity[env][3] in the world frame; None clears the table (pfc_set_body_params)."""
+        if spatial_inertia is None:
+            _check(lib().pfc_set_body_params(self._h, 0, None, None))
+            return
+        H = _a(spatial_inertia)
+        if H.ndim != 4 or H.shape[1:] != (self.n_body, 6, 6):
+            raise ValueError(f"spatial_inertia must have shape [n_env, {self.n_body}, 6, 6], got {H.shape}")
+        g = _a(gravity)
+        if g.shape != (H.shape[0], 3):
+            raise ValueError(f"gravity must have shape [{H.shape[0]}, 3], got {g.shape}")
+        _check(lib().pfc_set_body_params(self._h, H.shape[0], _p(H), _p(g)))
 
     def calcxd_f64(self, x, tau_ext=None):
         """x[env][n_x] (host) -> dict(xdot[env][n_x], n_pairs, flags)."""

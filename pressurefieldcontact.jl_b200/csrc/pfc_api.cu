@@ -231,6 +231,7 @@ struct pfc_ctx {
         DevBuf<RadauEnv> env;
         DevBuf<double> X, Xp, Fp, taup, xx0, jac, invc, shift, x, tau, t, h;
         DevBuf<InsParam> paramp, params_c;   // contact-parameter rows gathered per stage state / per compact roll-out slot: grown on first use
+        DevBuf<int> rowp;                    // body table: row of each stage state (DynDev::row of the stage evaluations), grown on first use
         DevBuf<int> index, state_list, env_list, state_pos, inv_base, counts, stats, flags, flags_stage, info;
         DevBuf<long long> np, np_stage;
         // roll-outs (pfc_radau_rollout): grown on first use
@@ -249,6 +250,9 @@ struct pfc_ctx {
     DevBuf<InsParam> d_params;
     int64_t params_n_env = 0;
     const InsParam* last_params = nullptr;   // the table the last evaluation read (pfc_get_traction re-runs its narrow phase)
+    // per-environment body parameters (pfc_set_body_params): H, H^-1 [env][body][36] and gravity [env][3]; body_n_env = 0 while no table is set
+    DevBuf<double> d_body_H, d_body_Hinv, d_body_g;
+    int64_t body_n_env = 0;
 };
 
 namespace {
@@ -1384,6 +1388,7 @@ int pfc_set_bodies(pfc_ctx* c, int n_body, const int32_t* joint_type, const int3
                    const int32_t* mesh_body, int nq, int nv) {
     if (!c || !c->finalized) return fail(PFC_E_ARG, "pfc_set_bodies: call after pfc_finalize");
     if (n_body < 1 || !joint_type || !q0 || !v0 || !mesh_body || nq < 0 || nv < 0) return fail(PFC_E_ARG, "pfc_set_bodies: bad argument");
+    c->body_n_env = 0;   // a body table's rows were checked against the previous mechanism
     c->h_bodies.assign(n_body, BodyDev{});
     for (int b = 0; b < n_body; ++b) {
         BodyDev& d = c->h_bodies[b];
@@ -1523,20 +1528,26 @@ static bool spd6_inverse(const double* H, double* inv) {
     return true;
 }
 
+// one floating body's spatial inertia: copied to H and factored into Hi; nullptr, or why it is rejected
+static const char* factor_inertia(const double* src, double* H, double* Hi) {
+    for (int i = 0; i < 36; ++i) H[i] = src[i];
+    for (int i = 0; i < 6; ++i)
+        for (int j = 0; j < i; ++j)
+            if (std::fabs(H[6 * i + j] - H[6 * j + i]) > 1e-12 * (std::fabs(H[6 * i + i]) + std::fabs(H[6 * j + j]))) return "spatial inertia is not symmetric";
+    if (!spd6_inverse(H, Hi)) return "spatial inertia is not positive definite";
+    return nullptr;
+}
+
 int pfc_set_dynamics(pfc_ctx* c, int n_body, const double* spatial_inertia, const double* gravity) {
     if (!c || !c->has_bodies) return fail(PFC_E_ARG, "pfc_set_dynamics: call after pfc_set_bodies");
     if (n_body != c->state.n_body || !spatial_inertia || !gravity) return fail(PFC_E_ARG, "pfc_set_dynamics: bad argument");
     std::vector<double> H(36 * size_t(n_body), 0.0), Hi(36 * size_t(n_body), 0.0);
     for (int b = 0; b < n_body; ++b) {
         if (c->h_bodies[b].joint == 0) continue;
-        for (int i = 0; i < 36; ++i) H[36 * b + i] = spatial_inertia[36 * b + i];
-        for (int i = 0; i < 6; ++i)
-            for (int j = 0; j < i; ++j)
-                if (std::fabs(H[36 * b + 6 * i + j] - H[36 * b + 6 * j + i]) > 1e-12 * (std::fabs(H[36 * b + 6 * i + i]) + std::fabs(H[36 * b + 6 * j + j])))
-                    return fail(PFC_E_ARG, "pfc_set_dynamics: spatial inertia is not symmetric");
-        if (!spd6_inverse(&H[36 * b], &Hi[36 * b])) return fail(PFC_E_ARG, "pfc_set_dynamics: spatial inertia is not positive definite");
+        if (const char* why = factor_inertia(&spatial_inertia[36 * b], &H[36 * b], &Hi[36 * b])) return fail(PFC_E_ARG, std::string("pfc_set_dynamics: ") + why);
     }
     CU(cudaSetDevice(c->device));
+    c->body_n_env = 0;   // a body table's rows were checked against the previous mechanism
     CU(c->d_H.ensure(H.size())); CU(c->d_Hinv.ensure(Hi.size()));
     CU(cudaMemcpy(c->d_H.p, H.data(), sizeof(double) * H.size(), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(c->d_Hinv.p, Hi.data(), sizeof(double) * Hi.size(), cudaMemcpyHostToDevice));
@@ -1546,8 +1557,61 @@ int pfc_set_dynamics(pfc_ctx* c, int n_body, const double* spatial_inertia, cons
     return PFC_OK;
 }
 
-static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, double* xdot, long long* n_pairs, int* flags,
-                         int* status = nullptr) {
+// ---- per-environment body parameters ---------------------------------------------------------------------------------------
+// the rigid-body data of an entry point: the scene's own, with the context's per-environment table while one is set
+static DynDev ctx_dyn(const pfc_ctx* c) {
+    DynDev d = c->dyn;
+    if (c->body_n_env > 0) { d.H_env = c->d_body_H.p; d.Hinv_env = c->d_body_Hinv.p; d.g_env = c->d_body_g.p; }
+    return d;
+}
+static int body_params_check(const pfc_ctx* c, const char* who, int64_t n_env) {
+    if (c->body_n_env > 0 && n_env != c->body_n_env)
+        return fail(PFC_E_ARG, std::string(who) + ": n_env differs from the batch of the body-parameter table (pfc_set_body_params)");
+    return PFC_OK;
+}
+
+int pfc_set_body_params(pfc_ctx* c, int64_t n_env, const double* spatial_inertia, const double* gravity) {
+    if (!c || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_set_body_params: call after pfc_set_dynamics");
+    if (n_env < 0 || n_env > c->max_env) return fail(PFC_E_ARG, "pfc_set_body_params: n_env must be in 0..max_env");
+    if (n_env > 0 && (!spatial_inertia || !gravity)) return fail(PFC_E_ARG, "pfc_set_body_params: spatial_inertia or gravity is NULL");
+    CU(cudaSetDevice(c->device));
+    if (n_env == 0) {   // back to pfc_set_dynamics' values (the buffers are kept for the next table)
+        c->body_n_env = 0;
+        return PFC_OK;
+    }
+    // each row factored as pfc_set_dynamics factors it, so a row of the scene's own values holds the same H and H^-1 bits
+    const size_t nb = size_t(c->state.n_body), ne = size_t(n_env);
+    std::vector<double> H(36 * nb * ne, 0.0), Hi(36 * nb * ne, 0.0), g(3 * ne);
+    for (size_t e = 0; e < ne; ++e) {
+        const std::string where = " (environment " + std::to_string(e);
+        for (int i = 0; i < 3; ++i) {
+            g[3 * e + i] = gravity[3 * e + i];
+            if (!std::isfinite(g[3 * e + i])) return fail(PFC_E_ARG, "pfc_set_body_params: non-finite gravity" + where + ")");
+        }
+        for (size_t b = 0; b < nb; ++b) {
+            if (c->h_bodies[b].joint == 0) continue;
+            const size_t o = 36 * (e * nb + b);
+            const std::string at = where + ", body " + std::to_string(b) + ")";
+            for (int i = 0; i < 36; ++i)
+                if (!std::isfinite(spatial_inertia[o + i])) return fail(PFC_E_ARG, "pfc_set_body_params: non-finite spatial inertia" + at);
+            if (const char* why = factor_inertia(&spatial_inertia[o], &H[o], &Hi[o])) return fail(PFC_E_ARG, std::string("pfc_set_body_params: ") + why + at);
+        }
+    }
+    // in stream order behind the calls already queued (they read the previous table), and complete before the host rows go
+    if (H.size() > c->d_body_H.n || g.size() > c->d_body_g.n) {
+        c->body_n_env = 0;   // (growing frees the previous table: should the allocation fail, no table is left in force)
+        CU(c->d_body_H.ensure(H.size())); CU(c->d_body_Hinv.ensure(Hi.size())); CU(c->d_body_g.ensure(g.size()));
+    }
+    CU(cudaMemcpyAsync(c->d_body_H.p, H.data(), sizeof(double) * H.size(), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->d_body_Hinv.p, Hi.data(), sizeof(double) * Hi.size(), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->d_body_g.p, g.data(), sizeof(double) * g.size(), cudaMemcpyHostToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    c->body_n_env = n_env;
+    return PFC_OK;
+}
+
+static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* xdot,
+                         long long* n_pairs, int* flags, int* status = nullptr) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle);
     CU(c->d_X.ensure(16 * ne * ni)); CU(c->d_tw.ensure(6 * ne * ni)); CU(c->d_w.ensure(6 * ne * ni));
     if (nb) { CU(c->d_s.ensure(6 * ne * nb)); CU(c->d_sd.ensure(6 * ne * nb)); }
@@ -1558,7 +1622,7 @@ static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const doubl
     io.sdot = nb ? c->d_sd.p : nullptr; io.n_pairs = n_pairs; io.flags = flags; io.params = params;
     int rc = eval_device(c, io);
     if (rc != PFC_OK) return rc;
-    CU(launch_state_dynamics(c->state, c->dyn, n_env, int(ni), int(nb), x, c->d_w.p, tau_ext, nb ? c->d_sd.p : nullptr, xdot, c->stream, &nl, flags, status));
+    CU(launch_state_dynamics(c->state, dyn, n_env, int(ni), int(nb), x, c->d_w.p, tau_ext, nb ? c->d_sd.p : nullptr, xdot, c->stream, &nl, flags, status));
     c->launches += nl;
     return PFC_OK;
 }
@@ -1567,16 +1631,18 @@ int pfc_calcxd_f64_device(pfc_ctx* c, int64_t n_env, const double* x, const doub
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_f64_device", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = body_params_check(c, "pfc_calcxd_f64_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: NULL buffer");
     CU(cudaSetDevice(c->device));
-    return calcxd_device(c, n_env, x, tau_ext, ctx_params(c), xdot, reinterpret_cast<long long*>(n_pairs), flags);
+    return calcxd_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), xdot, reinterpret_cast<long long*>(n_pairs), flags);
 }
 
 int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* xdot, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_f64: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_f64: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_f64", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = body_params_check(c, "pfc_calcxd_f64", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot) return fail(PFC_E_ARG, "pfc_calcxd_f64: NULL buffer");
     CU(cudaSetDevice(c->device));
@@ -1589,7 +1655,7 @@ int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau
     }
     CU(cudaMemsetAsync(c->d_xdot.p, 0, sizeof(double) * ne * nx, c->stream));
     CU(status_begin(c));
-    int rc = calcxd_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = calcxd_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(xdot, c->d_xdot.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     if (n_pairs) CU(cudaMemcpyAsync(n_pairs, c->d_np.p, sizeof(long long) * ne * ni, cudaMemcpyDeviceToHost, c->stream));
@@ -1631,7 +1697,8 @@ static int dual_shared_f64(pfc_ctx* c, int64_t n_env, long long* n_pairs, int* f
 // calcXd! in Jacobian mode for the same scenes: x (Float64) with Dual seeds on x[seed_start .. seed_start + 6) -> x_dot as 7 doubles per
 // entry (value, then d x_dot / d x[seed_start + k]).  Device pipeline: Float64 prologue + broad phase (the reference always traverses
 // with m.float), Dual prologue, Dual narrow phase / friction (pfc_dual.cu), Dual J' w and rigid-body terms.
-static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, int seed_start, double* xdot7,
+static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, int seed_start,
+                                    double* xdot7,
                                     long long* n_pairs, int* flags, int* status) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle);
     CU(c->d_X.ensure(16 * ne * ni)); CU(c->d_tw.ensure(6 * ne * ni));
@@ -1652,14 +1719,14 @@ static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, 
                                     &nl);
         if (rc != PFC_OK) return rc;
     }
-    CU(launch_state_dynamics_dual6(c->state, c->dyn, n_env, int(ni), int(nb), x, seed_start, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr, xdot7,
+    CU(launch_state_dynamics_dual6(c->state, dyn, n_env, int(ni), int(nb), x, seed_start, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr, xdot7,
                                    c->stream, &nl, flags, status));
     c->launches += nl + 1;
     return PFC_OK;
 }
-static int calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, int seed_start, double* xdot7,
-                               long long* n_pairs, int* flags, int* status) {
-    PFC_REQUEUE_LOOP({ const int rc_ = calcxd_dual6_device_once(c, n_env, x, tau_ext, params, seed_start, xdot7, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
+static int calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, int seed_start,
+                               double* xdot7, long long* n_pairs, int* flags, int* status) {
+    PFC_REQUEUE_LOOP({ const int rc_ = calcxd_dual6_device_once(c, n_env, x, tau_ext, params, dyn, seed_start, xdot7, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
     return PFC_OK;
 }
 
@@ -1668,17 +1735,19 @@ int pfc_calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const do
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_dual6_device", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = body_params_check(c, "pfc_calcxd_dual6_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot7 || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: NULL buffer");
     if (seed_start < 0 || seed_start >= c->state.n_x) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: seed_start out of range");
     CU(cudaSetDevice(c->device));
-    return calcxd_dual6_device(c, n_env, x, tau_ext, ctx_params(c), seed_start, xdot7, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
+    return calcxd_dual6_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), seed_start, xdot7, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
 }
 
 int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, int seed_start, double* xdot7, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_dual6: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_dual6: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_dual6", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = body_params_check(c, "pfc_calcxd_dual6", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot7) return fail(PFC_E_ARG, "pfc_calcxd_dual6: NULL buffer");
     if (seed_start < 0 || seed_start >= c->state.n_x) return fail(PFC_E_ARG, "pfc_calcxd_dual6: seed_start out of range");
@@ -1692,7 +1761,7 @@ int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* t
     }
     CU(cudaMemsetAsync(c->d_xdot.p, 0, sizeof(double) * 7 * ne * nx, c->stream));
     CU(status_begin(c));
-    int rc = calcxd_dual6_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), seed_start, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = calcxd_dual6_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), seed_start, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(xdot7, c->d_xdot.p, sizeof(double) * 7 * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     if (n_pairs) CU(cudaMemcpyAsync(n_pairs, c->d_np.p, sizeof(long long) * ne * ni, cudaMemcpyDeviceToHost, c->stream));
@@ -1707,7 +1776,7 @@ int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* t
 // seed chunks are a grid axis of the Dual kernels ("environment" (g, env) = chunk g of real environment env) as far as the work space
 // allows, and the rigid-body kernel writes the partials straight into jac[env][row][col].  Scenes with bristle instructions go chunk by
 // chunk (their reference-order pipeline is sized per real environment) but still share the broad phase.
-static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, double* jac, double* xdot,
+static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* jac, double* xdot,
                                 long long* n_pairs, int* flags, int* status) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle), nx = size_t(c->state.n_x);
     const int n_chunk = int((nx + 5) / 6);
@@ -1734,15 +1803,15 @@ static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, cons
             int rc = eval_bristle_exact(c, n_env, c->d_X7.p, c->d_tw7.p, c->d_s7.p, c->d_w7.p, c->d_sd7.p, n_pairs, flags, params, 1, false, &nl);
             if (rc != PFC_OK) return rc;
         }
-        CU(launch_state_dynamics_dual6(c->state, c->dyn, n_virtual, int(ni), int(nb), x, 6 * g0, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr,
+        CU(launch_state_dynamics_dual6(c->state, dyn, n_virtual, int(ni), int(nb), x, 6 * g0, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr,
                                        g0 == 0 ? xdot : nullptr, c->stream, &nl, flags, status, n_env, jac));
     }
     c->launches += nl;
     return PFC_OK;
 }
-static int jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, double* jac, double* xdot,
+static int jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* jac, double* xdot,
                            long long* n_pairs, int* flags, int* status) {
-    PFC_REQUEUE_LOOP({ const int rc_ = jacobian_device_once(c, n_env, x, tau_ext, params, jac, xdot, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
+    PFC_REQUEUE_LOOP({ const int rc_ = jacobian_device_once(c, n_env, x, tau_ext, params, dyn, jac, xdot, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
     return PFC_OK;
 }
 
@@ -1751,16 +1820,18 @@ int pfc_calcxd_jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_jacobian_device", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = body_params_check(c, "pfc_calcxd_jacobian_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !jac || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: NULL buffer");
     CU(cudaSetDevice(c->device));
-    return jacobian_device(c, n_env, x, tau_ext, ctx_params(c), jac, xdot, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
+    return jacobian_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), jac, xdot, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
 }
 
 int pfc_calcxd_jacobian(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* jac, double* xdot, int64_t* n_pairs, int32_t* flags) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_jacobian", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = body_params_check(c, "pfc_calcxd_jacobian", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !jac) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: NULL buffer");
     CU(cudaSetDevice(c->device));
@@ -1772,7 +1843,7 @@ int pfc_calcxd_jacobian(pfc_ctx* c, int64_t n_env, const double* x, const double
         CU(cudaMemcpyAsync(c->d_tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
     }
     CU(status_begin(c));
-    int rc = jacobian_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), c->d_jac.p, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = jacobian_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), c->d_jac.p, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(jac, c->d_jac.p, sizeof(double) * ne * nx * nx, cudaMemcpyDeviceToHost, c->stream));
     if (xdot) CU(cudaMemcpyAsync(xdot, c->d_xdot.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
@@ -1840,6 +1911,7 @@ int pfc_radau_init(pfc_ctx* c, int64_t n_env, int max_rule, double h0, double h_
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, "pfc_radau_init: pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_radau_init: negative n_env");
     { const int rc = params_check(c, "pfc_radau_init", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = body_params_check(c, "pfc_radau_init", n_env); if (rc != PFC_OK) return rc; }
     if (max_rule < 1 || max_rule > kRadauMaxRule) return fail(PFC_E_ARG, "pfc_radau_init: max_rule must be 1, 2 or 3");
     if (c->state.n_x < 1 || c->state.n_x > 96) return fail(PFC_E_ARG, "pfc_radau_init: the state must have 1 to 96 entries");
     if (!(std::isfinite(h0) && h0 > 0.0) || !(std::isfinite(h_max) && h_max > 0.0)) return fail(PFC_E_ARG, "pfc_radau_init: h0 and h_max must be finite and positive");
@@ -1866,7 +1938,8 @@ static int radau_check(pfc_ctx* c, const char* who, int64_t n_env) {
     if (!c || !c->finalized || !c->has_dynamics) return fail(PFC_E_ARG, std::string(who) + ": pfc_finalize, pfc_set_bodies and pfc_set_dynamics first");
     if (c->radau.n_env < 0) return fail(PFC_E_ARG, std::string(who) + ": pfc_radau_init first");
     if (n_env != c->radau.n_env) return fail(PFC_E_ARG, std::string(who) + ": n_env differs from the one given to pfc_radau_init");
-    return params_check(c, who, n_env);
+    { const int rc = params_check(c, who, n_env); if (rc != PFC_OK) return rc; }
+    return body_params_check(c, who, n_env);
 }
 
 static void radau_info_reset(pfc_ctx::RadauState& r) {
@@ -1879,8 +1952,10 @@ static void radau_info_reset(pfc_ctx::RadauState& r) {
 // The buffer set is the caller's: the context's own for pfc_radau_step, the compact sub-batch of a roll-out round; the work space is sized
 // for pfc_radau_init's n_env, which n_env never exceeds.  The step info (rounds, synchronisations, phase times) is added to.
 // params: the contact-parameter rows [env][ins] of these environments (or nullptr); they travel like tau_ext, gathered per stage state.
-static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x, const double* tau_ext, const InsParam* params, double* t, double* h_taken,
-                             int32_t* stats) {
+// dyn: their rigid-body data; a body table is reached through dyn.row (or indexed by these environments), the stage evaluations' through
+// the row of each packed state's environment, which the gather kernel writes.
+static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* t,
+                             double* h_taken, int32_t* stats) {
     pfc_ctx::RadauState& r = c->radau;
     const int nx = c->state.n_x, nv = c->state.nv, ni = c->scene.n_ins;
     RadauBufs b{};
@@ -1892,6 +1967,11 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
     if (params) {
         CU(r.paramp.ensure(std::max<size_t>(size_t(r.n_env) * r.s_max * ni, 1)));
         b.params = params; b.paramp = r.paramp.p;
+    }
+    DynDev stage_dyn = dyn;
+    if (dyn.H_env) {
+        CU(r.rowp.ensure(std::max<size_t>(size_t(r.n_env) * r.s_max, 1)));
+        b.row = dyn.row; b.rowp = r.rowp.p; stage_dyn.row = r.rowp.p;
     }
     // phase timing (pfc_set_timing): events around every phase, read after the step's last synchronisation
     std::vector<std::pair<int, int>> marks;   // (phase, index of its start event; the end event follows)
@@ -1918,7 +1998,7 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
     CU(cudaMemsetAsync(r.counts.p, 0, 4 * sizeof(int), c->stream));
     // calcJacobian! once per step: xx_0 and -J (a retry reuses them, radau_solve.jl:23-28)
     CU(mark(0, true));
-    { const int rc = jacobian_device(c, n_env, x, tau_ext, params, r.jac.p, r.xx0.p, r.np.p, r.flags.p, nullptr); if (rc != PFC_OK) return rc; }
+    { const int rc = jacobian_device(c, n_env, x, tau_ext, params, dyn, r.jac.p, r.xx0.p, r.np.p, r.flags.p, nullptr); if (rc != PFC_OK) return rc; }
     CU(launch_radau_prepare(b, r.flags.p, c->d_status.p, c->stream));
     CU(mark(0, false));
     c->launches += 1;
@@ -1942,8 +2022,8 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
             CU(mark(1, true));
             CU(launch_radau_gather(b, n_states, c->stream));
             CU(cudaMemsetAsync(r.Fp.p, 0, sizeof(double) * size_t(n_states) * nx, c->stream));
-            { const int rc = calcxd_device(c, n_states, r.Xp.p, tau_ext ? r.taup.p : nullptr, params ? r.paramp.p : nullptr, r.Fp.p, r.np_stage.p, r.flags_stage.p,
-                                          c->d_status.p); if (rc != PFC_OK) return rc; }
+            { const int rc = calcxd_device(c, n_states, r.Xp.p, tau_ext ? r.taup.p : nullptr, params ? r.paramp.p : nullptr, stage_dyn, r.Fp.p, r.np_stage.p,
+                                          r.flags_stage.p, c->d_status.p); if (rc != PFC_OK) return rc; }
             CU(mark(1, false));
             CU(mark(3, true));
             CU(launch_radau_newton(b, n_active, c->stream));
@@ -1972,7 +2052,7 @@ int pfc_radau_step_device(pfc_ctx* c, int64_t n_env, double* x, const double* ta
     if (!x || !t || !h_taken) return fail(PFC_E_ARG, "pfc_radau_step_device: NULL buffer");
     CU(cudaSetDevice(c->device));
     radau_info_reset(c->radau);
-    return radau_step_device(c, n_env, c->radau.env.p, x, tau_ext, ctx_params(c), t, h_taken, stats);
+    return radau_step_device(c, n_env, c->radau.env.p, x, tau_ext, ctx_params(c), ctx_dyn(c), t, h_taken, stats);
 }
 
 int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
@@ -1988,7 +2068,7 @@ int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, 
     CU(cudaMemcpyAsync(r.t.p, t, sizeof(double) * ne, cudaMemcpyHostToDevice, c->stream));
     if (tau_ext) CU(cudaMemcpyAsync(r.tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
     radau_info_reset(r);
-    const int rc = radau_step_device(c, n_env, r.env.p, r.x.p, tau_ext ? r.tau.p : nullptr, ctx_params(c), r.t.p, r.h.p, r.stats.p);
+    const int rc = radau_step_device(c, n_env, r.env.p, r.x.p, tau_ext ? r.tau.p : nullptr, ctx_params(c), ctx_dyn(c), r.t.p, r.h.p, r.stats.p);
     if (rc != PFC_OK) { cudaStreamSynchronize(c->stream); return rc; }
     CU(cudaMemcpyAsync(x, r.x.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(t, r.t.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
@@ -2027,6 +2107,10 @@ static int radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const dou
     b.stats = r.ro_stats.p; b.list = r.list.p; b.env_c = r.env_c.p; b.x_c = r.x_c.p; b.tau_c = r.tau_c.p; b.t_c = r.t_c.p; b.h_c = r.h_c.p;
     b.h_save = r.h_save.p; b.stats_c = r.stats_c.p; b.count = r.ro_count.p;
     b.params = params; b.params_c = params ? r.params_c.p : nullptr; b.n_ins = c->scene.n_ins;
+    // the compact sub-batch reads a body table where it is, through the slots' environment list (copying the rows of every slot per
+    // round through the one-CTA select kernel cost 7.5 % of the 20-knot roll-out of scripts/run_radau_rollout.py, B200)
+    DynDev dyn_c = ctx_dyn(c);
+    if (dyn_c.H_env) dyn_c.row = r.list.p;
     radau_info_reset(r);
     CU(cudaMemcpyAsync(r.knots.p, t_knot, sizeof(double) * n_knot, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemsetAsync(r.knot.p, 0, sizeof(int) * ne, c->stream));
@@ -2042,8 +2126,8 @@ static int radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const dou
         if (round == 0 && x_knot) CU(cudaMemsetAsync(x_knot, 0xFF, sizeof(double) * n_knot * ne * nx, c->stream));   // all-ones bytes: a NaN
         const long long n_active = r.h_counts[5];
         if (n_active == 0) break;
-        { const int rc = radau_step_device(c, n_active, r.env_c.p, r.x_c.p, tau_ext ? r.tau_c.p : nullptr, params ? r.params_c.p : nullptr, r.t_c.p, r.h_c.p,
-                                           r.stats_c.p); if (rc != PFC_OK) return rc; }
+        { const int rc = radau_step_device(c, n_active, r.env_c.p, r.x_c.p, tau_ext ? r.tau_c.p : nullptr, params ? r.params_c.p : nullptr, dyn_c, r.t_c.p,
+                                           r.h_c.p, r.stats_c.p); if (rc != PFC_OK) return rc; }
         CU(launch_radau_finish(b, n_active, c->stream));
         c->launches += 1;
     }

@@ -82,6 +82,12 @@ struct DynDev {
     const double* H;      // [n_body][36]
     const double* Hinv;   // [n_body][36]
     double gravity[3];
+    // per-environment table (pfc_set_body_params), nullptr while none is set: environment env of a launch reads row
+    // row ? row[env] : env (env = the real environment in the whole-Jacobian mode) instead of H / Hinv / gravity
+    const double* H_env;      // [row][n_body][36]
+    const double* Hinv_env;   // [row][n_body][36]
+    const double* g_env;      // [row][3]
+    const int* row;           // [env] or nullptr
 };
 cudaError_t launch_state_dynamics(const StateDev& sd, const DynDev& dd, long long n_env, int n_ins, int n_bristle, const double* x, const double* wrench,
                                   const double* tau_ext, const double* sdot, double* xdot, cudaStream_t stream, int* n_launches,
@@ -128,6 +134,9 @@ struct RadauBufs {
     double* taup;               // [state][nv] (with tau)
     const InsParam* params;     // [env][n_ins] contact parameters, or nullptr for the scene's own
     InsParam* paramp;           // [state][n_ins] (with params): the environment's rows, gathered next to taup
+    const int* row;             // [env] body-table row of the environment (DynDev::row of the step), or nullptr: identity
+    int* rowp;                  // [state] body-table row of the packed state, or nullptr: with a body table (pfc_set_body_params), the
+                                // DynDev::row of the stage evaluations, so they read the environment's row where it is
     const double* xx0;          // [env][nx] calcXd!(x)
     double* jac;                // [env][nx][nx] d xdot / d x, negated in place into -J
     double* invc;               // [matrix][nx][nx] complex: (h^-1 lambda_i I - J)^-1, matrices in the order of the round's plan

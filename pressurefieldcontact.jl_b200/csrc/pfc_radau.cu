@@ -159,12 +159,13 @@ __global__ void radau_prepare_kernel(RadauBufs b, const int* __restrict__ flags,
     if (bad) atomicOr(status, bad);
 }
 
-// one CTA per packed state: its stage vector (x0 at the first iteration of an attempt, which also initialises the stage), tau_ext and the
-// environment's contact parameters
+// one CTA per packed state: its stage vector (x0 at the first iteration of an attempt, which also initialises the stage), tau_ext, the
+// environment's contact parameters and, with a body table, the environment's row index (the rows themselves are not copied)
 __global__ void __launch_bounds__(64) radau_gather_kernel(RadauBufs b) {
     const long long p = blockIdx.x;
     const int code = b.state_list[p], e = code >> 3, st = code & 7;
     const bool first = b.env[e].k_iter == 0;
+    if (b.rowp && threadIdx.x == 0) b.rowp[p] = b.row ? b.row[e] : e;
     double* Xs = b.X + ((long long)e * b.s_max + st) * b.nx;
     const double* x0 = b.x + (long long)e * b.nx;
     for (int n = threadIdx.x; n < b.nx; n += blockDim.x) {

@@ -236,7 +236,9 @@ PFC_D void emit_row(const XdotOut& o, long long env_real, int row, int seed, boo
     if (first_chunk && o.xdot) o.xdot[env_real * o.n_x + row] = v.v;
 }
 
-template <class T>
+// kTable: read H, H^-1 and gravity from the per-environment table of dd (pfc_set_body_params).  A separate instantiation, so the kernel
+// without a table keeps its registers and stack frame (the run-time select cost the Dual<6> kernel 24 bytes of stack).
+template <class T, bool kTable>
 __global__ void __launch_bounds__(128) state_dynamics_kernel(StateDev sd, DynDev dd, long long n_env, long long n_real, int n_ins, int n_bristle,
                                                              const double* __restrict__ x, int seed0, const double* __restrict__ wrench,
                                                              const double* __restrict__ tau_ext, const double* __restrict__ sdot, XdotOut out,
@@ -266,6 +268,14 @@ __global__ void __launch_bounds__(128) state_dynamics_kernel(StateDev sd, DynDev
         }
         const double* H = dd.H + 36 * b;
         const double* Hi = dd.Hinv + 36 * b;
+        double g[3] = {dd.gravity[0], dd.gravity[1], dd.gravity[2]};
+        if (kTable) {   // the environment's row of the table
+            const long long r = dd.row ? dd.row[er] : er;
+            H = dd.H_env + 36 * (r * sd.n_body + b);
+            Hi = dd.Hinv_env + 36 * (r * sd.n_body + b);
+#pragma unroll
+            for (int i = 0; i < 3; ++i) g[i] = dd.g_env[3 * r + i];
+        }
         T h[6];
 #pragma unroll
         for (int i = 0; i < 6; ++i) {
@@ -291,7 +301,6 @@ __global__ void __launch_bounds__(128) state_dynamics_kernel(StateDev sd, DynDev
         T p[3] = {xr(body.q0), xr(body.q0 + 1), xr(body.q0 + 2)};
         T Rj[9], g_b[3], qd_t[3];
         mrp_to_rot(p, Rj);
-        const double g[3] = {dd.gravity[0], dd.gravity[1], dd.gravity[2]};
         mat_t_vec(fb.R, g, g_b);
         mat_vec(Rj, v + 3, qd_t);
         const T pp = p[0] * p[0] + p[1] * p[1] + p[2] * p[2], pw = p[0] * v[0] + p[1] * v[1] + p[2] * v[2];
@@ -348,7 +357,8 @@ cudaError_t launch_state_dynamics(const StateDev& sd, const DynDev& dd, long lon
                                   const double* tau_ext, const double* sdot, double* xdot, cudaStream_t stream, int* n_launches, const int* flags, int* status) {
     const long long n = n_env * sd.n_body;
     if (n == 0) return cudaSuccess;
-    state_dynamics_kernel<double><<<state_blocks(n), 128, 0, stream>>>(sd, dd, n_env, n_env, n_ins, n_bristle, x, 0, wrench, tau_ext, sdot, XdotOut{xdot, nullptr, sd.n_x}, flags, status);
+    (dd.H_env ? state_dynamics_kernel<double, true> : state_dynamics_kernel<double, false>)<<<state_blocks(n), 128, 0, stream>>>(
+        sd, dd, n_env, n_env, n_ins, n_bristle, x, 0, wrench, tau_ext, sdot, XdotOut{xdot, nullptr, sd.n_x}, flags, status);
     if (n_launches) *n_launches += 1;
     return cudaGetLastError();
 }
@@ -358,8 +368,8 @@ cudaError_t launch_state_dynamics_dual6(const StateDev& sd, const DynDev& dd, lo
                                         int* n_launches, const int* flags, int* status, long long n_real, double* jac) {
     const long long n = n_env * sd.n_body;
     if (n == 0) return cudaSuccess;
-    state_dynamics_kernel<D6><<<state_blocks(n), 128, 0, stream>>>(sd, dd, n_env, n_real > 0 ? n_real : n_env, n_ins, n_bristle, x, seed0, wrench7, tau_ext, sdot7,
-                                                                   XdotOut{xdot7, jac, sd.n_x}, flags, status);
+    (dd.H_env ? state_dynamics_kernel<D6, true> : state_dynamics_kernel<D6, false>)<<<state_blocks(n), 128, 0, stream>>>(
+        sd, dd, n_env, n_real > 0 ? n_real : n_env, n_ins, n_bristle, x, seed0, wrench7, tau_ext, sdot7, XdotOut{xdot7, jac, sd.n_x}, flags, status);
     if (n_launches) *n_launches += 1;
     return cudaGetLastError();
 }
