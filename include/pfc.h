@@ -143,6 +143,35 @@ int pfc_set_dynamics(pfc_ctx* ctx, int n_body, const double* spatial_inertia, co
  * pointer with n_env > 0, a non-finite entry, or a non-symmetric or non-positive-definite inertia (the message names the environment
  * and the body). */
 int pfc_set_body_params(pfc_ctx* ctx, int64_t n_env, const double* spatial_inertia, const double* gravity);
+/* Continuous affine state feedback inside calcXd! (the reference's continuous_controller hook, non_friction.jl:29, restricted to a
+ * piecewise-constant affine law), after pfc_set_dynamics: TVLQR / iLQR forward passes, a PD or LQR prior under sampling MPC, stiff PD
+ * targets.  n_seg segments for n_env environments, row-major:
+ *   K[seg][env][nv][nq + nv]     x_ref[seg][env][nq + nv]
+ * While a table is set, calcXd! of environment e uses the generalized force
+ *   tau = tau_ext[e] + K[seg][e] (x_ref[seg][e] - x[e][0 : nq + nv])
+ * (tau_ext may be NULL: then only the feedback term), evaluated at the state being evaluated (every stage state of a Radau step), so the
+ * integrator sees the feedback law and not a held torque.  The Jacobian entry points include its derivative: d v_dot / d x gains -H^-1 K in
+ * the columns of [q; v] (pfc_calcxd_dual6 in its seed columns below nq + nv; the bristle columns get nothing), so a Radau step treats stiff
+ * gains implicitly.
+ * Which segment applies: pfc_radau_rollout[_device] uses segment k on (t_knot[k-1], t_knot[k]], the interval of tau_ext[k]; n_seg must be
+ * 1 (every interval uses segment 0: one table for a constant PD law) or n_knot, else the roll-out returns PFC_E_ARG and modifies nothing.
+ * Each environment goes through its knots on its own and reads the segment of its own next knot.  pfc_calcxd_f64[_device],
+ * pfc_calcxd_dual6[_device], pfc_calcxd_jacobian[_device] and pfc_radau_step[_device] use segment 0.
+ * Which calls read it: those above; they and pfc_radau_init require n_env to equal the table's.  The contact-only evaluations (pfc_eval_*,
+ * pfc_eval_state_f64[_device], sharded and group calls, pfc_get_*) ignore it.  With contact and body tables set as well, environment e takes
+ * row e of each.
+ * Coordinates: x_ref - x is a plain difference of the raw coordinates (MRPs and translations in q, body-frame [omega; v] in v), not an
+ * error on SO(3); the bristle states s are not fed back.  A Radau step's principal_value! replaces an MRP whose norm exceeds 1 by its shadow
+ * (-p / |p|^2), so an x_ref far from x in MRP terms may describe a nearby attitude; an x_ref taken from this integrator's own output uses
+ * the same shadow sets as the states it is compared with.
+ * n_env = 0 clears the table, and so does a later pfc_set_bodies or pfc_set_dynamics (nq and nv may change).  PFC_E_ARG, with the table in
+ * force unchanged, before pfc_set_dynamics, for n_env outside 0..max_env, n_seg < 1 or n_seg * n_env >= 2^31 with n_env > 0, a NULL
+ * pointer with n_env > 0, or a non-finite entry.
+ * pfc_set_feedback copies from host pointers.  pfc_set_feedback_device reads device pointers during the call: it checks finiteness on the
+ * device (one flag read back, one synchronisation), then copies device to device on the context's stream; both are synchronous at return
+ * and keep no caller pointer.  Calls already queued on the stream read the previous contents. */
+int pfc_set_feedback(pfc_ctx* ctx, int64_t n_env, int n_seg, const double* K, const double* x_ref);
+int pfc_set_feedback_device(pfc_ctx* ctx, int64_t n_env, int n_seg, const double* K, const double* x_ref);
 /* x[env][n_x] -> xdot[env][n_x] = [q_dot; v_dot; s_dot] (copyto!, src/extensions.jl:40-50).  tau_ext[env][nv] = external generalized
  * forces (the controller's tau_ext, :46-47) or NULL.  Host pointers; n_pairs / flags [env][ins] may be NULL. */
 int pfc_calcxd_f64(pfc_ctx* ctx, int64_t n_env, const double* x, const double* tau_ext, double* xdot, int64_t* n_pairs, int32_t* flags);

@@ -216,6 +216,21 @@ function set_body_params!(m::MechanismScenario, H::Union{Array{Float64,3},Nothin
     return nothing
 end
 
+"Continuous affine state feedback inside calcXd! (pfc_set_feedback), after `finalize_floating_gpu!`: calcXd! of environment `env` uses
+`tau_ext + K[:, :, env, seg]' * (x_ref[:, env, seg] - x[1:nq+nv, env])`, with `K[:, i, env, seg]` the gains of generalized force `i`
+((nq + nv) x nv x n_env x n_seg: column-major, so the bytes are pfc.h's K[seg][env][nv][nq + nv]) and `x_ref` (nq + nv) x n_env x n_seg.
+Roll-outs use segment k on the k-th knot interval (n_seg = 1 or n_knot); the other calls use segment 1.  `nothing` clears the table."
+function set_feedback!(m::MechanismScenario, K::Union{Array{Float64,4},Nothing}, x_ref::Union{Array{Float64,3},Nothing}=nothing)
+    if K === nothing
+        check(ccall((:pfc_set_feedback, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Ptr{Float64}, Ptr{Float64}), CTX[m], 0, 0, C_NULL, C_NULL))
+    else
+        (x_ref !== nothing && size(x_ref) == (size(K, 1), size(K, 3), size(K, 4))) || error("x_ref must be (nq + nv) x n_env x n_seg")
+        GC.@preserve K x_ref check(ccall((:pfc_set_feedback, LIB), Cint, (Ptr{Cvoid}, Int64, Cint, Ptr{Float64}, Ptr{Float64}),
+                                         CTX[m], size(K, 3), size(K, 4), K, x_ref))
+    end
+    return nothing
+end
+
 "forceAllElasticIntersections! for a batch of states `x[:, env]`: generalized forces `f[:, env]` and `sdot` (pfc_eval_state_f64)."
 function force_all_batch_gpu!(f::Matrix{Float64}, sdot::Matrix{Float64}, m::MechanismScenario, x::Matrix{Float64})
     GC.@preserve x f sdot check(ccall((:pfc_eval_state_f64, LIB), Cint,

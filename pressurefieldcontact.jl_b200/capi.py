@@ -22,7 +22,7 @@ _vp = C.c_void_p
 SYMBOLS = [
     "pfc_create", "pfc_destroy", "pfc_add_mesh", "pfc_add_instruction", "pfc_finalize", "pfc_set_contact_params", "pfc_eval_f64", "pfc_eval_f64_device",
     "pfc_eval_dual6", "pfc_set_debug", "pfc_get_pairs", "pfc_get_traction", "pfc_set_shard", "pfc_eval_sharded_begin", "pfc_eval_sharded_partials", "pfc_eval_sharded_step", "pfc_sync", "pfc_stream",
-    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_set_body_params", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_rollout", "pfc_radau_rollout_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
+    "pfc_set_bodies", "pfc_eval_state_f64", "pfc_eval_state_f64_device", "pfc_get_boundary", "pfc_set_dynamics", "pfc_set_body_params", "pfc_set_feedback", "pfc_set_feedback_device", "pfc_calcxd_f64", "pfc_calcxd_f64_device", "pfc_calcxd_dual6", "pfc_calcxd_dual6_device", "pfc_calcxd_jacobian", "pfc_calcxd_jacobian_device", "pfc_radau_inv_c_device", "pfc_radau_init", "pfc_radau_step", "pfc_radau_step_device", "pfc_radau_rollout", "pfc_radau_rollout_device", "pfc_radau_step_info", "pfc_refit_mesh", "pfc_launch_count", "pfc_counters", "pfc_measure_fp64_peak", "pfc_set_timing", "pfc_kernel_times", "pfc_last_error", "pfc_version",
     "pfc_comm_unique_id", "pfc_comm_init_rank", "pfc_eval_sharded_f64_device", "pfc_group_create", "pfc_group_destroy", "pfc_group_size", "pfc_group_ctx",
     "pfc_group_add_mesh", "pfc_group_add_instruction", "pfc_group_finalize", "pfc_group_eval_f64",
 ]
@@ -64,6 +64,8 @@ def lib():
         L.pfc_get_boundary.argtypes = [_vp, C.c_int64, _vp, _vp, _vp]
         L.pfc_set_dynamics.argtypes = [_vp, C.c_int, _d, _d]
         L.pfc_set_body_params.argtypes = [_vp, C.c_int64, _vp, _vp]
+        L.pfc_set_feedback.argtypes = [_vp, C.c_int64, C.c_int, _vp, _vp]
+        L.pfc_set_feedback_device.argtypes = [_vp, C.c_int64, C.c_int, _vp, _vp]
         L.pfc_calcxd_f64.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
         L.pfc_calcxd_f64_device.argtypes = [_vp, C.c_int64, _vp, _vp, _vp, _vp, _vp]
         L.pfc_calcxd_dual6.argtypes = [_vp, C.c_int64, _vp, _vp, C.c_int, _vp, _vp, _vp]
@@ -251,6 +253,30 @@ class Context:
         if g.shape != (H.shape[0], 3):
             raise ValueError(f"gravity must have shape [{H.shape[0]}, 3], got {g.shape}")
         _check(lib().pfc_set_body_params(self._h, H.shape[0], _p(H), _p(g)))
+
+    def set_feedback(self, K, x_ref=None):
+        """Continuous affine state feedback inside calcXd!: tau = tau_ext + K[seg][env] (x_ref[seg][env] - x[env][:nq + nv]) with
+        K[n_seg][n_env][nv][nq + nv] and x_ref[n_seg][n_env][nq + nv].  numpy arrays go through pfc_set_feedback, CUDA torch tensors
+        (float64, contiguous, on this context's device) through pfc_set_feedback_device; None clears the table."""
+        if K is None:
+            _check(lib().pfc_set_feedback(self._h, 0, 0, None, None))
+            return
+        nc = self.nq + self.nv
+        if K.ndim != 4 or tuple(K.shape[2:]) != (self.nv, nc):
+            raise ValueError(f"K must have shape [n_seg, n_env, {self.nv}, {nc}], got {tuple(K.shape)}")
+        if x_ref is None or tuple(x_ref.shape) != (K.shape[0], K.shape[1], nc):
+            raise ValueError(f"x_ref must have shape [{K.shape[0]}, {K.shape[1]}, {nc}], got {None if x_ref is None else tuple(x_ref.shape)}")
+        n_seg, n_env = int(K.shape[0]), int(K.shape[1])
+        if isinstance(K, np.ndarray):
+            Ka, xa = _a(K), _a(x_ref)
+            _check(lib().pfc_set_feedback(self._h, n_env, n_seg, _p(Ka), _p(xa)))
+            return
+        for name, t in (("K", K), ("x_ref", x_ref)):
+            if not (getattr(t, "is_cuda", False) and str(t.dtype) == "torch.float64" and t.is_contiguous() and t.device.index == self.device):
+                raise TypeError(f"{name} must be a numpy array or a contiguous float64 CUDA tensor on device {self.device}")
+        import torch
+        torch.cuda.current_stream(K.device).synchronize()   # the library reads the tensors on its own stream
+        _check(lib().pfc_set_feedback_device(self._h, n_env, n_seg, K.data_ptr(), x_ref.data_ptr()))
 
     def calcxd_f64(self, x, tau_ext=None):
         """x[env][n_x] (host) -> dict(xdot[env][n_x], n_pairs, flags)."""

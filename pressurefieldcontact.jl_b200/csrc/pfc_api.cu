@@ -232,6 +232,7 @@ struct pfc_ctx {
         DevBuf<double> X, Xp, Fp, taup, xx0, jac, invc, shift, x, tau, t, h;
         DevBuf<InsParam> paramp, params_c;   // contact-parameter rows gathered per stage state / per compact roll-out slot: grown on first use
         DevBuf<int> rowp;                    // body table: row of each stage state (DynDev::row of the stage evaluations), grown on first use
+        DevBuf<int> fb_rowp, fb_list;        // feedback table: row of each stage state / compact roll-out slot (FeedbackDev::row), grown on first use
         DevBuf<int> index, state_list, env_list, state_pos, inv_base, counts, stats, flags, flags_stage, info;
         DevBuf<long long> np, np_stage;
         // roll-outs (pfc_radau_rollout): grown on first use
@@ -253,6 +254,11 @@ struct pfc_ctx {
     // per-environment body parameters (pfc_set_body_params): H, H^-1 [env][body][36] and gravity [env][3]; body_n_env = 0 while no table is set
     DevBuf<double> d_body_H, d_body_Hinv, d_body_g;
     int64_t body_n_env = 0;
+    // continuous affine state feedback (pfc_set_feedback): K [seg][env][nv][nq + nv], x_ref [seg][env][nq + nv]; fb_n_env = 0 while no table is set
+    DevBuf<double> d_fb_K, d_fb_xref;
+    DevBuf<int> d_fb_bad;
+    int64_t fb_n_env = 0;
+    int fb_n_seg = 0;
 };
 
 namespace {
@@ -1389,6 +1395,7 @@ int pfc_set_bodies(pfc_ctx* c, int n_body, const int32_t* joint_type, const int3
     if (!c || !c->finalized) return fail(PFC_E_ARG, "pfc_set_bodies: call after pfc_finalize");
     if (n_body < 1 || !joint_type || !q0 || !v0 || !mesh_body || nq < 0 || nv < 0) return fail(PFC_E_ARG, "pfc_set_bodies: bad argument");
     c->body_n_env = 0;   // a body table's rows were checked against the previous mechanism
+    c->fb_n_env = 0;     // and a feedback table's rows have the previous nq and nv
     c->h_bodies.assign(n_body, BodyDev{});
     for (int b = 0; b < n_body; ++b) {
         BodyDev& d = c->h_bodies[b];
@@ -1548,6 +1555,7 @@ int pfc_set_dynamics(pfc_ctx* c, int n_body, const double* spatial_inertia, cons
     }
     CU(cudaSetDevice(c->device));
     c->body_n_env = 0;   // a body table's rows were checked against the previous mechanism
+    c->fb_n_env = 0;     // a feedback table is cleared with it (pfc_set_feedback documents both)
     CU(c->d_H.ensure(H.size())); CU(c->d_Hinv.ensure(Hi.size()));
     CU(cudaMemcpy(c->d_H.p, H.data(), sizeof(double) * H.size(), cudaMemcpyHostToDevice));
     CU(cudaMemcpy(c->d_Hinv.p, Hi.data(), sizeof(double) * Hi.size(), cudaMemcpyHostToDevice));
@@ -1610,8 +1618,83 @@ int pfc_set_body_params(pfc_ctx* c, int64_t n_env, const double* spatial_inertia
     return PFC_OK;
 }
 
-static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* xdot,
-                         long long* n_pairs, int* flags, int* status = nullptr) {
+// ---- continuous affine state feedback -------------------------------------------------------------------------------------
+// the feedback of an entry point: segment 0 of the context's table (K = nullptr while none is set); a roll-out maps its own rows
+static FeedbackDev ctx_feedback(const pfc_ctx* c) {
+    FeedbackDev f{};
+    f.ncol = c->state.nq + c->state.nv;
+    if (c->fb_n_env > 0) { f.K = c->d_fb_K.p; f.x_ref = c->d_fb_xref.p; }
+    return f;
+}
+static int feedback_check(const pfc_ctx* c, const char* who, int64_t n_env) {
+    if (c->fb_n_env > 0 && n_env != c->fb_n_env)
+        return fail(PFC_E_ARG, std::string(who) + ": n_env differs from the batch of the feedback table (pfc_set_feedback)");
+    return PFC_OK;
+}
+
+// The checks both entry points share; 1 when the arguments describe a table to copy, PFC_OK after clearing it, or the error.
+static int feedback_args(pfc_ctx* c, const char* who, int64_t n_env, int n_seg, const double* K, const double* x_ref) {
+    if (!c || !c->has_dynamics) return fail(PFC_E_ARG, std::string(who) + ": call after pfc_set_dynamics");
+    if (n_env < 0 || n_env > c->max_env) return fail(PFC_E_ARG, std::string(who) + ": n_env must be in 0..max_env");
+    if (n_env == 0) {   // back to open-loop calcXd! (the buffers are kept for the next table)
+        c->fb_n_env = 0;
+        return PFC_OK;
+    }
+    if (n_seg < 1) return fail(PFC_E_ARG, std::string(who) + ": n_seg must be at least 1");
+    if (int64_t(n_seg) * n_env > INT32_MAX) return fail(PFC_E_ARG, std::string(who) + ": n_seg * n_env must fit in 32 bits");
+    if (!K || !x_ref) return fail(PFC_E_ARG, std::string(who) + ": K or x_ref is NULL");
+    return 1;
+}
+// Room for a table of n_k entries of K and n_x of x_ref.  The calls already queued read the previous table, so they finish before it is freed.
+static int feedback_reserve(pfc_ctx* c, size_t n_k, size_t n_x) {
+    if (n_k > c->d_fb_K.n || n_x > c->d_fb_xref.n) {
+        CU(cudaStreamSynchronize(c->stream));
+        c->fb_n_env = 0;   // (growing frees the previous table: should the allocation fail, no table is left in force)
+        CU(c->d_fb_K.ensure(n_k)); CU(c->d_fb_xref.ensure(n_x));
+    }
+    return PFC_OK;
+}
+
+int pfc_set_feedback(pfc_ctx* c, int64_t n_env, int n_seg, const double* K, const double* x_ref) {
+    { const int rc = feedback_args(c, "pfc_set_feedback", n_env, n_seg, K, x_ref); if (rc != 1) return rc; }
+    const size_t ncol = size_t(c->state.nq + c->state.nv), rows = size_t(n_seg) * size_t(n_env);
+    const size_t n_k = rows * size_t(c->state.nv) * ncol, n_x = rows * ncol;
+    for (size_t i = 0; i < n_k; ++i) if (!std::isfinite(K[i])) return fail(PFC_E_ARG, "pfc_set_feedback: non-finite entry of K");
+    for (size_t i = 0; i < n_x; ++i) if (!std::isfinite(x_ref[i])) return fail(PFC_E_ARG, "pfc_set_feedback: non-finite entry of x_ref");
+    CU(cudaSetDevice(c->device));
+    { const int rc = feedback_reserve(c, n_k, n_x); if (rc != PFC_OK) return rc; }
+    CU(cudaMemcpyAsync(c->d_fb_K.p, K, sizeof(double) * n_k, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->d_fb_xref.p, x_ref, sizeof(double) * n_x, cudaMemcpyHostToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));   // complete before the caller's arrays go
+    c->fb_n_env = n_env; c->fb_n_seg = n_seg;
+    return PFC_OK;
+}
+
+int pfc_set_feedback_device(pfc_ctx* c, int64_t n_env, int n_seg, const double* K, const double* x_ref) {
+    { const int rc = feedback_args(c, "pfc_set_feedback_device", n_env, n_seg, K, x_ref); if (rc != 1) return rc; }
+    const size_t ncol = size_t(c->state.nq + c->state.nv), rows = size_t(n_seg) * size_t(n_env);
+    const size_t n_k = rows * size_t(c->state.nv) * ncol, n_x = rows * ncol;
+    CU(cudaSetDevice(c->device));
+    // finiteness on the device, from the caller's buffers: one flag back
+    CU(c->d_fb_bad.ensure(1));
+    CU(cudaMemsetAsync(c->d_fb_bad.p, 0, sizeof(int), c->stream));
+    CU(launch_check_finite(K, (long long)n_k, c->d_fb_bad.p, c->stream));
+    CU(launch_check_finite(x_ref, (long long)n_x, c->d_fb_bad.p, c->stream));
+    c->launches += 2;
+    int bad = 0;
+    CU(cudaMemcpyAsync(&bad, c->d_fb_bad.p, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+    CU(cudaStreamSynchronize(c->stream));
+    if (bad) return fail(PFC_E_ARG, "pfc_set_feedback_device: non-finite entry of K or x_ref");
+    { const int rc = feedback_reserve(c, n_k, n_x); if (rc != PFC_OK) return rc; }
+    CU(cudaMemcpyAsync(c->d_fb_K.p, K, sizeof(double) * n_k, cudaMemcpyDeviceToDevice, c->stream));
+    CU(cudaMemcpyAsync(c->d_fb_xref.p, x_ref, sizeof(double) * n_x, cudaMemcpyDeviceToDevice, c->stream));
+    CU(cudaStreamSynchronize(c->stream));   // the library keeps no caller pointer
+    c->fb_n_env = n_env; c->fb_n_seg = n_seg;
+    return PFC_OK;
+}
+
+static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, const FeedbackDev& fb,
+                         double* xdot, long long* n_pairs, int* flags, int* status = nullptr) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle);
     CU(c->d_X.ensure(16 * ne * ni)); CU(c->d_tw.ensure(6 * ne * ni)); CU(c->d_w.ensure(6 * ne * ni));
     if (nb) { CU(c->d_s.ensure(6 * ne * nb)); CU(c->d_sd.ensure(6 * ne * nb)); }
@@ -1623,6 +1706,7 @@ static int calcxd_device(pfc_ctx* c, int64_t n_env, const double* x, const doubl
     int rc = eval_device(c, io);
     if (rc != PFC_OK) return rc;
     CU(launch_state_dynamics(c->state, dyn, n_env, int(ni), int(nb), x, c->d_w.p, tau_ext, nb ? c->d_sd.p : nullptr, xdot, c->stream, &nl, flags, status));
+    if (fb.K) CU(launch_state_feedback(c->state, dyn, fb, n_env, x, 0, 0, xdot, nullptr, c->stream, &nl));
     c->launches += nl;
     return PFC_OK;
 }
@@ -1632,10 +1716,11 @@ int pfc_calcxd_f64_device(pfc_ctx* c, int64_t n_env, const double* x, const doub
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_f64_device", n_env); if (rc != PFC_OK) return rc; }
     { const int rc = body_params_check(c, "pfc_calcxd_f64_device", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = feedback_check(c, "pfc_calcxd_f64_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_f64_device: NULL buffer");
     CU(cudaSetDevice(c->device));
-    return calcxd_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), xdot, reinterpret_cast<long long*>(n_pairs), flags);
+    return calcxd_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), ctx_feedback(c), xdot, reinterpret_cast<long long*>(n_pairs), flags);
 }
 
 int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* xdot, int64_t* n_pairs, int32_t* flags) {
@@ -1643,6 +1728,7 @@ int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_f64: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_f64", n_env); if (rc != PFC_OK) return rc; }
     { const int rc = body_params_check(c, "pfc_calcxd_f64", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = feedback_check(c, "pfc_calcxd_f64", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot) return fail(PFC_E_ARG, "pfc_calcxd_f64: NULL buffer");
     CU(cudaSetDevice(c->device));
@@ -1655,7 +1741,8 @@ int pfc_calcxd_f64(pfc_ctx* c, int64_t n_env, const double* x, const double* tau
     }
     CU(cudaMemsetAsync(c->d_xdot.p, 0, sizeof(double) * ne * nx, c->stream));
     CU(status_begin(c));
-    int rc = calcxd_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = calcxd_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), ctx_feedback(c), c->d_xdot.p, c->d_np.p, c->d_fl.p,
+                           c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(xdot, c->d_xdot.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     if (n_pairs) CU(cudaMemcpyAsync(n_pairs, c->d_np.p, sizeof(long long) * ne * ni, cudaMemcpyDeviceToHost, c->stream));
@@ -1697,9 +1784,8 @@ static int dual_shared_f64(pfc_ctx* c, int64_t n_env, long long* n_pairs, int* f
 // calcXd! in Jacobian mode for the same scenes: x (Float64) with Dual seeds on x[seed_start .. seed_start + 6) -> x_dot as 7 doubles per
 // entry (value, then d x_dot / d x[seed_start + k]).  Device pipeline: Float64 prologue + broad phase (the reference always traverses
 // with m.float), Dual prologue, Dual narrow phase / friction (pfc_dual.cu), Dual J' w and rigid-body terms.
-static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, int seed_start,
-                                    double* xdot7,
-                                    long long* n_pairs, int* flags, int* status) {
+static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn,
+                                    const FeedbackDev& fb, int seed_start, double* xdot7, long long* n_pairs, int* flags, int* status) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle);
     CU(c->d_X.ensure(16 * ne * ni)); CU(c->d_tw.ensure(6 * ne * ni));
     CU(c->d_X7.ensure(112 * ne * ni)); CU(c->d_tw7.ensure(42 * ne * ni)); CU(c->d_w7.ensure(42 * ne * ni)); CU(c->d_dual_ticket.ensure(1));
@@ -1721,12 +1807,13 @@ static int calcxd_dual6_device_once(pfc_ctx* c, int64_t n_env, const double* x, 
     }
     CU(launch_state_dynamics_dual6(c->state, dyn, n_env, int(ni), int(nb), x, seed_start, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr, xdot7,
                                    c->stream, &nl, flags, status));
+    if (fb.K) CU(launch_state_feedback(c->state, dyn, fb, n_env, x, 1, seed_start, xdot7, nullptr, c->stream, &nl));
     c->launches += nl + 1;
     return PFC_OK;
 }
-static int calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, int seed_start,
-                               double* xdot7, long long* n_pairs, int* flags, int* status) {
-    PFC_REQUEUE_LOOP({ const int rc_ = calcxd_dual6_device_once(c, n_env, x, tau_ext, params, dyn, seed_start, xdot7, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
+static int calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn,
+                               const FeedbackDev& fb, int seed_start, double* xdot7, long long* n_pairs, int* flags, int* status) {
+    PFC_REQUEUE_LOOP({ const int rc_ = calcxd_dual6_device_once(c, n_env, x, tau_ext, params, dyn, fb, seed_start, xdot7, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
     return PFC_OK;
 }
 
@@ -1736,11 +1823,13 @@ int pfc_calcxd_dual6_device(pfc_ctx* c, int64_t n_env, const double* x, const do
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_dual6_device", n_env); if (rc != PFC_OK) return rc; }
     { const int rc = body_params_check(c, "pfc_calcxd_dual6_device", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = feedback_check(c, "pfc_calcxd_dual6_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot7 || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: NULL buffer");
     if (seed_start < 0 || seed_start >= c->state.n_x) return fail(PFC_E_ARG, "pfc_calcxd_dual6_device: seed_start out of range");
     CU(cudaSetDevice(c->device));
-    return calcxd_dual6_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), seed_start, xdot7, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
+    return calcxd_dual6_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), ctx_feedback(c), seed_start, xdot7, reinterpret_cast<long long*>(n_pairs), flags,
+                               nullptr);
 }
 
 int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, int seed_start, double* xdot7, int64_t* n_pairs, int32_t* flags) {
@@ -1748,6 +1837,7 @@ int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* t
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_dual6: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_dual6", n_env); if (rc != PFC_OK) return rc; }
     { const int rc = body_params_check(c, "pfc_calcxd_dual6", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = feedback_check(c, "pfc_calcxd_dual6", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !xdot7) return fail(PFC_E_ARG, "pfc_calcxd_dual6: NULL buffer");
     if (seed_start < 0 || seed_start >= c->state.n_x) return fail(PFC_E_ARG, "pfc_calcxd_dual6: seed_start out of range");
@@ -1761,7 +1851,8 @@ int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* t
     }
     CU(cudaMemsetAsync(c->d_xdot.p, 0, sizeof(double) * 7 * ne * nx, c->stream));
     CU(status_begin(c));
-    int rc = calcxd_dual6_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), seed_start, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = calcxd_dual6_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), ctx_feedback(c), seed_start, c->d_xdot.p, c->d_np.p,
+                                 c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(xdot7, c->d_xdot.p, sizeof(double) * 7 * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     if (n_pairs) CU(cudaMemcpyAsync(n_pairs, c->d_np.p, sizeof(long long) * ne * ni, cudaMemcpyDeviceToHost, c->stream));
@@ -1776,8 +1867,8 @@ int pfc_calcxd_dual6(pfc_ctx* c, int64_t n_env, const double* x, const double* t
 // seed chunks are a grid axis of the Dual kernels ("environment" (g, env) = chunk g of real environment env) as far as the work space
 // allows, and the rigid-body kernel writes the partials straight into jac[env][row][col].  Scenes with bristle instructions go chunk by
 // chunk (their reference-order pipeline is sized per real environment) but still share the broad phase.
-static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* jac, double* xdot,
-                                long long* n_pairs, int* flags, int* status) {
+static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn,
+                                const FeedbackDev& fb, double* jac, double* xdot, long long* n_pairs, int* flags, int* status) {
     const size_t ne = size_t(n_env), ni = size_t(c->scene.n_ins), nb = size_t(c->n_bristle), nx = size_t(c->state.n_x);
     const int n_chunk = int((nx + 5) / 6);
     // chunks per pass: all of them if the Dual boundary arrays (196 doubles per (chunk, environment, instruction)) stay below 1 GiB
@@ -1806,12 +1897,13 @@ static int jacobian_device_once(pfc_ctx* c, int64_t n_env, const double* x, cons
         CU(launch_state_dynamics_dual6(c->state, dyn, n_virtual, int(ni), int(nb), x, 6 * g0, c->d_w7.p, tau_ext, nb ? c->d_sd7.p : nullptr,
                                        g0 == 0 ? xdot : nullptr, c->stream, &nl, flags, status, n_env, jac));
     }
+    if (fb.K) CU(launch_state_feedback(c->state, dyn, fb, n_env, x, 2, 0, xdot, jac, c->stream, &nl));   // -H^-1 K once, after every chunk
     c->launches += nl;
     return PFC_OK;
 }
-static int jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* jac, double* xdot,
-                           long long* n_pairs, int* flags, int* status) {
-    PFC_REQUEUE_LOOP({ const int rc_ = jacobian_device_once(c, n_env, x, tau_ext, params, dyn, jac, xdot, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
+static int jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, const FeedbackDev& fb,
+                           double* jac, double* xdot, long long* n_pairs, int* flags, int* status) {
+    PFC_REQUEUE_LOOP({ const int rc_ = jacobian_device_once(c, n_env, x, tau_ext, params, dyn, fb, jac, xdot, n_pairs, flags, status); if (rc_ != PFC_OK) return rc_; })
     return PFC_OK;
 }
 
@@ -1821,10 +1913,11 @@ int pfc_calcxd_jacobian_device(pfc_ctx* c, int64_t n_env, const double* x, const
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_jacobian_device", n_env); if (rc != PFC_OK) return rc; }
     { const int rc = body_params_check(c, "pfc_calcxd_jacobian_device", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = feedback_check(c, "pfc_calcxd_jacobian_device", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !jac || !n_pairs || !flags) return fail(PFC_E_ARG, "pfc_calcxd_jacobian_device: NULL buffer");
     CU(cudaSetDevice(c->device));
-    return jacobian_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), jac, xdot, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
+    return jacobian_device(c, n_env, x, tau_ext, ctx_params(c), ctx_dyn(c), ctx_feedback(c), jac, xdot, reinterpret_cast<long long*>(n_pairs), flags, nullptr);
 }
 
 int pfc_calcxd_jacobian(pfc_ctx* c, int64_t n_env, const double* x, const double* tau_ext, double* jac, double* xdot, int64_t* n_pairs, int32_t* flags) {
@@ -1832,6 +1925,7 @@ int pfc_calcxd_jacobian(pfc_ctx* c, int64_t n_env, const double* x, const double
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: negative n_env");
     { const int rc = params_check(c, "pfc_calcxd_jacobian", n_env); if (rc != PFC_OK) return rc; }
     { const int rc = body_params_check(c, "pfc_calcxd_jacobian", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = feedback_check(c, "pfc_calcxd_jacobian", n_env); if (rc != PFC_OK) return rc; }
     if (n_env == 0) return PFC_OK;   // an empty batch is a no-op whatever the pointers are
     if (!x || !jac) return fail(PFC_E_ARG, "pfc_calcxd_jacobian: NULL buffer");
     CU(cudaSetDevice(c->device));
@@ -1843,7 +1937,8 @@ int pfc_calcxd_jacobian(pfc_ctx* c, int64_t n_env, const double* x, const double
         CU(cudaMemcpyAsync(c->d_tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
     }
     CU(status_begin(c));
-    int rc = jacobian_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), c->d_jac.p, c->d_xdot.p, c->d_np.p, c->d_fl.p, c->d_status.p);
+    int rc = jacobian_device(c, n_env, c->d_x.p, tau_ext ? c->d_tau.p : nullptr, ctx_params(c), ctx_dyn(c), ctx_feedback(c), c->d_jac.p, c->d_xdot.p, c->d_np.p,
+                             c->d_fl.p, c->d_status.p);
     if (rc != PFC_OK) return rc;
     CU(cudaMemcpyAsync(jac, c->d_jac.p, sizeof(double) * ne * nx * nx, cudaMemcpyDeviceToHost, c->stream));
     if (xdot) CU(cudaMemcpyAsync(xdot, c->d_xdot.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
@@ -1912,6 +2007,7 @@ int pfc_radau_init(pfc_ctx* c, int64_t n_env, int max_rule, double h0, double h_
     if (n_env < 0) return fail(PFC_E_ARG, "pfc_radau_init: negative n_env");
     { const int rc = params_check(c, "pfc_radau_init", n_env); if (rc != PFC_OK) return rc; }
     { const int rc = body_params_check(c, "pfc_radau_init", n_env); if (rc != PFC_OK) return rc; }
+    { const int rc = feedback_check(c, "pfc_radau_init", n_env); if (rc != PFC_OK) return rc; }
     if (max_rule < 1 || max_rule > kRadauMaxRule) return fail(PFC_E_ARG, "pfc_radau_init: max_rule must be 1, 2 or 3");
     if (c->state.n_x < 1 || c->state.n_x > 96) return fail(PFC_E_ARG, "pfc_radau_init: the state must have 1 to 96 entries");
     if (!(std::isfinite(h0) && h0 > 0.0) || !(std::isfinite(h_max) && h_max > 0.0)) return fail(PFC_E_ARG, "pfc_radau_init: h0 and h_max must be finite and positive");
@@ -1939,7 +2035,8 @@ static int radau_check(pfc_ctx* c, const char* who, int64_t n_env) {
     if (c->radau.n_env < 0) return fail(PFC_E_ARG, std::string(who) + ": pfc_radau_init first");
     if (n_env != c->radau.n_env) return fail(PFC_E_ARG, std::string(who) + ": n_env differs from the one given to pfc_radau_init");
     { const int rc = params_check(c, who, n_env); if (rc != PFC_OK) return rc; }
-    return body_params_check(c, who, n_env);
+    { const int rc = body_params_check(c, who, n_env); if (rc != PFC_OK) return rc; }
+    return feedback_check(c, who, n_env);
 }
 
 static void radau_info_reset(pfc_ctx::RadauState& r) {
@@ -1953,9 +2050,9 @@ static void radau_info_reset(pfc_ctx::RadauState& r) {
 // for pfc_radau_init's n_env, which n_env never exceeds.  The step info (rounds, synchronisations, phase times) is added to.
 // params: the contact-parameter rows [env][ins] of these environments (or nullptr); they travel like tau_ext, gathered per stage state.
 // dyn: their rigid-body data; a body table is reached through dyn.row (or indexed by these environments), the stage evaluations' through
-// the row of each packed state's environment, which the gather kernel writes.
-static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn, double* t,
-                             double* h_taken, int32_t* stats) {
+// the row of each packed state's environment, which the gather kernel writes.  fb: their feedback, reached the same way through fb.row.
+static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x, const double* tau_ext, const InsParam* params, const DynDev& dyn,
+                             const FeedbackDev& fb, double* t, double* h_taken, int32_t* stats) {
     pfc_ctx::RadauState& r = c->radau;
     const int nx = c->state.n_x, nv = c->state.nv, ni = c->scene.n_ins;
     RadauBufs b{};
@@ -1972,6 +2069,11 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
     if (dyn.H_env) {
         CU(r.rowp.ensure(std::max<size_t>(size_t(r.n_env) * r.s_max, 1)));
         b.row = dyn.row; b.rowp = r.rowp.p; stage_dyn.row = r.rowp.p;
+    }
+    FeedbackDev stage_fb = fb;
+    if (fb.K) {
+        CU(r.fb_rowp.ensure(std::max<size_t>(size_t(r.n_env) * r.s_max, 1)));
+        b.fb_row = fb.row; b.fb_rowp = r.fb_rowp.p; stage_fb.row = r.fb_rowp.p;
     }
     // phase timing (pfc_set_timing): events around every phase, read after the step's last synchronisation
     std::vector<std::pair<int, int>> marks;   // (phase, index of its start event; the end event follows)
@@ -1998,7 +2100,7 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
     CU(cudaMemsetAsync(r.counts.p, 0, 4 * sizeof(int), c->stream));
     // calcJacobian! once per step: xx_0 and -J (a retry reuses them, radau_solve.jl:23-28)
     CU(mark(0, true));
-    { const int rc = jacobian_device(c, n_env, x, tau_ext, params, dyn, r.jac.p, r.xx0.p, r.np.p, r.flags.p, nullptr); if (rc != PFC_OK) return rc; }
+    { const int rc = jacobian_device(c, n_env, x, tau_ext, params, dyn, fb, r.jac.p, r.xx0.p, r.np.p, r.flags.p, nullptr); if (rc != PFC_OK) return rc; }
     CU(launch_radau_prepare(b, r.flags.p, c->d_status.p, c->stream));
     CU(mark(0, false));
     c->launches += 1;
@@ -2022,8 +2124,8 @@ static int radau_step_device(pfc_ctx* c, int64_t n_env, RadauEnv* env, double* x
             CU(mark(1, true));
             CU(launch_radau_gather(b, n_states, c->stream));
             CU(cudaMemsetAsync(r.Fp.p, 0, sizeof(double) * size_t(n_states) * nx, c->stream));
-            { const int rc = calcxd_device(c, n_states, r.Xp.p, tau_ext ? r.taup.p : nullptr, params ? r.paramp.p : nullptr, stage_dyn, r.Fp.p, r.np_stage.p,
-                                          r.flags_stage.p, c->d_status.p); if (rc != PFC_OK) return rc; }
+            { const int rc = calcxd_device(c, n_states, r.Xp.p, tau_ext ? r.taup.p : nullptr, params ? r.paramp.p : nullptr, stage_dyn, stage_fb, r.Fp.p,
+                                          r.np_stage.p, r.flags_stage.p, c->d_status.p); if (rc != PFC_OK) return rc; }
             CU(mark(1, false));
             CU(mark(3, true));
             CU(launch_radau_newton(b, n_active, c->stream));
@@ -2052,7 +2154,7 @@ int pfc_radau_step_device(pfc_ctx* c, int64_t n_env, double* x, const double* ta
     if (!x || !t || !h_taken) return fail(PFC_E_ARG, "pfc_radau_step_device: NULL buffer");
     CU(cudaSetDevice(c->device));
     radau_info_reset(c->radau);
-    return radau_step_device(c, n_env, c->radau.env.p, x, tau_ext, ctx_params(c), ctx_dyn(c), t, h_taken, stats);
+    return radau_step_device(c, n_env, c->radau.env.p, x, tau_ext, ctx_params(c), ctx_dyn(c), ctx_feedback(c), t, h_taken, stats);
 }
 
 int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, double* t, double* h_taken, int32_t* stats) {
@@ -2068,7 +2170,7 @@ int pfc_radau_step(pfc_ctx* c, int64_t n_env, double* x, const double* tau_ext, 
     CU(cudaMemcpyAsync(r.t.p, t, sizeof(double) * ne, cudaMemcpyHostToDevice, c->stream));
     if (tau_ext) CU(cudaMemcpyAsync(r.tau.p, tau_ext, sizeof(double) * ne * nv, cudaMemcpyHostToDevice, c->stream));
     radau_info_reset(r);
-    const int rc = radau_step_device(c, n_env, r.env.p, r.x.p, tau_ext ? r.tau.p : nullptr, ctx_params(c), ctx_dyn(c), r.t.p, r.h.p, r.stats.p);
+    const int rc = radau_step_device(c, n_env, r.env.p, r.x.p, tau_ext ? r.tau.p : nullptr, ctx_params(c), ctx_dyn(c), ctx_feedback(c), r.t.p, r.h.p, r.stats.p);
     if (rc != PFC_OK) { cudaStreamSynchronize(c->stream); return rc; }
     CU(cudaMemcpyAsync(x, r.x.p, sizeof(double) * ne * nx, cudaMemcpyDeviceToHost, c->stream));
     CU(cudaMemcpyAsync(t, r.t.p, sizeof(double) * ne, cudaMemcpyDeviceToHost, c->stream));
@@ -2087,6 +2189,8 @@ static int radau_rollout_check(pfc_ctx* c, const char* who, int64_t n_env, int n
         if (k > 0 && !(t_knot[k] - t_knot[k - 1] >= kRadauHMin)) return fail(PFC_E_ARG, std::string(who) + ": knot times must increase by at least h_min = 1e-8");
     }
     if (max_steps < 1) return fail(PFC_E_ARG, std::string(who) + ": max_steps must be at least 1");
+    if (c->fb_n_env > 0 && c->fb_n_seg != 1 && c->fb_n_seg != n_knot)
+        return fail(PFC_E_ARG, std::string(who) + ": the feedback table (pfc_set_feedback) must have 1 or n_knot segments");
     return PFC_OK;
 }
 
@@ -2111,6 +2215,12 @@ static int radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const dou
     // round through the one-CTA select kernel cost 7.5 % of the 20-knot roll-out of scripts/run_radau_rollout.py, B200)
     DynDev dyn_c = ctx_dyn(c);
     if (dyn_c.H_env) dyn_c.row = r.list.p;
+    // a feedback table likewise: the select kernel writes each slot's row (segment of its next knot, environment) into fb_list
+    FeedbackDev fb_c = ctx_feedback(c);
+    if (fb_c.K) {
+        CU(r.fb_list.ensure(ne));
+        b.n_seg = c->fb_n_seg; b.fb_list = r.fb_list.p; fb_c.row = r.fb_list.p;
+    }
     radau_info_reset(r);
     CU(cudaMemcpyAsync(r.knots.p, t_knot, sizeof(double) * n_knot, cudaMemcpyHostToDevice, c->stream));
     CU(cudaMemsetAsync(r.knot.p, 0, sizeof(int) * ne, c->stream));
@@ -2126,8 +2236,8 @@ static int radau_rollout_device(pfc_ctx* c, int64_t n_env, int n_knot, const dou
         if (round == 0 && x_knot) CU(cudaMemsetAsync(x_knot, 0xFF, sizeof(double) * n_knot * ne * nx, c->stream));   // all-ones bytes: a NaN
         const long long n_active = r.h_counts[5];
         if (n_active == 0) break;
-        { const int rc = radau_step_device(c, n_active, r.env_c.p, r.x_c.p, tau_ext ? r.tau_c.p : nullptr, params ? r.params_c.p : nullptr, dyn_c, r.t_c.p,
-                                           r.h_c.p, r.stats_c.p); if (rc != PFC_OK) return rc; }
+        { const int rc = radau_step_device(c, n_active, r.env_c.p, r.x_c.p, tau_ext ? r.tau_c.p : nullptr, params ? r.params_c.p : nullptr, dyn_c, fb_c,
+                                           r.t_c.p, r.h_c.p, r.stats_c.p); if (rc != PFC_OK) return rc; }
         CU(launch_radau_finish(b, n_active, c->stream));
         c->launches += 1;
     }

@@ -106,6 +106,25 @@ cudaError_t launch_state_dynamics_dual6(const StateDev& sd, const DynDev& dd, lo
 cudaError_t launch_state_epilogue(const StateDev& sd, long long n_env, int n_ins, const double* x, const double* wrench, double* f_gen, cudaStream_t stream,
                                   int* n_launches, const int* flags = nullptr, int* status = nullptr);
 
+// continuous affine state feedback (pfc_set_feedback): tau += K (x_ref - x) on top of calcXd!.  K == nullptr while no table is set.
+// Environment env of a launch reads table row r = row ? row[env] : env (a row is seg * n_env + env of the table).
+struct FeedbackDev {
+    const double* K;       // [r][nv][ncol]
+    const double* x_ref;   // [r][ncol]
+    int ncol;              // nq + nv: the bristle states are not fed back
+    const int* row;        // [env] or nullptr
+};
+// The feedback term added to what launch_state_dynamics[_dual6] wrote for the same n_env (real) environments.  v_dot is linear in the
+// generalized force, so the term is H^-1 K (x_ref - x), with H^-1 from dd (its body table included).  One warp per (environment, body).
+//   mode 0 (Float64): xdot[env][n_x] += the term.
+//   mode 1 (one Dual<6> chunk, seeds on x[seed0 .. seed0 + 6)): xdot7[env][n_x][7] value += the term, partial k -= (H^-1 K)[row][seed0 + k].
+//   mode 2 (whole Jacobian): jac[env][row][col] -= (H^-1 K)[row][col] for the [q; v] columns; xdot[env][row] += the term (xdot may be nullptr).
+// The term and H^-1 K come from one routine in one operation order, so the whole Jacobian still equals its Dual<6> chunks bit for bit.
+cudaError_t launch_state_feedback(const StateDev& sd, const DynDev& dd, const FeedbackDev& fb, long long n_env, const double* x, int mode, int seed0,
+                                  double* xdot, double* jac, cudaStream_t stream, int* n_launches);
+// *bad = 1 if some entry of a[0 .. n) is not finite (*bad is not cleared first)
+cudaError_t launch_check_finite(const double* a, long long n, int* bad, cudaStream_t stream);
+
 // Refit of one mesh after its vertices moved (pfc_refit.cu): primitive records, leaf boxes, internal boxes bottom-up.  idx / eps / xyz /
 // level_nodes are device arrays of the mesh; nodes / tris / tets point at the mesh's slices; level_ptr is a HOST array of n_level + 1
 // offsets into level_nodes (internal nodes grouped by depth); aabb is scratch of 6 n_node doubles; *err gets bit 0 for a bad tetrahedron.
@@ -137,7 +156,10 @@ struct RadauBufs {
     const int* row;             // [env] body-table row of the environment (DynDev::row of the step), or nullptr: identity
     int* rowp;                  // [state] body-table row of the packed state, or nullptr: with a body table (pfc_set_body_params), the
                                 // DynDev::row of the stage evaluations, so they read the environment's row where it is
-    const double* xx0;          // [env][nx] calcXd!(x)
+    const int* fb_row;          // [env] feedback-table row of the environment (FeedbackDev::row of the step), or nullptr: identity
+    int* fb_rowp;               // [state] feedback-table row of the packed state, or nullptr: with a feedback table (pfc_set_feedback), the
+                                // FeedbackDev::row of the stage evaluations
+    const double* xx0;         // [env][nx] calcXd!(x)
     double* jac;                // [env][nx][nx] d xdot / d x, negated in place into -J
     double* invc;               // [matrix][nx][nx] complex: (h^-1 lambda_i I - J)^-1, matrices in the order of the round's plan
     double* shift;              // [matrix][2]
@@ -178,6 +200,8 @@ struct RadauRolloutBufs {
     RadauEnv* env_c; double* x_c; double* tau_c; double* t_c; double* h_c; double* h_save; int* stats_c;   // [slot] compact step arrays
     InsParam* params_c;         // [slot][n_ins] (with params)
     int n_ins;
+    int n_seg;                  // segments of the feedback table (1 or n_knot) ...
+    int* fb_list;               // ... [slot] its row (segment of the slot's next knot) * n_env + environment, or nullptr: no table
     int* count;                 // [2]: compact slots of the last selection; 1 if some environment starts within h_min of knot 0
 };
 // One CTA: lists the environments with knot < n_knot and steps < max_steps (environment order), gathers them (with their parameter rows)

@@ -160,12 +160,13 @@ __global__ void radau_prepare_kernel(RadauBufs b, const int* __restrict__ flags,
 }
 
 // one CTA per packed state: its stage vector (x0 at the first iteration of an attempt, which also initialises the stage), tau_ext, the
-// environment's contact parameters and, with a body table, the environment's row index (the rows themselves are not copied)
+// environment's contact parameters and, with a body or a feedback table, the environment's row index (the rows themselves are not copied)
 __global__ void __launch_bounds__(64) radau_gather_kernel(RadauBufs b) {
     const long long p = blockIdx.x;
     const int code = b.state_list[p], e = code >> 3, st = code & 7;
     const bool first = b.env[e].k_iter == 0;
     if (b.rowp && threadIdx.x == 0) b.rowp[p] = b.row ? b.row[e] : e;
+    if (b.fb_rowp && threadIdx.x == 0) b.fb_rowp[p] = b.fb_row ? b.fb_row[e] : e;
     double* Xs = b.X + ((long long)e * b.s_max + st) * b.nx;
     const double* x0 = b.x + (long long)e * b.nx;
     for (int n = threadIdx.x; n < b.nx; n += blockDim.x) {
@@ -329,6 +330,7 @@ __global__ void __launch_bounds__(kPlanThreads) radau_select_kernel(RadauRollout
             }
             if (b.params)
                 for (int n = 0; n < b.n_ins; ++n) b.params_c[p * b.n_ins + n] = b.params[e * b.n_ins + n];
+            if (b.fb_list) b.fb_list[p] = (int)((b.n_seg == 1 ? 0 : (long long)k) * b.n_env + e);
         }
         base += agg;
     }

@@ -324,6 +324,85 @@ __global__ void __launch_bounds__(128) state_dynamics_kernel(StateDev sd, DynDev
 
 unsigned state_blocks(long long n) { return (unsigned)((n + 127) / 128 < 148 * 16 ? (n + 127) / 128 : 148 * 16); }
 
+// sum_m h[m] k[m] in the order m = 0 .. 5, as explicit FMAs: every mode of the feedback kernel rounds these sums alike
+PFC_D double dot6(const double* h, const double* k) {
+    double a = 0.0;
+#pragma unroll
+    for (int m = 0; m < 6; ++m) a = fma(h[m], k[m], a);
+    return a;
+}
+
+// The feedback term of launch_state_feedback, one warp per (environment, body); see pfc_launch.h for the modes.  The term is subtracted
+// as H^-1 K (x - x_ref): with K = 0 every sum is +0.0, so the outputs keep their bits (a signed zero included).  K is read coalesced,
+// lanes over its columns; u = K (x - x_ref) is summed per lane in column order, then over the lanes by a butterfly that leaves the same
+// bits in every lane, so the result does not depend on the batch or on the launch shape.
+template <int kMode>
+__global__ void __launch_bounds__(128) state_feedback_kernel(StateDev sd, DynDev dd, FeedbackDev fb, long long n_env, const double* __restrict__ x,
+                                                             int seed0, double* __restrict__ xdot, double* __restrict__ jac) {
+    const int lane = threadIdx.x & 31;
+    const long long n = n_env * sd.n_body;
+    for (long long id = (blockIdx.x * (long long)blockDim.x + threadIdx.x) >> 5; id < n; id += ((long long)gridDim.x * blockDim.x) >> 5) {
+        const long long env = id / sd.n_body;
+        const int b = (int)(id - env * sd.n_body);
+        const BodyDev& body = sd.bodies[b];
+        if (body.joint == 0) continue;   // the same for the whole warp
+        const int nc = fb.ncol, nx = sd.n_x;
+        const long long r = fb.row ? fb.row[env] : env;
+        const double* Kb = fb.K + (r * sd.nv + body.v0) * nc;   // the body's six rows of K
+        const double* xref = fb.x_ref + r * nc;
+        const double* xe = x + env * nx;
+        const double* Hi = dd.Hinv + 36 * b;
+        if (dd.Hinv_env) Hi = dd.Hinv_env + 36 * ((dd.row ? dd.row[env] : env) * sd.n_body + b);
+        double u[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+        for (int j = lane; j < nc; j += 32) {
+            const double d = xe[j] - xref[j];
+#pragma unroll
+            for (int m = 0; m < 6; ++m) u[m] = fma(Kb[m * nc + j], d, u[m]);
+        }
+#pragma unroll
+        for (int m = 0; m < 6; ++m)
+#pragma unroll
+            for (int s = 16; s > 0; s >>= 1) u[m] = u[m] + __shfl_xor_sync(0xffffffffu, u[m], s);
+        if (kMode == 2) {   // -(H^-1 K) into the [q; v] columns of the body's v_dot rows, once for all seed chunks
+            double* jb = jac + ((size_t)env * nx + sd.nq + body.v0) * nx;
+            for (int j = lane; j < nc; j += 32) {
+                double kc[6];
+#pragma unroll
+                for (int m = 0; m < 6; ++m) kc[m] = Kb[m * nc + j];
+#pragma unroll
+                for (int i = 0; i < 6; ++i) jb[(size_t)i * nx + j] = jb[(size_t)i * nx + j] - dot6(Hi + 6 * i, kc);
+            }
+        }
+        if (lane < 6) {   // lane i: v_dot row i of the body
+            double h[6];
+#pragma unroll
+            for (int m = 0; m < 6; ++m) h[m] = Hi[6 * lane + m];
+            const double a = dot6(h, u);
+            const long long o = env * nx + sd.nq + body.v0 + lane;
+            if (kMode == 0 || (kMode == 2 && xdot)) xdot[o] = xdot[o] - a;
+            if (kMode == 1) {
+                double* p = xdot + 7 * o;
+                p[0] = p[0] - a;
+#pragma unroll
+                for (int k = 0; k < 6; ++k) {
+                    const int col = seed0 + k;
+                    if (col >= nc) break;   // bristle seeds: the feedback does not read s
+                    double kc[6];
+#pragma unroll
+                    for (int m = 0; m < 6; ++m) kc[m] = Kb[m * nc + col];
+                    p[1 + k] = p[1 + k] - dot6(h, kc);
+                }
+            }
+        }
+    }
+}
+
+__global__ void __launch_bounds__(256) check_finite_kernel(const double* __restrict__ a, long long n, int* __restrict__ bad) {
+    int b = 0;
+    for (long long id = blockIdx.x * (long long)blockDim.x + threadIdx.x; id < n; id += (long long)gridDim.x * blockDim.x) b |= !isfinite(a[id]);
+    if (__syncthreads_or(b) && threadIdx.x == 0) atomicOr(bad, 1);
+}
+
 }  // namespace
 
 cudaError_t launch_state_prologue(const StateDev& sd, long long n_env, int n_ins, int n_bristle, const double* x, double* X, double* twist, double* s,
@@ -371,6 +450,23 @@ cudaError_t launch_state_dynamics_dual6(const StateDev& sd, const DynDev& dd, lo
     (dd.H_env ? state_dynamics_kernel<D6, true> : state_dynamics_kernel<D6, false>)<<<state_blocks(n), 128, 0, stream>>>(
         sd, dd, n_env, n_real > 0 ? n_real : n_env, n_ins, n_bristle, x, seed0, wrench7, tau_ext, sdot7, XdotOut{xdot7, jac, sd.n_x}, flags, status);
     if (n_launches) *n_launches += 1;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_state_feedback(const StateDev& sd, const DynDev& dd, const FeedbackDev& fb, long long n_env, const double* x, int mode, int seed0,
+                                  double* xdot, double* jac, cudaStream_t stream, int* n_launches) {
+    const long long n = n_env * sd.n_body;
+    if (n == 0) return cudaSuccess;
+    auto kern = mode == 0 ? state_feedback_kernel<0> : mode == 1 ? state_feedback_kernel<1> : state_feedback_kernel<2>;
+    kern<<<state_blocks(32 * n), 128, 0, stream>>>(sd, dd, fb, n_env, x, seed0, xdot, jac);
+    if (n_launches) *n_launches += 1;
+    return cudaGetLastError();
+}
+
+cudaError_t launch_check_finite(const double* a, long long n, int* bad, cudaStream_t stream) {
+    if (n == 0) return cudaSuccess;
+    const long long blocks = (n + 255) / 256 < 148 * 8 ? (n + 255) / 256 : 148 * 8;
+    check_finite_kernel<<<(unsigned)blocks, 256, 0, stream>>>(a, n, bad);
     return cudaGetLastError();
 }
 
